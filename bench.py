@@ -402,14 +402,25 @@ def run_product_arm(args, rank, local_rank, world):
     per_step_all = []
     totals = []
     for _ in range(REPEATS):
-        totals.append(timed(toast_graphed, args.steps)[0])
+        t_, last = timed(toast_graphed, args.steps)
+        totals.append(t_)
         per_step_all += timed.last_per_step
     total_ms = min(totals)
-    # distribution of the per-step device time over >= 100 steps (this rank; SURVEY.md §8d asks for median, p10, p90)
-    while len(per_step_all) < 100:
-        timed(toast_graphed, max(args.steps, 20))
-        per_step_all += timed.last_per_step
+    # distribution of the per-step device time over the REPEATS x K timed steps (this rank; SURVEY.md §8d asks for
+    # median, p10, p90)
     step_stats = dist_stats(per_step_all)
+    # what the caller of the timed step received from its last replay: the image, the radii and the packed [P,14]
+    # gradients (summed over the ranks), copied to the host now, before other legs reuse the device buffers
+    last_outputs = None
+    if args.dump_outputs:
+        b = (step_no[0] - 1) & 1
+        if pending[b] is not None:
+            pending[b].wait()
+        torch.cuda.synchronize(device)
+        n_last = graphs[b].num_rendered() if graphs is not None else last[2]
+        last_outputs = {k: v.detach().float().cpu().numpy() for k, v in
+                        (("image", last[0]), ("radii", last[1]), ("grads", grad_bufs[b]))}
+        last_outputs["num_rendered"] = np.float64(n_last)
     if graphs is not None and not graphs[0].capacity_ok():
         raise SystemExit("the captured instance capacity was exceeded (cannot happen with a fixed scene)")
     launches = kernels_per_step * args.steps
@@ -579,7 +590,7 @@ def run_product_arm(args, rank, local_rank, world):
         for _ in range(3):
             R5 = c5_eager()
         torch.cuda.synchronize(device)
-        n5 = max(5, args.steps // 2)
+        n5 = args.steps
         e5_ms = min(timed(c5_eager, n5)[0] for _ in range(2))
         g5_ms = min(timed(step5, n5)[0] for _ in range(2)) if step5 is not None else None
         config5 = {"workload": "2M Gaussians, 3840x2160, forward + backward of one view (BASELINE.json configs[4])",
@@ -656,7 +667,7 @@ def run_product_arm(args, rank, local_rank, world):
             elif world > 1:
                 dist.all_reduce(buf3, op=dist.ReduceOp.SUM)      # on the compute stream: the step ends when it has
 
-        n3 = max(5, args.steps // 2)
+        n3 = args.steps
         for _ in range(3):
             c3_step()
         torch.cuda.synchronize(device)
@@ -704,7 +715,7 @@ def run_product_arm(args, rank, local_rank, world):
             for _ in range(3):
                 step()
             torch.cuda.synchronize(device)
-            return min(timed(step, max(5, args.steps // 2))[0] for _ in range(2)) / max(5, args.steps // 2)
+            return min(timed(step, args.steps)[0] for _ in range(2)) / args.steps
 
         epilogue = {"anchors": Na, "visible": nv_, "n_offsets": Ka,
                     "fused_fwd_ms": ep_run(neural_gaussians_epilogue, False), "torch_fwd_ms": ep_run(reference_epilogue, False, K=Ka),
@@ -790,9 +801,9 @@ def run_product_arm(args, rank, local_rank, world):
 
     e2e_steps(6)      # per slot: one eager step (sizes the binning buffer), then the CUDA-graph capture
 
-    # the pipeline's fill (first upload + exchange) and drain (last exchange + read-back) are inside the timed region;
-    # over the driver's 20-step window they would be 5 % of it, so the e2e leg runs at least 100 steps (stated below)
-    E2E_STEPS = max(args.steps, 100)
+    # the pipeline's fill (first upload + exchange) and drain (last exchange + read-back) are inside the timed region:
+    # about 1 % of 100 steps, 5 % of 20
+    E2E_STEPS = args.steps
 
     def e2e_run():
         sync_all()
@@ -1018,6 +1029,10 @@ def run_product_arm(args, rank, local_rank, world):
                 "sample": (f"C oracle (oracle/splat_oracle.c, OpenMP, {cores} host threads), same scene, ONE view "
                            f"forward+backward over all {P} Gaussians and every pixel: best of 30 whole "
                            f"view-iterations, {best:.2f} s each ({sum(r[1] for r in reps):.0f} s of CPU-side work)")}
+        if last_outputs is not None:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, a in last_outputs.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
         emit(line)
     if world > 1:
         dist.destroy_process_group()
@@ -1050,7 +1065,14 @@ def main():
     ap.add_argument("--impl", default="gsvc", choices=["gsvc", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-gpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the timed step returned in its last step (image, radii, packed [P,14] gradients, "
+                         "instance count) as DIR/<name>.npy, float32 / float64, about 38 MB; the inputs are seeded")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "gsvc":
+        ap.error("--dump-outputs writes the outputs of the product arm (--impl gsvc)")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
