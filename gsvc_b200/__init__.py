@@ -2,7 +2,8 @@
 
   rasterizer   GaussianRasterizationSettings / GaussianRasterizer: the reference-shaped drop-in (renderer.py:63-98)
   views        ViewBatch / rasterize_views / render_toast: a frame's front + back view (or a window) in one chain
-  graphed      GraphedStep: CUDA-graph replay of forward + backward on static tensors
+  graphed      GraphedStep: CUDA-graph replay of forward + backward on static tensors (optionally with its own loss)
+  loss         photometric_loss: the fused L1 + D-SSIM training loss (SPEC U9)
   hostpipe     HostStepPipeline: pinned host parameters in, pinned host gradients out, copies overlapped
   sharding     frame-sharded rendering, packed [P,14] gradients, NCCL all-reduce
   frames       cube geometry and the synthetic workload generator

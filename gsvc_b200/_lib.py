@@ -95,6 +95,9 @@ SIGNATURES = {
     "gsvc_gen_epilogue_scratch_bytes": (_sz, [_i32, _i32]),
     "gsvc_gen_epilogue_forward": (C.c_int, [_i32, _i32] + [_vp] * 20 + [_vp, C.c_uint32, _vp]),
     "gsvc_gen_epilogue_backward": (C.c_int, [_i32, _i32] + [_vp] * 26),
+    "gsvc_rast_loss_scratch_bytes": (_sz, [_i32, _i32, _i32]),
+    "gsvc_rast_loss_forward": (C.c_int, [_i32, _i32, _i32, _vp, _vp, C.c_float, _vp, _vp, _vp]),
+    "gsvc_rast_loss_backward": (C.c_int, [_i32, _i32, _i32, _vp, _vp, C.c_float, _vp, _vp, _vp]),
 }
 
 STAGES = ("preprocess", "tile_scan", "scatter", "sort_tiles", "render_forward", "render_backward",

@@ -26,6 +26,7 @@ SOURCES = {
     "render.cu": [],
     "preprocess_bwd.cu": [],
     "epilogue.cu": [],
+    "loss.cu": [],
     "collective.cu": [],
     "api.cu": [],
 }

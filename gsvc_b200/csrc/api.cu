@@ -41,7 +41,8 @@ struct StageScope {
     }
 };
 
-static int fail(int code, const char* fmt, ...)
+// (also the error channel of loss.cu)
+int fail(int code, const char* fmt, ...)
 {
     va_list ap;
     va_start(ap, fmt);

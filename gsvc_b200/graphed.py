@@ -13,6 +13,13 @@ the 8 kernels back to back with their programmatic-dependent-launch edges preser
     ...
     if not step.capacity_ok(): step.recapture()        # after a synchronisation, e.g. once per N steps
 
+The step can also own its loss: with a static target tensor the captured graph renders, evaluates the fused
+L1 + D-SSIM loss (gsvc_b200.loss) against it and back-propagates, so the whole step is one graph launch:
+
+    step = GraphedStep(batch, params, None, loss_target=target, lambda_dssim=0.2)   # target [n_out,3,H,W]
+    target.copy_(frames)                                # this iteration's target frames, in place
+    color, radii, grads = step()                        # step.loss: the per-image losses of this replay
+
 The binning capacity is fixed at capture time from an eager warm-up (+50 % + 64 Ki instances);
 `capacity_ok()` compares it with the instance count the device published for the last replay.
 """
@@ -23,6 +30,7 @@ from typing import Dict, Optional
 import torch
 
 from . import rasterizer as R
+from .loss import _check_lambda, photometric_loss
 from .rasterizer import RasterizerError
 from .sharding import GRAD_LAYOUT, GRAD_WIDTH, packed_backward
 from .views import ViewBatch, rasterize_views
@@ -30,19 +38,34 @@ from .views import ViewBatch, rasterize_views
 
 class GraphedStep:
     def __init__(self, rast, params: Dict[str, torch.Tensor], dL: Optional[torch.Tensor],
-                 packed: Optional[torch.Tensor] = None, warmup: int = 2, exchange=None):
+                 packed: Optional[torch.Tensor] = None, warmup: int = 2, exchange=None,
+                 loss_target: Optional[torch.Tensor] = None, lambda_dssim: float = 0.2):
         """`rast`: a GaussianRasterizer (one view, dL [3,H,W]) or a views.ViewBatch (all its views in one chain,
         dL [n_out,3,H,W], gradients summed over the views).  `dL` None: forward only.  `packed`: optional [P,14]
         buffer the backward writes (sharding.GRAD_LAYOUT); allocated here if omitted.  `exchange`: a
         sharding.SwitchAllReduce over P*14 floats — the backward then writes into ITS buffer and carries the sum over the
-        ranks in its own launches (ViewBatch steps only; every rank builds and replays the same step)."""
+        ranks in its own launches (ViewBatch steps only; every rank builds and replays the same step).
+        `loss_target`: a static CUDA tensor shaped like the rendered image ([3,H,W] / [n_out,3,H,W]) instead of `dL`:
+        the step then evaluates photometric_loss(image, loss_target, lambda_dssim) into the static `self.loss` (0-dim /
+        [n_out]) and back-propagates the MEAN of the per-image losses.  Write each iteration's targets into it in
+        place."""
         self.rast, self.params, self.dL = rast, params, dL
         self.batch = rast if isinstance(rast, ViewBatch) else None
         m = params["means3D"]
         if not m.is_cuda:
             raise RasterizerError("GraphedStep needs CUDA tensors: gsvc_b200 has no CPU fallback")
         self.device, self.P = m.device, int(m.shape[0])
-        self.backward = dL is not None
+        self.loss_target, self.loss = loss_target, None
+        if loss_target is not None:
+            if dL is not None:
+                raise RasterizerError("pass either dL (a fixed seed gradient) or loss_target (the step's own loss)")
+            self.lambda_dssim = _check_lambda(lambda_dssim)
+            if not isinstance(loss_target, torch.Tensor) or loss_target.device != self.device:
+                raise RasterizerError(f"loss_target must be a tensor on {self.device}")
+            if loss_target.dtype != torch.float32 or not loss_target.is_contiguous():
+                # a converted copy would be baked into the graph: in-place updates of the caller's tensor would be lost
+                raise RasterizerError("loss_target must be a contiguous fp32 tensor (the graph reads it in place)")
+        self.backward = dL is not None or loss_target is not None
         self.exchange = exchange
         if exchange is not None:
             if self.batch is None or not self.backward:
@@ -74,13 +97,19 @@ class GraphedStep:
         p = self.params
         if not self.backward:
             with torch.no_grad():
-                return self._call(p, p["means3D"])
+                return (*self._call(p, p["means3D"]), None)
         leaves = {k: p[k].detach().requires_grad_(True) for k, _ in GRAD_LAYOUT}
         means2D = None if self.batch is not None else torch.zeros_like(leaves["means3D"], requires_grad=True)
         color, radii, n = self._call(leaves, means2D)
+        loss = None
+        if self.loss_target is not None:
+            loss = photometric_loss(color, self.loss_target, self.lambda_dssim)
+            with packed_backward(self.packed, exchange=self.exchange):
+                torch.autograd.grad(loss.mean(), [leaves[k] for k, _ in GRAD_LAYOUT])
+            return color, radii, n, loss
         with packed_backward(self.packed, exchange=self.exchange):
             torch.autograd.grad(color, [leaves[k] for k, _ in GRAD_LAYOUT], grad_outputs=self.dL)
-        return color, radii, n
+        return color, radii, n, loss
 
     def recapture(self) -> None:
         """(Re)build the graph: eager warm-up on a side stream (sets the capacity hint), then capture."""
@@ -89,14 +118,14 @@ class GraphedStep:
         side.wait_stream(cur)
         with torch.cuda.stream(side):
             for _ in range(self.warmup):
-                _, _, n = self._run()
+                _, _, n, _ = self._run()
         cur.wait_stream(side)
         torch.cuda.synchronize(self.device)
         R.overflow_events(self.device)      # an eager warm-up call that outgrew its hint re-ran by itself: not ours
         self.num_rendered_at_capture = n
         self.graph = torch.cuda.CUDAGraph()
         with R.own_count_slot(self.slot), torch.cuda.graph(self.graph):
-            self.color, self.radii, _ = self._run()
+            self.color, self.radii, _, self.loss = self._run()
         rs = self.batch.settings[0] if self.batch is not None else self.rast.raster_settings
         key = (self.device.index, self.P, int(rs.image_height), int(rs.image_width))
         self.capacity = R._captured_caps.get(key + ((self.batch.n_views,) if self.batch is not None else ()))

@@ -381,6 +381,29 @@ GSVC_RAST_API int gsvc_gen_epilogue_backward(int32_t n_vis, int32_t K, const int
                                              float *d_scale_rot, float *d_neural_offset, float *d_anchor,
                                              float *d_grid_offsets, float *d_grid_scaling, float *d_masks, void *stream);
 
+/*
+ * Photometric training loss (docs/SPEC.md "Photometric loss", decision U9): the L1 + D-SSIM term of the reference's
+ * iteration (pipeline/train.py:407-444, the upstream 3DGS ssim of utils/loss_utils.py:41-72), fused.  For each image n
+ * of x = image, y = target, both [n_images,3,H,W] fp32:
+ *     loss[n] = (1 - lambda) * mean|x - y| + lambda * (1 - mean S)        means over the image's 3*H*W values
+ *     S = (2 mu_x mu_y + C1)(2 sigma_xy + C2) / ((mu_x^2 + mu_y^2 + C1)(sigma_x^2 + sigma_y^2 + C2))
+ * with the moments taken per channel through the 11x11 Gaussian window (sigma 1.5) with zero padding of 5 (F.conv2d
+ * semantics), C1 = 0.01^2, C2 = 0.03^2.  lambda_dssim in [0, 1] (upstream default 0.2; 0 = L1, 1 = 1 - SSIM).
+ *   gsvc_rast_loss_forward   writes loss [n_images] (device).  scratch: gsvc_rast_loss_scratch_bytes(n_images, H, W)
+ *                            bytes for the per-CTA partial sums (their per-image sum runs in a fixed order: the result
+ *                            is bit-reproducible).  Two launches.
+ *   gsvc_rast_loss_backward  writes dL_dimage [n_images,3,H,W] = dL_dloss[n] * d loss[n] / d image, dL_dloss [n_images]
+ *                            read on the device (no host synchronisation).  It recomputes the moments from image and
+ *                            target (the forward leaves nothing behind) and needs no scratch.  One launch, no atomics.
+ * The target gets no gradient.  d|x - y|/dx is 0 where x == y.
+ */
+GSVC_RAST_API size_t gsvc_rast_loss_scratch_bytes(int32_t n_images, int32_t H, int32_t W);
+GSVC_RAST_API int gsvc_rast_loss_forward(int32_t n_images, int32_t H, int32_t W, const float *image, const float *target,
+                                         float lambda_dssim, float *loss, void *scratch, void *stream);
+GSVC_RAST_API int gsvc_rast_loss_backward(int32_t n_images, int32_t H, int32_t W, const float *image,
+                                          const float *target, float lambda_dssim, const float *dL_dloss,
+                                          float *dL_dimage, void *stream);
+
 #ifdef __cplusplus
 }
 #endif
