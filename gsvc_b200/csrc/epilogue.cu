@@ -175,6 +175,8 @@ __global__ void __launch_bounds__(128) epi_backward_kernel(EpiIn in, const int32
     for (int c = 0; c < 6; c++) g.d_grid_scaling[(size_t)n * 6 + c] = d_gs[c];
 }
 
+int fail(int code, const char* fmt, ...);   // api.cu: the last_error channel
+
 cudaError_t launch_compact_scan(int n_ctas, const unsigned int* cta_count, unsigned int* cta_offset,
                                 unsigned long long* count_dev, unsigned long long* host_slot, unsigned int ticket,
                                 cudaStream_t st);
@@ -201,7 +203,8 @@ int gsvc_gen_epilogue_forward(int32_t n_vis, int32_t K, const int32_t* visible_i
                               uint64_t* count_slot_host, uint32_t ticket, void* stream_)
 {
     cudaStream_t st = static_cast<cudaStream_t>(stream_);
-    if (n_vis < 0 || K < 1) return GSVC_RAST_ERR_INVALID;
+    if (n_vis < 0 || K < 1)
+        return fail(GSVC_RAST_ERR_INVALID, "epilogue_forward: n_vis must be >= 0 and K >= 1, got %d, %d", n_vis, K);
     if (n_vis == 0) {
         if (count_slot_host) *count_slot_host = (uint64_t)(ticket & 0xFFFFFFu) << 40;
         return GSVC_RAST_OK;
@@ -209,9 +212,10 @@ int gsvc_gen_epilogue_forward(int32_t n_vis, int32_t K, const int32_t* visible_i
     if (!anchor || !grid_offsets || !grid_scaling || !masks || !neural_opacity || !color || !scale_rot || !neural_offset ||
         !bound_min || !bound_max || !xyz || !color_out || !opacity_out || !scaling_out || !rot_out || !neural_opacity_full ||
         !selection_mask || !rank || !scratch)
-        return GSVC_RAST_ERR_INVALID;
+        return fail(GSVC_RAST_ERR_INVALID, "epilogue_forward: an input, output or scratch pointer is NULL");
     const long long total = (long long)n_vis * K;
-    if (total > 0x7fffffffll) return GSVC_RAST_ERR_INVALID;
+    if (total > 0x7fffffffll)
+        return fail(GSVC_RAST_ERR_INVALID, "epilogue_forward: n_vis * K = %lld exceeds 2^31 - 1", total);
     const int n_ctas = (int)((total + 255) / 256);
     char* p = static_cast<char*>(scratch);
     unsigned long long* count_dev = carve<unsigned long long>(p, 1);
@@ -230,7 +234,7 @@ int gsvc_gen_epilogue_forward(int32_t n_vis, int32_t K, const int32_t* visible_i
         e = launch_pdl(epi_write_kernel, dim3(n_ctas), dim3(256), st, in, (const unsigned int*)ballots,
                        (const unsigned int*)cta_offset, rank, xyz, color_out, opacity_out, scaling_out, rot_out,
                        (const float*)neural_opacity_full);
-    return e == cudaSuccess ? GSVC_RAST_OK : GSVC_RAST_ERR_CUDA;
+    return e == cudaSuccess ? GSVC_RAST_OK : fail(GSVC_RAST_ERR_CUDA, "epilogue_forward: %s", cudaGetErrorString(e));
 }
 
 int gsvc_gen_epilogue_backward(int32_t n_vis, int32_t K, const int32_t* visible_indices, const float* anchor,
@@ -243,20 +247,21 @@ int gsvc_gen_epilogue_backward(int32_t n_vis, int32_t K, const int32_t* visible_
                                float* d_grid_scaling, float* d_masks, void* stream_)
 {
     cudaStream_t st = static_cast<cudaStream_t>(stream_);
-    if (n_vis < 0 || K < 1) return GSVC_RAST_ERR_INVALID;
+    if (n_vis < 0 || K < 1)
+        return fail(GSVC_RAST_ERR_INVALID, "epilogue_backward: n_vis must be >= 0 and K >= 1, got %d, %d", n_vis, K);
     if (n_vis == 0) return GSVC_RAST_OK;
     if (!anchor || !grid_offsets || !grid_scaling || !masks || !neural_opacity || !scale_rot || !neural_offset || !rank ||
         !bound_min || !bound_max || !dL_dxyz || !dL_dcolor || !dL_dopacity || !dL_dscaling || !dL_drot ||
         !d_neural_opacity || !d_color || !d_scale_rot || !d_neural_offset || !d_anchor || !d_grid_offsets ||
         !d_grid_scaling || !d_masks)
-        return GSVC_RAST_ERR_INVALID;
+        return fail(GSVC_RAST_ERR_INVALID, "epilogue_backward: an input, gradient or output pointer is NULL");
     EpiIn in{n_vis, K, visible_indices, anchor, grid_offsets, grid_scaling, masks, neural_opacity, nullptr, scale_rot,
              neural_offset, bound_min, bound_max};
     EpiGrads g{dL_dxyz, dL_dcolor, dL_dopacity, dL_dscaling, dL_drot, dL_dnop_full, d_neural_opacity, d_color,
                d_scale_rot, d_neural_offset, d_anchor, d_grid_offsets, d_grid_scaling, d_masks};
     count_launch();
     cudaError_t e = launch_pdl(epi_backward_kernel, dim3((n_vis + 127) / 128), dim3(128), st, in, rank, g);
-    return e == cudaSuccess ? GSVC_RAST_OK : GSVC_RAST_ERR_CUDA;
+    return e == cudaSuccess ? GSVC_RAST_OK : fail(GSVC_RAST_ERR_CUDA, "epilogue_backward: %s", cudaGetErrorString(e));
 }
 
 }  // extern "C"

@@ -21,6 +21,7 @@ There is no CPU fallback.
 """
 from __future__ import annotations
 
+import weakref
 from typing import Optional, Sequence
 
 import torch
@@ -39,18 +40,22 @@ _bg_checked: dict = {}
 
 
 def _same_bg(a, b) -> bool:
-    """Background colours of two settings are equal.  Distinct CUDA tensors are compared once per pair of storages
-    (a device→host read); the reference keeps ONE background tensor for all its views (pipeline/train.py:328)."""
+    """Background colours of two settings are equal.  Distinct CUDA tensors are compared once per pair of tensors
+    (a device→host read); the reference keeps ONE background tensor for all its views (pipeline/train.py:328).
+    An entry holds weak references to the two tensors it was computed from and is valid only while both are alive:
+    the caching allocator hands a freed background's address to the next small tensor, which may hold other values."""
     if a is b:
         return True
     ta, tb = torch.as_tensor(a), torch.as_tensor(b)
     if ta.is_cuda or tb.is_cuda:
         key = (ta.data_ptr(), tb.data_ptr(), ta._version, tb._version)
-        if key not in _bg_checked:
+        hit = _bg_checked.get(key)
+        if hit is None or hit[0]() is not ta or hit[1]() is not tb:
             if len(_bg_checked) > 256:
                 _bg_checked.clear()
-            _bg_checked[key] = ta.detach().cpu().reshape(-1).tolist() == tb.detach().cpu().reshape(-1).tolist()
-        return _bg_checked[key]
+            same = ta.detach().cpu().reshape(-1).tolist() == tb.detach().cpu().reshape(-1).tolist()
+            hit = _bg_checked[key] = (weakref.ref(ta), weakref.ref(tb), same)
+        return hit[2]
     return torch.equal(ta.float(), tb.float())
 
 

@@ -159,3 +159,115 @@ def test_exchange_entry_points_validate_before_any_cuda_work(lib):
     assert lib.gsvc_rast_backward_views_exchange(*args, p, C.byref(x), None) == _lib.ERR_INVALID      # no mover CTA
     x = _lib.Exchange(None, p, p, p, 0, 16, 0, 0)
     assert lib.gsvc_rast_backward_views_exchange(*args, p, C.byref(x), None) == _lib.ERR_INVALID      # peer path > 8 ranks
+
+
+def _poison(lib):
+    """Leave a known message in last_error (a failing call of another entry point), so that a test can tell a fresh
+    message from a stale one."""
+    assert lib.gsvc_rast_wait_count(None, 1, None) == _lib.ERR_INVALID
+    assert lib.gsvc_rast_last_error() == b"count_slot_host is NULL"
+
+
+def test_view_batch_entry_points_validate_the_map_before_any_cuda_work(lib):
+    """The three batched-view entry points reject a bad view map with ERR_INVALID and a message of their own.
+    Every other argument is a plausible placeholder that is never dereferenced: the map is checked first."""
+    p = 0x1000
+    s = _lib.Settings()
+    s.image_height, s.image_width, s.viewmatrix, s.bg, s.vm_stride_r, s.vm_stride_c = 48, 64, p, p, 4, 1
+
+    def views(out_image, null_vm=()):
+        arr = (_lib.View * max(len(out_image), 1))()
+        for v, o in enumerate(out_image):
+            arr[v].viewmatrix = None if v in null_vm else p
+            arr[v].vm_stride_r, arr[v].vm_stride_c = 4, 1
+            arr[v].out_image, arr[v].flip_x, arr[v].weight = o, 0, 1.0
+        return arr
+
+    def launch(n_views, arr, n_out):
+        return lib.gsvc_rast_forward_views_launch(C.byref(s), n_views, arr, n_out, 100, 0, p, None, p, p, p, p, None,
+                                                  p, p, p, 1000, None, p, p, None, 0, None)
+
+    def render(n_views, arr, n_out):
+        return lib.gsvc_rast_forward_views_render(C.byref(s), n_views, arr, n_out, 100, p, p, p, 1000, p, None)
+
+    def backward(n_views, arr, n_out):
+        return lib.gsvc_rast_backward_views(C.byref(s), n_views, arr, n_out, 100, 0, 1000, p, None, p, p, p, None, p,
+                                            p, p, p, p, 0, p, p, p, p, p, p, p, None, None, None, None)
+
+    cases = [
+        (0, views([]), 1, b"n_views must be in 1..16, got 0"),
+        (17, views([0] * 17), 1, b"n_views must be in 1..16, got 17"),
+        (2, views([0, 1]), 0, b"n_out must be in 1..n_views"),
+        (2, views([0, 1]), 3, b"n_out must be in 1..n_views"),
+        (3, views([0, 2, 1]), 2, b"out_image of view 1 is 2, expected 0..1"),
+        (2, views([0, -1]), 2, b"out_image of view 1 is -1, expected 0..1"),
+        (3, views([0, 0, 0]), 2, b"output image 1 has no view"),
+        (4, views([0, 1, 2, 0]), 4, b"output image 3 has no view"),
+        (2, None, 1, b"views is NULL"),
+        (3, views([0, 1, 2], null_vm=(1,)), 3, b"viewmatrix of view 1 is NULL"),
+    ]
+    for fn in (launch, render, backward):
+        for n_views, arr, n_out, msg in cases:
+            _poison(lib)
+            assert fn(n_views, arr, n_out) == _lib.ERR_INVALID, (fn.__name__, n_views, n_out, msg)
+            assert lib.gsvc_rast_last_error() == msg, (fn.__name__, lib.gsvc_rast_last_error(), msg)
+    # the same placeholders with a valid map get past the map: the next check (both colour sources) rejects them
+    _poison(lib)
+    assert lib.gsvc_rast_forward_views_launch(C.byref(s), 2, views([0, 0]), 1, 100, 0, p, p, p, p, p, p, None, p, p,
+                                              p, 1000, None, p, p, None, 0, None) == _lib.ERR_INVALID
+    assert b"SHs or precomputed colors" in lib.gsvc_rast_last_error()
+
+
+# gsvc_gen_epilogue_forward: (n_vis, K, visible_indices, 19 required pointers, count_slot_host, ticket, stream)
+_EPI_FWD_REQUIRED = ("anchor", "grid_offsets", "grid_scaling", "masks", "neural_opacity", "color", "scale_rot",
+                     "neural_offset", "bound_min", "bound_max", "xyz", "color_out", "opacity_out", "scaling_out",
+                     "rot_out", "neural_opacity_full", "selection_mask", "rank", "scratch")
+# gsvc_gen_epilogue_backward: (n_vis, K, visible_indices, 13 required, dL_dnop_full (optional), 8 required, stream)
+_EPI_BWD_REQUIRED = ("anchor", "grid_offsets", "grid_scaling", "masks", "neural_opacity", "scale_rot", "neural_offset",
+                     "bound_min", "bound_max", "rank", "dL_dxyz", "dL_dcolor", "dL_dopacity", "dL_dscaling", "dL_drot")
+_EPI_BWD_OUTPUTS = ("d_neural_opacity", "d_color", "d_scale_rot", "d_neural_offset", "d_anchor", "d_grid_offsets",
+                    "d_grid_scaling", "d_masks")
+
+
+def test_generator_epilogue_reports_argument_errors_through_last_error(lib):
+    """Bad arguments of the generator epilogue return ERR_INVALID and leave a message that names the problem in
+    last_error, instead of the message of whichever call failed before.  Nothing here reaches a launch."""
+    p = 0x1000
+
+    def fwd(n_vis, K, null=None):
+        ptrs = [None if name == null else p for name in _EPI_FWD_REQUIRED]
+        return lib.gsvc_gen_epilogue_forward(n_vis, K, None, *ptrs, None, 0, None)
+
+    def bwd(n_vis, K, null=None):
+        ins = [None if name == null else p for name in _EPI_BWD_REQUIRED]
+        outs = [None if name == null else p for name in _EPI_BWD_OUTPUTS]
+        return lib.gsvc_gen_epilogue_backward(n_vis, K, None, *ins, None, *outs, None)
+
+    for call, name in ((fwd, "epilogue_forward"), (bwd, "epilogue_backward")):
+        for n_vis, K in ((10, 0), (-1, 4), (10, -3)):
+            _poison(lib)
+            assert call(n_vis, K) == _lib.ERR_INVALID
+            err = lib.gsvc_rast_last_error().decode()
+            assert name in err and f"got {n_vis}, {K}" in err, err
+        for null in (_EPI_FWD_REQUIRED if call is fwd else _EPI_BWD_REQUIRED + _EPI_BWD_OUTPUTS):
+            _poison(lib)
+            assert call(10, 4, null=null) == _lib.ERR_INVALID, null
+            err = lib.gsvc_rast_last_error().decode()
+            assert name in err and "NULL" in err, (null, err)
+    # n_vis * K past 2^31 - 1 (the forward's element index is 32-bit); the backward loops over K per anchor instead
+    _poison(lib)
+    assert fwd(65536, 32768) == _lib.ERR_INVALID
+    err = lib.gsvc_rast_last_error().decode()
+    assert "epilogue_forward" in err and "2147483648" in err, err
+
+
+def test_generator_epilogue_with_no_visible_anchor_publishes_an_empty_count(lib):
+    """n_vis = 0: nothing to launch; the forward still publishes a count of 0 under the caller's ticket (low 24 bits)
+    in the host slot, so that a caller waiting on that slot returns."""
+    for ticket in (0x123, 0x1234567):
+        slot = C.c_uint64(0xFFFF_FFFF_FFFF_FFFF)
+        assert lib.gsvc_gen_epilogue_forward(0, 4, *([None] * 20), C.byref(slot), ticket, None) == _lib.OK
+        assert slot.value == (ticket & 0xFFFFFF) << 40
+        assert lib.gsvc_rast_wait_count(C.byref(slot), ticket, None) == 0
+    assert lib.gsvc_gen_epilogue_forward(0, 4, *([None] * 20), None, 1, None) == _lib.OK
+    assert lib.gsvc_gen_epilogue_backward(0, 4, *([None] * 26)) == _lib.OK
