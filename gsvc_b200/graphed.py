@@ -33,7 +33,7 @@ from . import rasterizer as R
 from .loss import _check_lambda, photometric_loss
 from .rasterizer import RasterizerError
 from .sharding import GRAD_LAYOUT, GRAD_WIDTH, packed_backward
-from .views import ViewBatch, rasterize_views
+from .views import ViewBatch, capacity_shape, render_params
 
 
 class GraphedStep:
@@ -50,7 +50,6 @@ class GraphedStep:
         [n_out]) and back-propagates the MEAN of the per-image losses.  Write each iteration's targets into it in
         place."""
         self.rast, self.params, self.dL = rast, params, dL
-        self.batch = rast if isinstance(rast, ViewBatch) else None
         m = params["means3D"]
         if not m.is_cuda:
             raise RasterizerError("GraphedStep needs CUDA tensors: gsvc_b200 has no CPU fallback")
@@ -68,7 +67,7 @@ class GraphedStep:
         self.backward = dL is not None or loss_target is not None
         self.exchange = exchange
         if exchange is not None:
-            if self.batch is None or not self.backward:
+            if not isinstance(rast, ViewBatch) or not self.backward:
                 raise RasterizerError("a step carries the exchange in its batched-view backward: pass a ViewBatch and dL")
             if packed is not None:
                 raise RasterizerError("with `exchange` the packed buffer is the exchange's own")
@@ -86,21 +85,13 @@ class GraphedStep:
         self.capacity = None
         self.recapture()
 
-    def _call(self, p, means2D):
-        if self.batch is not None:
-            return rasterize_views(self.batch, means3D=p["means3D"], opacities=p["opacities"], means2D=None,
-                                   colors_precomp=p["colors_precomp"], scales=p["scales"], rotations=p["rotations"])
-        return self.rast(means3D=p["means3D"], means2D=means2D, shs=None, colors_precomp=p["colors_precomp"],
-                         opacities=p["opacities"], scales=p["scales"], rotations=p["rotations"], cov3D_precomp=None)
-
     def _run(self):
         p = self.params
         if not self.backward:
             with torch.no_grad():
-                return (*self._call(p, p["means3D"]), None)
+                return (*render_params(self.rast, p, means2D=p["means3D"]), None)   # no gradient: any tensor serves
         leaves = {k: p[k].detach().requires_grad_(True) for k, _ in GRAD_LAYOUT}
-        means2D = None if self.batch is not None else torch.zeros_like(leaves["means3D"], requires_grad=True)
-        color, radii, n = self._call(leaves, means2D)
+        color, radii, n = render_params(self.rast, leaves)
         loss = None
         if self.loss_target is not None:
             loss = photometric_loss(color, self.loss_target, self.lambda_dssim)
@@ -126,9 +117,7 @@ class GraphedStep:
         self.graph = torch.cuda.CUDAGraph()
         with R.own_count_slot(self.slot), torch.cuda.graph(self.graph):
             self.color, self.radii, _, self.loss = self._run()
-        rs = self.batch.settings[0] if self.batch is not None else self.rast.raster_settings
-        key = (self.device.index, self.P, int(rs.image_height), int(rs.image_width))
-        self.capacity = R._captured_caps.get(key + ((self.batch.n_views,) if self.batch is not None else ()))
+        self.capacity = R.captured_capacity(self.device, self.P, *capacity_shape(self.rast))
 
     def __call__(self):
         if self.exchange is not None and self.exchange.generation != self._exchange_generation:

@@ -39,7 +39,7 @@ import torch
 
 from .rasterizer import RasterizerError
 from .sharding import GRAD_LAYOUT, GRAD_WIDTH, packed_backward
-from .views import ViewBatch, rasterize_views
+from .views import capacity_shape, render_params
 
 
 class HostStepPipeline:
@@ -259,15 +259,7 @@ class HostStepPipeline:
 
     def _compute(self, b: int, rast, dL: torch.Tensor) -> int:
         p = {k: v.requires_grad_(True) for k, v in self.views(self.dev_flat[b]).items()}
-        if isinstance(rast, ViewBatch):
-            color, radii, n = rasterize_views(rast, means3D=p["means3D"], opacities=p["opacities"],
-                                              colors_precomp=p["colors_precomp"], scales=p["scales"],
-                                              rotations=p["rotations"])
-        else:
-            means2D = torch.zeros_like(p["means3D"], requires_grad=True)
-            color, radii, n = rast(means3D=p["means3D"], means2D=means2D, shs=None,
-                                   colors_precomp=p["colors_precomp"], opacities=p["opacities"], scales=p["scales"],
-                                   rotations=p["rotations"], cov3D_precomp=None)
+        color, radii, n = render_params(rast, p)
         with packed_backward(self.dev_grads[b]):
             torch.autograd.grad(color, [p[k] for k, _ in GRAD_LAYOUT], grad_outputs=dL)
         return n
@@ -278,10 +270,7 @@ class HostStepPipeline:
         from . import rasterizer as R
         if R.overflow_events(self.device) > 0:
             return False
-        batch = rast if isinstance(rast, ViewBatch) else None
-        rs = batch.settings[0] if batch is not None else rast.raster_settings
-        return R.captured_capacity_ok(self.device, self.P, int(rs.image_height), int(rs.image_width),
-                                      batch.n_views if batch is not None else None)
+        return R.captured_capacity_ok(self.device, self.P, *capacity_shape(rast))
 
     def recapture(self) -> None:
         self.graphs = [None] * self.slots

@@ -10,6 +10,10 @@ Drop-in for `diff_gaussian_rasterization.cuda_ortho_gaussian_rasterizer` as GSVC
 All arithmetic happens in libgsvc_rast.so (hand-written sm_100a CUDA behind the C-ABI of
 include/gsvc_rast.h).  PyTorch only provides device memory, the current stream and autograd
 plumbing.  There is no CPU / eager fallback: CPU tensors raise.
+
+The drop-in call and views.rasterize_views share one autograd Function: a drop-in call is a batch of
+one view through the batched entry points (gsvc_rast_forward_views_launch, + gsvc_rast_forward_views_render
+on overflow; gsvc_rast_backward_views), the same kernels and buffer sizes as the single-view entry points.
 """
 from __future__ import annotations
 
@@ -22,7 +26,7 @@ import torch
 import torch.nn as nn
 
 from . import _lib
-from ._lib import RasterizerError, Settings
+from ._lib import RasterizerError, Settings, View
 
 
 class GaussianRasterizationSettings(NamedTuple):
@@ -43,9 +47,9 @@ class GaussianRasterizationSettings(NamedTuple):
 
 # Instance-capacity prediction, so that the binning buffer can be sized — and scatter / sort / blend launched — before
 # the instance count of THIS call is known (no mid-pipeline host synchronisation):
-#   _capacity_hint[(device, P, H, W[, V])]  the last num_rendered seen for exactly this shape (CUDA-graph capture
+#   _capacity_hint[(device, P, H, W, V)]    the last num_rendered seen for exactly this shape (CUDA-graph capture
 #                                           requires it: a replay's capacity is fixed);
-#   _density_hint[(device, H, W[, V])]      instances per INPUT Gaussian at this image size, a slowly decaying
+#   _density_hint[(device, H, W, V)]        instances per INPUT Gaussian at this image size, a slowly decaying
 #                                           maximum.  The reference's render() hands over a different P on every
 #                                           call (the Gaussians of the anchors visible in THAT view,
 #                                           ortho_gaussian_renderer/renderer.py:28-37), so an exact-shape hint never
@@ -57,6 +61,11 @@ _count_slots = threading.local()
 # how often the predicted capacity fell short and scatter / sort / blend had to be re-enqueued on a larger buffer
 # (eager calls only; bench.py reports it for the variable-P drop-in leg)
 capacity_stats = {"calls": 0, "rerendered": 0, "cold": 0}
+
+
+def _capacity_keys(dev: Optional[int], P: int, H: int, W: int, n_views: int):
+    """(exact-shape key, density key) of a call of `n_views` views on device index `dev`; a drop-in call is one view."""
+    return (dev, P, H, W, n_views), (dev, H, W, n_views)
 
 
 def _predict_capacity(key_exact, key_density, P: int):
@@ -87,12 +96,18 @@ def last_num_rendered() -> int:
     return int(st.slot[0].item()) & ((1 << 40) - 1) if hasattr(st, "slot") else 0
 
 
+def captured_capacity(device, P: int, H: int, W: int, n_views: Optional[int] = None) -> Optional[int]:
+    """The binning capacity the last CUDA-graph capture of this shape fixed (None: never captured).  `n_views`: for
+    a graph around views.rasterize_views; None is one view."""
+    key, _ = _capacity_keys(torch.device(device).index, P, H, W, 1 if n_views is None else n_views)
+    return _captured_caps.get(key)
+
+
 def captured_capacity_ok(device, P: int, H: int, W: int, n_views: Optional[int] = None) -> bool:
     """After replaying a CUDA graph that contains the rasterizer (and synchronizing): did the binning capacity
     fixed at capture time hold the instances of the last replay?  If not, the replay's image is invalid and
     the step must be re-captured (or run eagerly).  `n_views`: for a graph around views.rasterize_views."""
-    key = (torch.device(device).index, P, H, W) + (() if n_views is None else (n_views,))
-    cap = _captured_caps.get(key)
+    cap = captured_capacity(device, P, H, W, n_views)
     return cap is None or last_num_rendered() <= cap
 
 
@@ -115,19 +130,16 @@ class _PackedTarget:
     exchange = None        # sharding.SwitchAllReduce whose buffer `buf` is: the backward that takes buf carries the exchange
     lock = threading.Lock()
 
-    def take(self, P, device, ok: bool):
-        return self.take_with_exchange(P, device, ok)[0]
-
-    def take_with_exchange(self, P, device, ok: bool):
-        """(buffer or None, exchange or None).  A backward that cannot carry the exchange (single-view entry point)
-        calls take(): the exchange is then left to the caller (SwitchAllReduce.run())."""
+    def take_with_exchange(self, P, device, ok: bool, carry: bool = True):
+        """(buffer or None, exchange or None).  A backward that does not carry the exchange (`carry` False: a drop-in
+        call) takes only the buffer and leaves the exchange to the caller (SwitchAllReduce.run())."""
         with self.lock:
             b = self.buf
             if (b is None or self.taken or not ok or tuple(b.shape) != (P, 14) or b.device != device or
                     b.dtype != torch.float32 or not b.is_contiguous()):
                 return None, None
             self.taken = True
-            x = self.exchange
+            x = self.exchange if carry else None
             if x is not None:
                 x.fused_launches += 1
             return b, x
@@ -169,7 +181,9 @@ class _NativeSettings:
         self.bg, self.vm = bg, vm  # strides honoured natively: renderer.py:77 passes a permuted (non-contiguous) view
         campos = rs.campos
         if isinstance(campos, torch.Tensor):
-            campos = campos.detach().reshape(-1).tolist()  # frame.py:41: lives on the CPU
+            # frame.py:41: lives on the CPU.  flatten() of a 1-D tensor is the tensor itself: 0.6 us per drop-in
+            # call against 2 us for detach().reshape(-1)
+            campos = campos.flatten().tolist()
         s = Settings()
         s.image_height, s.image_width = int(rs.image_height), int(rs.image_width)
         s.x_min, s.y_min, s.scale = float(rs.x_min), float(rs.y_min), float(rs.scale)
@@ -182,6 +196,26 @@ class _NativeSettings:
         s.prefiltered, s.debug = int(bool(rs.prefiltered)), int(bool(rs.debug))
         self.c = s
         self.ref = C.byref(s)
+
+
+class _NativeViews:
+    """The shared settings struct + the gsvc_rast_view array of `batch` (a views.ViewBatch); keeps the tensors they
+    point into alive.  `batch` None: the single view of a drop-in call's settings `rs` (one image, not flipped,
+    weight 1), built without a ViewBatch."""
+
+    __slots__ = ("ns", "n_views", "n_out", "views", "ref")
+
+    def __init__(self, batch, device: torch.device, rs=None):
+        settings, out_image, flip_x, weight = (((rs,), (0,), (False,), (1.0,)) if batch is None else
+                                               (batch.settings, batch.out_image, batch.flip_x, batch.weight))
+        self.ns = [_NativeSettings(x, device) for x in settings]
+        self.n_views, self.n_out = len(self.ns), max(out_image) + 1
+        self.views = (View * self.n_views)()
+        for v, ns in enumerate(self.ns):
+            x, c = self.views[v], ns.c
+            x.viewmatrix, x.vm_stride_r, x.vm_stride_c, x.campos = c.viewmatrix, c.vm_stride_r, c.vm_stride_c, c.campos
+            x.out_image, x.flip_x, x.weight = out_image[v], 1 if flip_x[v] else 0, weight[v]
+        self.ref = self.ns[0].ref
 
 
 def _stream_ptr(device) -> int:
@@ -278,16 +312,38 @@ def _align(n: int) -> int:
     return (n + 255) & ~255
 
 
-class _RasterizeGaussians(torch.autograd.Function):
+def _check_modes(scales, rotations, cov3D_precomp, colours=None):
+    """Upstream's checks of which inputs a call was given; `colours` (shs, colors_precomp) of a render call."""
+    if colours is not None and (colours[0] is None) == (colours[1] is None):
+        raise Exception("Please provide excatly one of either SHs or precomputed colors!")
+    if ((scales is None or rotations is None) and cov3D_precomp is None) or \
+            ((scales is not None or rotations is not None) and cov3D_precomp is not None):
+        raise Exception("Please provide exactly one of either scale/rotation pair or precomputed 3D covariance!")
+
+
+def _snapshot_settings(rs, batch) -> tuple:
+    """The settings part of a debug snapshot: upstream's tuple(raster_settings) for a drop-in call, the views and
+    their image map for a batch."""
+    if batch is None:
+        return (tuple(rs),)
+    return ([tuple(x) for x in batch.settings], batch.out_image, batch.flip_x, batch.weight)
+
+
+class _RasterizeViews(torch.autograd.Function):
+    """One kernel chain over the views of `batch` (a views.ViewBatch), or over the single view `rs` of a drop-in call
+    (`batch` None).  A drop-in call differs in two things only: its outputs have upstream's shapes (image [3,H,W],
+    radii [P], means2D gradient [P,3]), and its backward never carries the exchange of sharding.packed_backward."""
+
     @staticmethod
-    def forward(ctx, means3D, means2D, sh, colors_precomp, opacities, scales, rotations, cov3Ds_precomp,
-                raster_settings):
+    def forward(ctx, means3D, means2D, sh, colors_precomp, opacities, scales, rotations, cov3Ds_precomp, rs, batch):
         L = _lib.lib()
         _require_cuda(means3D, "means3D")
         device = means3D.device
-        rs = raster_settings
+        single = batch is None
         with _on_device(device):
-            ns = _NativeSettings(rs, device)
+            # the reference builds new settings on every render(): the drop-in's descriptor is built per call
+            nv = _NativeViews(None, device, rs) if single else batch.native(device)
+            V, n_out = nv.n_views, nv.n_out
             P = means3D.shape[0]
             means3D_c = _dev_f32(means3D, device, "means3D")
             sh_c = _dev_f32(sh, device, "shs") if sh.numel() else None
@@ -300,7 +356,7 @@ class _RasterizeGaussians(torch.autograd.Function):
             sh_M = sh_c.shape[1] if sh_c is not None else 0
             H, W = int(rs.image_height), int(rs.image_width)
 
-            hint_key, dens_key = (device.index, P, H, W), (device.index, H, W)
+            hint_key, dens_key = _capacity_keys(device.index, P, H, W, V)
             cap, hint = _predict_capacity(hint_key, dens_key, P)
             # CUDA-graph capture (torch.cuda.graph around the caller's step): nothing may wait on the device, so
             # the instance count of the last eager call stands in for num_rendered and the binning capacity is
@@ -314,9 +370,9 @@ class _RasterizeGaussians(torch.autograd.Function):
                 _captured_caps[hint_key] = cap
             # one allocation for all native state: [geom | image | backward accumulators | binning]
             need_grad = any(ctx.needs_input_grad)
-            n_geom = _align(L.gsvc_rast_geom_bytes(P, sh_M))
-            n_img = _align(L.gsvc_rast_image_bytes(W, H))
-            n_acc = _align(L.gsvc_rast_backward_scratch_bytes(P)) if need_grad else 0
+            n_geom = _align(L.gsvc_rast_geom_bytes(P * V, sh_M))
+            n_img = _align(L.gsvc_rast_image_bytes_views(W, H, V))
+            n_acc = _align(L.gsvc_rast_backward_scratch_bytes(P * V)) if need_grad else 0
             n_bin = L.gsvc_rast_binning_bytes(cap) if cap > 0 else 0
             state = _bytes(n_geom + n_img + n_acc + n_bin, device)
             base = state.data_ptr()
@@ -324,16 +380,18 @@ class _RasterizeGaussians(torch.autograd.Function):
             acc_p = base + n_geom + n_img if need_grad else None   # zeroed by the preprocess kernel
             binning = None
             bin_p = base + n_geom + n_img + n_acc if cap > 0 else None
-            color = torch.empty((3, H, W), dtype=_F32, device=device)
-            radii = torch.empty((P,), dtype=torch.int32, device=device)
+            # outputs allocated in the caller's shape: indexing a batch of one would put a select node (and its
+            # image-sized zero fill) into every backward
+            color = torch.empty((3, H, W) if single else (n_out, 3, H, W), dtype=_F32, device=device)
+            radii = torch.empty((P,) if single else (V, P), dtype=torch.int32, device=device)
             stream = _stream_ptr(device)
             slot, ticket = _count_slot()
             try:
                 L.gsvc_rast_count_overflows(1 if capturing else 0)   # a replay has nobody to re-run it; eager does
-                _lib.check(L.gsvc_rast_forward_launch(
-                    ns.ref, P, sh_M, _ptr(means3D_c), _ptr(sh_c), _ptr(col_c), _ptr(op_c), _ptr(sc_c), _ptr(rot_c),
-                    _ptr(cov_c), geom_p, image_p, bin_p, cap, acc_p, color.data_ptr(), radii.data_ptr(), slot, ticket,
-                    stream), "gsvc_rast_forward_launch")
+                _lib.check(L.gsvc_rast_forward_views_launch(
+                    nv.ref, V, nv.views, n_out, P, sh_M, _ptr(means3D_c), _ptr(sh_c), _ptr(col_c), _ptr(op_c),
+                    _ptr(sc_c), _ptr(rot_c), _ptr(cov_c), geom_p, image_p, bin_p, cap, acc_p, color.data_ptr(),
+                    radii.data_ptr(), slot, ticket, stream), "gsvc_rast_forward_views_launch")
                 # The reference API returns num_rendered as a Python int (renderer.py:90).  The scan kernel
                 # publishes it into pinned memory as soon as it is known, so this wait ends while the
                 # scatter / sort / blend kernels are still running: no stream synchronisation.
@@ -351,22 +409,20 @@ class _RasterizeGaussians(torch.autograd.Function):
                     cap = max(num_rendered, 1)
                     binning = _bytes(L.gsvc_rast_binning_bytes(cap), device)
                     bin_p = binning.data_ptr()
-                    _lib.check(L.gsvc_rast_forward_render(ns.ref, P, geom_p, image_p, bin_p, cap, color.data_ptr(),
-                                                          stream), "gsvc_rast_forward_render")
+                    _lib.check(L.gsvc_rast_forward_views_render(nv.ref, V, nv.views, n_out, P, geom_p, image_p, bin_p,
+                                                                cap, color.data_ptr(), stream),
+                               "gsvc_rast_forward_views_render")
                 if not capturing:
                     _record_capacity(hint_key, dens_key, P, num_rendered)
             except Exception:
                 if rs.debug:
-                    torch.save((means3D, sh, colors_precomp, opacities, scales, rotations, cov3Ds_precomp,
-                                tuple(rs)), "snapshot_fw.dump")
+                    torch.save((means3D, sh, colors_precomp, opacities, scales, rotations, cov3Ds_precomp)
+                               + _snapshot_settings(rs, batch), "snapshot_fw.dump")
                     print("\nAn error occured in forward. Please forward snapshot_fw.dump for debugging.")
                 raise
 
-        ctx.raster_settings = rs
-        ctx.ns = ns
-        ctx.num_rendered = num_rendered
-        ctx.sh_M = sh_M
-        ctx.capacity = cap
+        ctx.rs, ctx.batch, ctx.nv = rs, batch, nv
+        ctx.sh_M, ctx.capacity = sh_M, cap
         ctx.offsets = (n_geom, n_img, n_acc)
         ctx.save_for_backward(means3D_c, sh_c, col_c, sc_c, rot_c, cov_c, radii, state, binning)
         ctx.mark_non_differentiable(radii)
@@ -375,7 +431,8 @@ class _RasterizeGaussians(torch.autograd.Function):
     @staticmethod
     def backward(ctx, grad_out_color, _grad_radii=None, _grad_num=None):
         L = _lib.lib()
-        rs = ctx.raster_settings
+        nv, single = ctx.nv, ctx.batch is None
+        V, n_out = nv.n_views, nv.n_out
         means3D, sh, col, sc, rot, cov, radii, state, binning = ctx.saved_tensors
         device = means3D.device
         P = means3D.shape[0]
@@ -383,15 +440,20 @@ class _RasterizeGaussians(torch.autograd.Function):
         base = state.data_ptr()
         bin_p = binning.data_ptr() if binning is not None else base + n_geom + n_img + n_acc
         with _on_device(device):
-            ns = ctx.ns
             g_out = _dev_f32(grad_out_color, device, "grad_out_color")
             # frame-sharded training: write (means3D, colours, opacity, scales, rotation) gradients straight into
-            # the caller's [P,14] all-reduce buffer (gsvc_b200.sharding.packed_backward) and return views of it
-            packed = _packed_target.take(P, device, col is not None and sc is not None)
+            # the caller's [P,14] all-reduce buffer (gsvc_b200.sharding.packed_backward) and return views of it.  A
+            # drop-in backward takes the buffer only: packed_backward leaves that buffer un-reduced for the caller's
+            # exchange.run(), so carrying the exchange too would sum it twice.
+            packed, exchange = _packed_target.take_with_exchange(P, device, col is not None and sc is not None,
+                                                                 carry=not single)
+            if exchange is not None and (P % 2 or sh is not None or cov is not None):
+                raise RasterizerError("a backward that carries the exchange needs an even P, colors_precomp and the "
+                                      "scale / rotation pair")
             # one allocation for every gradient (contiguous slices) and the accumulator scratch
-            widths = (3, 3, 1, 3 if col is not None else 0, ctx.sh_M * 3 if sh is not None else 0,
+            widths = (3, 3 * V, 1, 3 if col is not None else 0, ctx.sh_M * 3 if sh is not None else 0,
                       3 if sc is not None else 0, 4 if rot is not None else 0, 6 if cov is not None else 0)
-            n_scratch = 0 if n_acc else L.gsvc_rast_backward_scratch_bytes(P) // 4
+            n_scratch = 0 if n_acc else L.gsvc_rast_backward_scratch_bytes(P * V) // 4
             # the accumulators inside the forward state were zeroed by the preprocess kernel; a backward
             # dirties them, so a second backward over the same graph (retain_graph) asks for a clear
             acc_clean = 1 if (n_acc and not getattr(ctx, "acc_dirty", False)) else 0
@@ -405,28 +467,52 @@ class _RasterizeGaussians(torch.autograd.Function):
             scratch_p = base + n_geom + n_img if n_acc else flat.data_ptr() + 4 * off
             g_means3D, g_means2D, g_opac, g_col, g_sh, g_sc, g_rot, g_cov = outs
             try:
-                _lib.check(L.gsvc_rast_backward(
-                    ns.ref, P, ctx.sh_M, ctx.capacity, _ptr(means3D), _ptr(sh), _ptr(col), _ptr(sc), _ptr(rot),
-                    _ptr(cov), _ptr(radii), base, base + n_geom, bin_p, scratch_p, acc_clean, _ptr(g_out),
-                    _ptr(g_means3D), _ptr(g_means2D), _ptr(g_col), _ptr(g_opac), _ptr(g_sc), _ptr(g_rot),
-                    _ptr(g_cov), _ptr(g_sh), _ptr(packed), _stream_ptr(device)), "gsvc_rast_backward")
+                if exchange is not None:
+                    _lib.check(L.gsvc_rast_backward_views_exchange(
+                        nv.ref, V, nv.views, n_out, P, ctx.sh_M, ctx.capacity, _ptr(means3D), _ptr(sh), _ptr(col),
+                        _ptr(sc), _ptr(rot), _ptr(cov), _ptr(radii), base, base + n_geom, bin_p, scratch_p, acc_clean,
+                        _ptr(g_out), _ptr(g_means2D), _ptr(packed), C.byref(exchange.exchange_struct()),
+                        _stream_ptr(device)), "gsvc_rast_backward_views_exchange")
+                else:
+                    _lib.check(L.gsvc_rast_backward_views(
+                        nv.ref, V, nv.views, n_out, P, ctx.sh_M, ctx.capacity, _ptr(means3D), _ptr(sh), _ptr(col),
+                        _ptr(sc), _ptr(rot), _ptr(cov), _ptr(radii), base, base + n_geom, bin_p, scratch_p, acc_clean,
+                        _ptr(g_out), _ptr(g_means3D), _ptr(g_means2D), _ptr(g_col), _ptr(g_opac), _ptr(g_sc),
+                        _ptr(g_rot), _ptr(g_cov), _ptr(g_sh), _ptr(packed), _stream_ptr(device)),
+                        "gsvc_rast_backward_views")
             except Exception:
-                if rs.debug:
-                    torch.save((means3D, sh, col, sc, rot, cov, radii, grad_out_color, tuple(rs)), "snapshot_bw.dump")
+                if ctx.rs.debug:
+                    torch.save((means3D, sh, col, sc, rot, cov, radii, grad_out_color)
+                               + _snapshot_settings(ctx.rs, ctx.batch), "snapshot_bw.dump")
                     print("\nAn error occured in backward. Writing snapshot_bw.dump for debugging.\n")
                 raise
         v = lambda t, *shape: None if t is None else t.view(*shape)
+        m2d = (P, 3) if single else (V, P, 3)
         if packed is not None:
-            return (packed[:, 0:3], v(g_means2D, P, 3), None, packed[:, 3:6], packed[:, 6:7], packed[:, 7:10],
-                    packed[:, 10:14], None, None)
-        return (v(g_means3D, P, 3), v(g_means2D, P, 3), v(g_sh, P, ctx.sh_M, 3), v(g_col, P, 3), v(g_opac, P, 1),
-                v(g_sc, P, 3), v(g_rot, P, 4), v(g_cov, P, 6), None)
+            return (packed[:, 0:3], v(g_means2D, *m2d), None, packed[:, 3:6], packed[:, 6:7], packed[:, 7:10],
+                    packed[:, 10:14], None, None, None)
+        return (v(g_means3D, P, 3), v(g_means2D, *m2d), v(g_sh, P, ctx.sh_M, 3), v(g_col, P, 3), v(g_opac, P, 1),
+                v(g_sc, P, 3), v(g_rot, P, 4), v(g_cov, P, 6), None, None)
+
+
+# upstream passes an absent input to rasterize_gaussians as torch.Tensor([]); one shared instance, never written,
+# saves building one (2 us) per call
+_EMPTY = torch.Tensor([])
+
+
+def _rasterize(rs, batch, means3D, means2D, opacities, shs, colors_precomp, scales, rotations, cov3D_precomp):
+    """GaussianRasterizer.forward / views.rasterize_views: upstream's input checks, then absent inputs as the empty
+    tensor upstream's rasterize_gaussians takes."""
+    _check_modes(scales, rotations, cov3D_precomp, (shs, colors_precomp))
+    opt = lambda t: _EMPTY if t is None else t
+    return _RasterizeViews.apply(means3D, opt(means2D), opt(shs), opt(colors_precomp), opacities, opt(scales),
+                                 opt(rotations), opt(cov3D_precomp), rs, batch)
 
 
 def rasterize_gaussians(means3D, means2D, sh, colors_precomp, opacities, scales, rotations, cov3Ds_precomp,
                         raster_settings):
-    return _RasterizeGaussians.apply(means3D, means2D, sh, colors_precomp, opacities, scales, rotations,
-                                     cov3Ds_precomp, raster_settings)
+    return _RasterizeViews.apply(means3D, means2D, sh, colors_precomp, opacities, scales, rotations, cov3Ds_precomp,
+                                 raster_settings, None)
 
 
 class GaussianRasterizer(nn.Module):
@@ -434,26 +520,31 @@ class GaussianRasterizer(nn.Module):
         super().__init__()
         self.raster_settings = raster_settings
 
+    def _filter_inputs(self, means3D, scales, rotations, cov3D_precomp):
+        """Checked and converted inputs of the visibility filters: (native settings, P, means3D, scales, rotations,
+        cov3D_precomp)."""
+        _check_modes(scales, rotations, cov3D_precomp)
+        _require_cuda(means3D, "means3D")
+        device = means3D.device
+        ns = _NativeSettings(self.raster_settings, device)
+        P = int(means3D.shape[0])
+        m = _dev_f32(means3D, device, "means3D")
+        s = _dev_f32(scales, device, "scales")
+        r = _dev_f32(rotations, device, "rotations")
+        c = _dev_f32(cov3D_precomp, device, "cov3D_precomp")
+        _check_shapes(P, 0, m, scales=s, rotations=r, cov=c)
+        return ns, P, m, s, r, c
+
     def visible_filter(self, means3D, scales=None, rotations=None, cov3D_precomp=None, index_range=None):
         """preprocess.py:99-104 — radii[P] int32 (> 0 where the anchor survives the TSW slab and image culls).
 
         `index_range=(lo, hi)` (slab-ordered anchors, SURVEY.md §8f row f4): the caller promises that anchors outside
         [lo, hi) are outside the TSW slab (frames.slab_index_range computes it from a z-interval table like the
         stream codec's, utils/encodings.py:827-862); they get radius 0 without being read."""
-        rs = self.raster_settings
-        if (scales is None or rotations is None) == (cov3D_precomp is None):
-            raise Exception("Please provide exactly one of either scale/rotation pair or precomputed 3D covariance!")
         L = _lib.lib()
-        _require_cuda(means3D, "means3D")
         device = means3D.device
-        with torch.no_grad(), torch.cuda.device(device):
-            ns = _NativeSettings(rs, device)
-            P = int(means3D.shape[0])
-            m = _dev_f32(means3D, device, "means3D")
-            s = _dev_f32(scales, device, "scales")
-            r = _dev_f32(rotations, device, "rotations")
-            c = _dev_f32(cov3D_precomp, device, "cov3D_precomp")
-            _check_shapes(P, 0, m, scales=s, rotations=r, cov=c)
+        with torch.no_grad(), _on_device(device):
+            ns, P, m, s, r, c = self._filter_inputs(means3D, scales, rotations, cov3D_precomp)
             radii = torch.empty((P,), dtype=torch.int32, device=device)
             lo, hi = self._index_range(index_range, P)
             if index_range is not None and lo == hi:
@@ -480,20 +571,10 @@ class GaussianRasterizer(nn.Module):
         the same kernel also writes the ascending indices of the visible anchors and publishes their count to
         pinned memory, so the caller gets `idx` (int32, == nonzero(radii > 0)) without synchronising the stream and
         gathers with `anchor.index_select(0, idx)` / `anchor[idx]`.  Returns (idx [count], radii [P] or None)."""
-        rs = self.raster_settings
-        if (scales is None or rotations is None) == (cov3D_precomp is None):
-            raise Exception("Please provide exactly one of either scale/rotation pair or precomputed 3D covariance!")
         L = _lib.lib()
-        _require_cuda(means3D, "means3D")
         device = means3D.device
-        with torch.no_grad(), torch.cuda.device(device):
-            ns = _NativeSettings(rs, device)
-            P = int(means3D.shape[0])
-            m = _dev_f32(means3D, device, "means3D")
-            s = _dev_f32(scales, device, "scales")
-            r = _dev_f32(rotations, device, "rotations")
-            c = _dev_f32(cov3D_precomp, device, "cov3D_precomp")
-            _check_shapes(P, 0, m, scales=s, rotations=r, cov=c)
+        with torch.no_grad(), _on_device(device):
+            ns, P, m, s, r, c = self._filter_inputs(means3D, scales, rotations, cov3D_precomp)
             radii = torch.empty((P,), dtype=torch.int32, device=device) if want_radii else None
             idx = torch.empty((P,), dtype=torch.int32, device=device)
             scratch = _bytes(L.gsvc_rast_compact_scratch_bytes(P), device)
@@ -510,20 +591,8 @@ class GaussianRasterizer(nn.Module):
 
     def forward(self, means3D, means2D, opacities, shs=None, colors_precomp=None, scales=None, rotations=None,
                 cov3D_precomp=None):
-        rs = self.raster_settings
-        if (shs is None and colors_precomp is None) or (shs is not None and colors_precomp is not None):
-            raise Exception("Please provide excatly one of either SHs or precomputed colors!")
-        if ((scales is None or rotations is None) and cov3D_precomp is None) or \
-                ((scales is not None or rotations is not None) and cov3D_precomp is not None):
-            raise Exception("Please provide exactly one of either scale/rotation pair or precomputed 3D covariance!")
-        empty = torch.Tensor([])
-        shs = empty if shs is None else shs
-        colors_precomp = empty if colors_precomp is None else colors_precomp
-        scales = empty if scales is None else scales
-        rotations = empty if rotations is None else rotations
-        cov3D_precomp = empty if cov3D_precomp is None else cov3D_precomp
-        return rasterize_gaussians(means3D, means2D, shs, colors_precomp, opacities, scales, rotations,
-                                   cov3D_precomp, rs)
+        return _rasterize(self.raster_settings, None, means3D, means2D, opacities, shs, colors_precomp, scales,
+                          rotations, cov3D_precomp)
 
 
 class RasterState:

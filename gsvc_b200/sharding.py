@@ -48,8 +48,8 @@ def packed_backward(buf: torch.Tensor, exchange=None):
     then CARRIES the all-reduce: the first CTAs of its per-Gaussian kernel sum the rows over the ranks chunk by chunk
     while the others still compute (gsvc_rast_backward_views_exchange), and the buffer holds the sum over the ranks
     when the backward's kernels have run — no separate collective launch.  Every rank must run the same backward;
-    `exchange.fused_launches` counts the launches that carried it (a backward that could not — a single-view call — leaves
-    the buffer un-reduced: call exchange.run())."""
+    `exchange.fused_launches` counts the launches that carried it (a backward that does not — a GaussianRasterizer call —
+    leaves the buffer un-reduced: call exchange.run())."""
     from . import rasterizer
     t = rasterizer._packed_target
     if exchange is not None and (buf.data_ptr() != exchange.buffer().data_ptr() or buf.numel() != exchange.numel):

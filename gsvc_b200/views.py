@@ -16,7 +16,9 @@ flip + average is folded into the blend's epilogue / the backward's prologue.
                                        scales=..., rotations=...)               # images [2,3,H,W]
     image, radii, n = render_toast(front, back, means3D=..., ...)               # (img_f + flip(img_b)) / 2
 
-Semantics per view are exactly those of `GaussianRasterizer` (same kernels, batch of one).
+Semantics per view are exactly those of `GaussianRasterizer`: both go through the one autograd Function of
+rasterizer.py and the gsvc_rast_*_views entry points, a `GaussianRasterizer` call being a batch of one.
+This module keeps the batch itself (ViewBatch: validation, the image map, its cached native descriptor).
 There is no CPU fallback.
 """
 from __future__ import annotations
@@ -26,13 +28,9 @@ from typing import Optional, Sequence
 
 import torch
 
-from . import _lib
-from ._lib import MAX_VIEWS, RasterizerError, View
-from . import rasterizer as R
-from .rasterizer import (GaussianRasterizationSettings, _NativeSettings, _align, _bytes, _check_shapes, _count_slot,
-                         _dev_f32, _ptr, _require_cuda, _stream_ptr)
+from ._lib import MAX_VIEWS, RasterizerError
+from .rasterizer import GaussianRasterizationSettings, _NativeViews, _rasterize
 
-_F32 = torch.float32
 _SHARED_FIELDS = ("image_height", "image_width", "x_min", "y_min", "scale", "threshold", "scale_modifier", "sh_degree")
 
 
@@ -117,158 +115,6 @@ class ViewBatch:
         return cls(settings, out_image=out, flip_x=flip, weight=w)
 
 
-class _NativeViews:
-    """The shared settings struct + the gsvc_rast_view array; keeps the tensors they point into alive."""
-
-    def __init__(self, batch: ViewBatch, device: torch.device):
-        self.ns = [_NativeSettings(rs, device) for rs in batch.settings]
-        self.common = self.ns[0]
-        arr = (View * batch.n_views)()
-        for v, ns in enumerate(self.ns):
-            c = ns.c
-            arr[v].viewmatrix = c.viewmatrix
-            arr[v].vm_stride_r, arr[v].vm_stride_c = c.vm_stride_r, c.vm_stride_c
-            arr[v].campos[0], arr[v].campos[1], arr[v].campos[2] = c.campos[0], c.campos[1], c.campos[2]
-            arr[v].out_image = batch.out_image[v]
-            arr[v].flip_x = 1 if batch.flip_x[v] else 0
-            arr[v].weight = batch.weight[v]
-        self.views = arr
-        self.ref = self.common.ref
-
-
-class _RasterizeViews(torch.autograd.Function):
-    @staticmethod
-    def forward(ctx, means3D, means2D, sh, colors_precomp, opacities, scales, rotations, cov3Ds_precomp, batch):
-        L = _lib.lib()
-        _require_cuda(means3D, "means3D")
-        device = means3D.device
-        rs = batch.settings[0]
-        V, n_out = batch.n_views, batch.n_out
-        with torch.cuda.device(device):
-            nv = batch.native(device)
-            P = means3D.shape[0]
-            means3D_c = _dev_f32(means3D, device, "means3D")
-            sh_c = _dev_f32(sh, device, "shs") if sh.numel() else None
-            col_c = _dev_f32(colors_precomp, device, "colors_precomp") if colors_precomp.numel() else None
-            op_c = _dev_f32(opacities, device, "opacities")
-            sc_c = _dev_f32(scales, device, "scales") if scales.numel() else None
-            rot_c = _dev_f32(rotations, device, "rotations") if rotations.numel() else None
-            cov_c = _dev_f32(cov3Ds_precomp, device, "cov3D_precomp") if cov3Ds_precomp.numel() else None
-            _check_shapes(int(P), rs.sh_degree, means3D_c, sh_c, col_c, op_c, sc_c, rot_c, cov_c)
-            sh_M = sh_c.shape[1] if sh_c is not None else 0
-            H, W = int(rs.image_height), int(rs.image_width)
-
-            hint_key, dens_key = (device.index, P, H, W, V), (device.index, H, W, V)
-            cap, hint = R._predict_capacity(hint_key, dens_key, P)
-            capturing = torch.cuda.is_current_stream_capturing()
-            if capturing:
-                if hint is None:
-                    raise RasterizerError("run rasterize_views once eagerly with these shapes before capturing it in "
-                                          "a CUDA graph (the binning capacity comes from that call)")
-                cap = int(hint * 1.5) + 65536
-                R._captured_caps[hint_key] = cap
-            need_grad = any(ctx.needs_input_grad)
-            n_geom = _align(L.gsvc_rast_geom_bytes(P * V, sh_M))
-            n_img = _align(L.gsvc_rast_image_bytes_views(W, H, V))
-            n_acc = _align(L.gsvc_rast_backward_scratch_bytes(P * V)) if need_grad else 0
-            n_bin = L.gsvc_rast_binning_bytes(cap) if cap > 0 else 0
-            state = _bytes(n_geom + n_img + n_acc + n_bin, device)
-            base = state.data_ptr()
-            geom_p, image_p = base, base + n_geom
-            acc_p = base + n_geom + n_img if need_grad else None
-            binning = None
-            bin_p = base + n_geom + n_img + n_acc if cap > 0 else None
-            color = torch.empty((n_out, 3, H, W), dtype=_F32, device=device)
-            radii = torch.empty((V, P), dtype=torch.int32, device=device)
-            stream = _stream_ptr(device)
-            slot, ticket = _count_slot()
-            try:
-                L.gsvc_rast_count_overflows(1 if capturing else 0)   # a replay has nobody to re-run it; eager does
-                _lib.check(L.gsvc_rast_forward_views_launch(
-                    nv.ref, V, nv.views, n_out, P, sh_M, _ptr(means3D_c), _ptr(sh_c), _ptr(col_c), _ptr(op_c), _ptr(sc_c),
-                    _ptr(rot_c), _ptr(cov_c), geom_p, image_p, bin_p, cap, acc_p, color.data_ptr(), radii.data_ptr(), slot,
-                    ticket, stream), "gsvc_rast_forward_views_launch")
-                if capturing:
-                    num_rendered = hint
-                else:
-                    num_rendered = _lib.check(L.gsvc_rast_wait_count(slot, ticket, stream), "gsvc_rast_wait_count")
-                if num_rendered > 0xFFFFFFFF:
-                    raise RasterizerError(f"num_rendered {num_rendered} exceeds 32-bit tile ranges")
-                if num_rendered > cap or cap == 0:
-                    cap = max(num_rendered, 1)
-                    binning = _bytes(L.gsvc_rast_binning_bytes(cap), device)
-                    bin_p = binning.data_ptr()
-                    _lib.check(L.gsvc_rast_forward_views_render(nv.ref, V, nv.views, n_out, P, geom_p, image_p, bin_p, cap,
-                                                                color.data_ptr(), stream), "gsvc_rast_forward_views_render")
-                if not capturing:
-                    R._record_capacity(hint_key, dens_key, P, num_rendered)
-
-            except Exception:
-                if rs.debug:   # upstream behaviour of the single-view call (snapshot for debugging)
-                    torch.save((means3D, sh, colors_precomp, opacities, scales, rotations, cov3Ds_precomp,
-                                [tuple(x) for x in batch.settings], batch.out_image, batch.flip_x, batch.weight),
-                               "snapshot_fw.dump")
-                    print("\nAn error occured in forward. Please forward snapshot_fw.dump for debugging.")
-                raise
-
-        ctx.batch, ctx.nv = batch, nv
-        ctx.num_rendered, ctx.sh_M, ctx.capacity = num_rendered, sh_M, cap
-        ctx.offsets = (n_geom, n_img, n_acc)
-        ctx.save_for_backward(means3D_c, sh_c, col_c, sc_c, rot_c, cov_c, radii, state, binning)
-        ctx.mark_non_differentiable(radii)
-        return color, radii, num_rendered
-
-    @staticmethod
-    def backward(ctx, grad_out_color, _grad_radii=None, _grad_num=None):
-        L = _lib.lib()
-        batch, nv = ctx.batch, ctx.nv
-        V, n_out = batch.n_views, batch.n_out
-        means3D, sh, col, sc, rot, cov, radii, state, binning = ctx.saved_tensors
-        device = means3D.device
-        P = means3D.shape[0]
-        n_geom, n_img, n_acc = ctx.offsets
-        base = state.data_ptr()
-        bin_p = binning.data_ptr() if binning is not None else base + n_geom + n_img + n_acc
-        with torch.cuda.device(device):
-            g_out = _dev_f32(grad_out_color, device, "grad_out_color")
-            packed, exchange = R._packed_target.take_with_exchange(P, device, col is not None and sc is not None)
-            if exchange is not None and (P % 2 or sh is not None or cov is not None):
-                raise RasterizerError("a backward that carries the exchange needs an even P, colors_precomp and the "
-                                      "scale / rotation pair")
-            widths = (3, 3 * V, 1, 3 if col is not None else 0, ctx.sh_M * 3 if sh is not None else 0,
-                      3 if sc is not None else 0, 4 if rot is not None else 0, 6 if cov is not None else 0)
-            n_scratch = 0 if n_acc else L.gsvc_rast_backward_scratch_bytes(P * V) // 4
-            acc_clean = 1 if (n_acc and not getattr(ctx, "acc_dirty", False)) else 0
-            ctx.acc_dirty = True
-            flat = torch.empty((sum(widths) * P + n_scratch + 64 + 4 * len(widths),), dtype=_F32, device=device)
-            outs, off = [], 0
-            for w in widths:
-                outs.append(flat[off:off + w * P] if w else None)
-                off = (off + w * P + 3) & ~3
-            off = (off + 63) & ~63
-            scratch_p = base + n_geom + n_img if n_acc else flat.data_ptr() + 4 * off
-            g_means3D, g_means2D, g_opac, g_col, g_sh, g_sc, g_rot, g_cov = outs
-            if exchange is not None:
-                import ctypes
-                _lib.check(L.gsvc_rast_backward_views_exchange(
-                    nv.ref, V, nv.views, n_out, P, ctx.sh_M, ctx.capacity, _ptr(means3D), _ptr(sh), _ptr(col), _ptr(sc),
-                    _ptr(rot), _ptr(cov), _ptr(radii), base, base + n_geom, bin_p, scratch_p, acc_clean, _ptr(g_out),
-                    _ptr(g_means2D), _ptr(packed), ctypes.byref(exchange.exchange_struct()), _stream_ptr(device)),
-                    "gsvc_rast_backward_views_exchange")
-            else:
-                _lib.check(L.gsvc_rast_backward_views(
-                    nv.ref, V, nv.views, n_out, P, ctx.sh_M, ctx.capacity, _ptr(means3D), _ptr(sh), _ptr(col), _ptr(sc),
-                    _ptr(rot), _ptr(cov), _ptr(radii), base, base + n_geom, bin_p, scratch_p, acc_clean, _ptr(g_out),
-                    _ptr(g_means3D), _ptr(g_means2D), _ptr(g_col), _ptr(g_opac), _ptr(g_sc), _ptr(g_rot), _ptr(g_cov),
-                    _ptr(g_sh), _ptr(packed), _stream_ptr(device)), "gsvc_rast_backward_views")
-        v = lambda t, *shape: None if t is None else t.view(*shape)
-        if packed is not None:
-            return (packed[:, 0:3], v(g_means2D, V, P, 3), None, packed[:, 3:6], packed[:, 6:7], packed[:, 7:10],
-                    packed[:, 10:14], None, None)
-        return (v(g_means3D, P, 3), v(g_means2D, V, P, 3), v(g_sh, P, ctx.sh_M, 3), v(g_col, P, 3), v(g_opac, P, 1),
-                v(g_sc, P, 3), v(g_rot, P, 4), v(g_cov, P, 6), None)
-
-
 def rasterize_views(views, means3D, opacities, means2D=None, shs=None, colors_precomp=None, scales=None,
                     rotations=None, cov3D_precomp=None):
     """Rasterize every view of `views` (a ViewBatch, or a sequence of GaussianRasterizationSettings = one image
@@ -278,21 +124,11 @@ def rasterize_views(views, means3D, opacities, means2D=None, shs=None, colors_pr
     Differentiable like GaussianRasterizer; parameter gradients are summed over the views.  `means2D`
     (optional, [n_views,P,3], requires_grad) receives each view's screen-space gradient (columns 0,1)."""
     batch = views if isinstance(views, ViewBatch) else ViewBatch(list(views))
-    if (shs is None) == (colors_precomp is None):
-        raise Exception("Please provide excatly one of either SHs or precomputed colors!")
-    if ((scales is None or rotations is None) and cov3D_precomp is None) or \
-            ((scales is not None or rotations is not None) and cov3D_precomp is not None):
-        raise Exception("Please provide exactly one of either scale/rotation pair or precomputed 3D covariance!")
-    empty = torch.Tensor([])
-    if means2D is None:
-        means2D = empty
-    elif tuple(means2D.shape) != (batch.n_views, means3D.shape[0], 3):
+    if means2D is not None and tuple(means2D.shape) != (batch.n_views, means3D.shape[0], 3):
         raise RasterizerError(f"means2D must be [n_views, P, 3] = {(batch.n_views, means3D.shape[0], 3)}, "
                               f"got {tuple(means2D.shape)}")
-    return _RasterizeViews.apply(means3D, means2D, empty if shs is None else shs,
-                                 empty if colors_precomp is None else colors_precomp, opacities,
-                                 empty if scales is None else scales, empty if rotations is None else rotations,
-                                 empty if cov3D_precomp is None else cov3D_precomp, batch)
+    return _rasterize(batch.settings[0], batch, means3D, means2D, opacities, shs, colors_precomp, scales, rotations,
+                      cov3D_precomp)
 
 
 def render_toast(front: GaussianRasterizationSettings, back: GaussianRasterizationSettings, means3D, opacities,
@@ -300,3 +136,23 @@ def render_toast(front: GaussianRasterizationSettings, back: GaussianRasterizati
     """One frame as the reference composes it (train.py:353-375): (front + flip_x(back)) / 2 → [3,H,W]."""
     images, radii, n = rasterize_views(ViewBatch.toast(front, back), means3D, opacities, **kw)
     return images[0], radii, n
+
+
+def render_params(rast, p, means2D=None):
+    """Render the GRAD_LAYOUT parameter dict `p` with a GaussianRasterizer (one view) or a ViewBatch (all its views in
+    one chain): (color, radii, num_rendered).  `means2D`: the GaussianRasterizer call's screen-space tensor, zeros by
+    default; a ViewBatch call takes none."""
+    if isinstance(rast, ViewBatch):
+        return rasterize_views(rast, means3D=p["means3D"], opacities=p["opacities"], colors_precomp=p["colors_precomp"],
+                               scales=p["scales"], rotations=p["rotations"])
+    if means2D is None:
+        means2D = torch.zeros_like(p["means3D"], requires_grad=True)
+    return rast(means3D=p["means3D"], means2D=means2D, shs=None, colors_precomp=p["colors_precomp"],
+                opacities=p["opacities"], scales=p["scales"], rotations=p["rotations"], cov3D_precomp=None)
+
+
+def capacity_shape(rast):
+    """(H, W, n_views) of a GaussianRasterizer (one view) or a ViewBatch: the shape rasterizer.captured_capacity
+    takes after P."""
+    rs, n_views = (rast.settings[0], rast.n_views) if isinstance(rast, ViewBatch) else (rast.raster_settings, 1)
+    return int(rs.image_height), int(rs.image_width), n_views

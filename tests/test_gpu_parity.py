@@ -453,6 +453,20 @@ def test_heavy_tile_after_an_overflowed_first_attempt(cuda_device):
         assert n == fo["num_rendered"]
         np.testing.assert_array_equal(radii.cpu().numpy(), fo["radii"])
         _check_forward(fo, color, max_fragile=5e-3)
+    # a batched call re-renders the same way, and is counted too
+    from gsvc_b200.views import rasterize_views
+    R._capacity_hint.clear(); R._density_hint.clear()
+    for sc in (small, scene):
+        g = _to_dev(sc["gaussians"], cuda_device)
+        before = R.capacity_stats["rerendered"]
+        images, radii, n = rasterize_views([product_settings(sc, cuda_device)] * 2, means3D=g["means3D"],
+                                           opacities=g["opacities"], colors_precomp=g["colors_precomp"],
+                                           scales=g["scales"], rotations=g["rotations"])
+    assert R.capacity_stats["rerendered"] == before + 1, "the batched attempt was meant to overflow"
+    assert n == 2 * fo["num_rendered"]
+    for v in range(2):
+        np.testing.assert_array_equal(radii[v].cpu().numpy(), fo["radii"])
+        _check_forward(fo, images[v], max_fragile=5e-3)
 
 
 def test_toast_two_view_composition(cuda_device):
@@ -469,24 +483,39 @@ def test_toast_two_view_composition(cuda_device):
 
 
 def test_packed_backward_writes_the_allreduce_buffer(cuda_device):
-    """sharding.packed_backward: the [P,14] buffer receives exactly the gradients the dense outputs carry."""
+    """sharding.packed_backward: the [P,14] buffer receives exactly the gradients the dense outputs carry.  Given an
+    exchange, a GaussianRasterizer backward still fills the buffer un-reduced and leaves the exchange to the caller
+    (exchange.run()): it must not count as a launch that carried it."""
     from gsvc_b200 import sharding
+
+    class FakeExchange:                      # what packed_backward reads of a SwitchAllReduce
+        def __init__(self, P):
+            self.t = torch.full((P * 14,), float("nan"), device=cuda_device)
+            self.numel = P * 14
+            self.fused_launches = 0
+
+        def buffer(self):
+            return self.t
+
     scene = make_scene(P=9000, W=160, H=96, F=160, seed=23)
     g, m2d, color, radii, n = _run_product(scene, cuda_device)
     dL = torch.randn(color.shape, generator=torch.Generator().manual_seed(4)).to(cuda_device)
     names = [k for k, _ in sharding.GRAD_LAYOUT]
     dense = torch.autograd.grad(color, [g[k] for k in names], grad_outputs=dL, retain_graph=True)
-    buf = torch.full((9000, 14), float("nan"), device=cuda_device)
-    with sharding.packed_backward(buf):
-        views = torch.autograd.grad(color, [g[k] for k in names] + [m2d], grad_outputs=dL)
     ref = sharding.pack_grads({k: d for k, d in zip(names, dense)})
-    # two backward passes differ in the order of the fp32 atomics, so compare to rounding, not bitwise
-    assert not torch.isnan(buf).any()
-    assert (buf - ref).abs().max() <= ATOMIC_RTOL * ref.abs().max()
-    unpacked = sharding.unpack_grads(buf)
-    for k, v, d in zip(names, views, dense):
-        assert v.shape == d.shape and torch.equal(v, unpacked[k].reshape(d.shape))   # views of the buffer itself
-    assert views[-1].shape == (9000, 3)
+    x = FakeExchange(9000)
+    for exchange in (None, x):
+        buf = x.buffer().view(9000, 14) if exchange else torch.full((9000, 14), float("nan"), device=cuda_device)
+        with sharding.packed_backward(buf, exchange=exchange):
+            views = torch.autograd.grad(color, [g[k] for k in names] + [m2d], grad_outputs=dL, retain_graph=True)
+        # two backward passes differ in the order of the fp32 atomics, so compare to rounding, not bitwise
+        assert not torch.isnan(buf).any()
+        assert (buf - ref).abs().max() <= ATOMIC_RTOL * ref.abs().max()
+        unpacked = sharding.unpack_grads(buf)
+        for k, v, d in zip(names, views, dense):
+            assert v.shape == d.shape and torch.equal(v, unpacked[k].reshape(d.shape))   # views of the buffer itself
+        assert views[-1].shape == (9000, 3)
+    assert x.fused_launches == 0
 
 
 def test_large_gaussians_nonzero_bg_scale_modifier_and_debug(cuda_device):

@@ -40,12 +40,16 @@ def _leaves(scene, device):
 
 
 def _single(scene, device, p, dL):
-    from gsvc_b200.rasterizer import GaussianRasterizer
+    from gsvc_b200.rasterizer import GaussianRasterizer, _RasterizeViews
     rast = GaussianRasterizer(raster_settings=product_settings(scene, device))
     m2d = torch.zeros_like(p["means3D"], requires_grad=True)
     color, radii, n = rast(means3D=p["means3D"], means2D=m2d, shs=None, colors_precomp=p["colors_precomp"],
                            opacities=p["opacities"], scales=p["scales"], rotations=p["rotations"], cov3D_precomp=None)
+    # the drop-in's outputs come in upstream's shapes straight from the Function: no select / index node in between
+    assert type(color.grad_fn) is _RasterizeViews._backward_cls
+    assert color.shape == (3,) + tuple(dL.shape[-2:]) and radii.shape == (p["means3D"].shape[0],)
     grads = torch.autograd.grad(color, [p[k] for k in NAMES] + [m2d], grad_outputs=dL)
+    assert grads[-1].shape == m2d.shape
     return color, radii, n, grads
 
 
@@ -75,6 +79,16 @@ def test_batched_views_equal_single_calls(cuda_device, W, H):
     assert n == total
     for k, a, b in zip(NAMES, grads[:-1], sums):
         assert (a - b).abs().max() <= ATOMIC_RTOL * b.abs().max(), k
+    # a batch of one view is the drop-in call
+    m2d1 = torch.zeros((1, P, 3), device=cuda_device, requires_grad=True)
+    images1, radii1, n1 = rasterize_views(settings[:1], means3D=p["means3D"], opacities=p["opacities"], means2D=m2d1,
+                                          colors_precomp=p["colors_precomp"], scales=p["scales"],
+                                          rotations=p["rotations"])
+    grads1 = torch.autograd.grad(images1, [p[k] for k in NAMES] + [m2d1], grad_outputs=dL[:1])
+    c1, r1, k1, g1 = _single(scenes[0], cuda_device, p, dL[0])
+    assert torch.equal(images1[0], c1) and torch.equal(radii1[0], r1) and n1 == k1
+    for k, a, b in zip(NAMES + ("means2D",), grads1, g1):
+        assert (a.reshape(b.shape) - b).abs().max() <= ATOMIC_RTOL * b.abs().max(), k
 
 
 @pytest.mark.parametrize("W,H", [(160, 96), (150, 90)])
@@ -110,7 +124,8 @@ def test_batched_binning_is_bit_exact_per_view(cuda_device):
     """Sorted keys / point list / tile ranges of a 2-view batch, view by view, against the oracle
     (virtual tile v*T+t, virtual Gaussian v*P+g, ranges offset by the instances of the views before)."""
     from gsvc_b200 import _lib
-    from gsvc_b200.views import ViewBatch, _NativeViews
+    from gsvc_b200.rasterizer import _NativeViews
+    from gsvc_b200.views import ViewBatch
     P, W, H = 6000, 128, 80
     scenes = _scenes(P, W, H, 128, seed=47, frames=(64,))
     fos = [_oracle(s) for s in scenes]

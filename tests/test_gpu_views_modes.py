@@ -148,7 +148,7 @@ def _check_against_single_calls(single, images, radii, n, grads, m2d_grad, names
 def _export_batch_geometry(batch, device, g, P, R):
     """Preprocess outputs of a directly launched batch, per view: the virtual Gaussian v*P+g of gsvc_rast_export_geom."""
     from gsvc_b200 import _lib
-    from gsvc_b200.views import _NativeViews
+    from gsvc_b200.rasterizer import _NativeViews
     L = _lib.lib()
     V = batch.n_views
     sh_M = g["shs"].shape[1] if "shs" in g else 0

@@ -250,6 +250,23 @@ def test_view_batch_layout_and_validation():
         ViewBatch([f, b], flip_x=[True])                          # one entry per view
 
 
+def test_dropin_view_descriptor_equals_a_batch_of_one():
+    """A GaussianRasterizer call builds its one-view native descriptor per call, without a ViewBatch; it must equal,
+    field for field, the descriptor of ViewBatch([rs]), since both go through the same batched entry points."""
+    from gsvc_b200.rasterizer import _NativeViews
+    from gsvc_b200.views import ViewBatch
+    cpu = torch.device("cpu")
+    rs = _cpu_settings()
+    one, batch = _NativeViews(None, cpu, rs), ViewBatch([rs]).native(cpu)
+    assert (one.n_views, one.n_out) == (batch.n_views, batch.n_out) == (1, 1)
+    a, b = one.views[0], batch.views[0]
+    assert a.viewmatrix == b.viewmatrix == rs.viewmatrix.data_ptr()
+    assert (a.vm_stride_r, a.vm_stride_c) == (b.vm_stride_r, b.vm_stride_c) == rs.viewmatrix.stride()
+    assert list(a.campos) == list(b.campos) == pytest.approx(list(rs.campos))
+    assert (a.out_image, a.flip_x, a.weight) == (b.out_image, b.flip_x, b.weight) == (0, 0, 1.0)
+    assert bytes(one.views) == bytes(batch.views) and bytes(one.ns[0].c) == bytes(batch.ns[0].c)
+
+
 def test_batched_and_host_paths_have_no_cpu_fallback():
     from gsvc_b200.graphed import GraphedStep
     from gsvc_b200.hostpipe import HostStepPipeline
