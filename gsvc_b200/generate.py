@@ -95,9 +95,9 @@ class _Epilogue(torch.autograd.Function):
             p = lambda t: None if t is None else t.data_ptr()
             _lib.check(L.gsvc_gen_epilogue_forward(
                 n_vis, K, p(vis), p(a), p(go), p(gs), p(mk), p(nop), p(col), p(sr), p(no), p(lo), p(hi), p(xyz), p(colo),
-                p(opa), p(sca), p(rot), p(nop_full), p(sel), p(rank), scratch.data_ptr(), slot, ticket, stream),
+                p(opa), p(sca), p(rot), p(nop_full), p(sel), p(rank), scratch.data_ptr(), slot.ptr, ticket, stream),
                 "gsvc_gen_epilogue_forward")
-            M = _lib.check(L.gsvc_rast_wait_count(slot, ticket, stream), "gsvc_rast_wait_count") if total else 0
+            M = _lib.check(L.gsvc_rast_wait_count(slot.ptr, ticket, stream), "gsvc_rast_wait_count") if total else 0
         ctx.save_for_backward(a, go, gs, mk, vis, nop, sr, no, lo, hi, rank)
         ctx.dims = (N, n_vis, K, M)
         ctx.shapes = (anchor.shape, grid_offsets.shape, grid_scaling.shape, masks.shape, neural_opacity.shape,

@@ -20,8 +20,9 @@ L1 + D-SSIM loss (gsvc_b200.loss) against it and back-propagates, so the whole s
     target.copy_(frames)                                # this iteration's target frames, in place
     color, radii, grads = step()                        # step.loss: the per-image losses of this replay
 
-The binning capacity is fixed at capture time from an eager warm-up (+50 % + 64 Ki instances);
-`capacity_ok()` compares it with the instance count the device published for the last replay.
+The binning capacity is fixed at capture time from an eager warm-up (+50 % + 64 Ki instances) and recorded on the
+step's own count slot; `capacity_ok()` compares it with the instance count the device published there for the last
+replay.
 """
 from __future__ import annotations
 
@@ -33,7 +34,28 @@ from . import rasterizer as R
 from .loss import _check_lambda, photometric_loss
 from .rasterizer import RasterizerError
 from .sharding import GRAD_LAYOUT, GRAD_WIDTH, packed_backward
-from .views import ViewBatch, capacity_shape, render_params
+from .views import ViewBatch, render_params
+
+
+def _packed_step(rast, params, dL, packed, exchange=None, loss_target=None, lambda_dssim=0.2):
+    """Forward + backward of `rast` on the GRAD_LAYOUT dict `params`, the gradients written into `packed`
+    (sharding.packed_backward); the backward is seeded with `dL`, or with the mean of photometric_loss(image,
+    loss_target) when a target is given.  Returns (color, radii, num_rendered, per-image loss or None)."""
+    leaves = {k: params[k].detach().requires_grad_(True) for k, _ in GRAD_LAYOUT}
+    color, radii, n = render_params(rast, leaves)
+    loss = None if loss_target is None else photometric_loss(color, loss_target, lambda_dssim)
+    with packed_backward(packed, exchange=exchange):
+        torch.autograd.grad(color if loss is None else loss.mean(), [leaves[k] for k, _ in GRAD_LAYOUT],
+                            grad_outputs=dL)
+    return color, radii, n, loss
+
+
+def _steps_fit(device, steps) -> bool:
+    """After a synchronisation: no rasterizer launch on `device` ran out of instance capacity since the last check
+    (the sticky device counter, reset here once), and the last replay of every one of `steps` fits its slot."""
+    if R.overflow_events(device) > 0:
+        return False
+    return all(step.slot.fits() for step in steps)
 
 
 class GraphedStep:
@@ -54,11 +76,11 @@ class GraphedStep:
         if not m.is_cuda:
             raise RasterizerError("GraphedStep needs CUDA tensors: gsvc_b200 has no CPU fallback")
         self.device, self.P = m.device, int(m.shape[0])
-        self.loss_target, self.loss = loss_target, None
+        self.loss_target, self.lambda_dssim, self.loss = loss_target, lambda_dssim, None
         if loss_target is not None:
             if dL is not None:
                 raise RasterizerError("pass either dL (a fixed seed gradient) or loss_target (the step's own loss)")
-            self.lambda_dssim = _check_lambda(lambda_dssim)
+            _check_lambda(lambda_dssim)
             if not isinstance(loss_target, torch.Tensor) or loss_target.device != self.device:
                 raise RasterizerError(f"loss_target must be a tensor on {self.device}")
             if loss_target.dtype != torch.float32 or not loss_target.is_contiguous():
@@ -80,7 +102,7 @@ class GraphedStep:
         self.graph = None
         self.color = self.radii = None
         # the graph's own pinned count word: its scan kernel publishes num_rendered here on every replay, whatever
-        # other graphs or eager calls of this thread do meanwhile
+        # other graphs or eager calls of this thread do meanwhile; the capture records its capacity on it
         self.slot = R.CountSlot()
         self.capacity = None
         self.recapture()
@@ -90,17 +112,7 @@ class GraphedStep:
         if not self.backward:
             with torch.no_grad():
                 return (*render_params(self.rast, p, means2D=p["means3D"]), None)   # no gradient: any tensor serves
-        leaves = {k: p[k].detach().requires_grad_(True) for k, _ in GRAD_LAYOUT}
-        color, radii, n = render_params(self.rast, leaves)
-        loss = None
-        if self.loss_target is not None:
-            loss = photometric_loss(color, self.loss_target, self.lambda_dssim)
-            with packed_backward(self.packed, exchange=self.exchange):
-                torch.autograd.grad(loss.mean(), [leaves[k] for k, _ in GRAD_LAYOUT])
-            return color, radii, n, loss
-        with packed_backward(self.packed, exchange=self.exchange):
-            torch.autograd.grad(color, [leaves[k] for k, _ in GRAD_LAYOUT], grad_outputs=self.dL)
-        return color, radii, n, loss
+        return _packed_step(self.rast, p, self.dL, self.packed, self.exchange, self.loss_target, self.lambda_dssim)
 
     def recapture(self) -> None:
         """(Re)build the graph: eager warm-up on a side stream (sets the capacity hint), then capture."""
@@ -117,7 +129,7 @@ class GraphedStep:
         self.graph = torch.cuda.CUDAGraph()
         with R.own_count_slot(self.slot), torch.cuda.graph(self.graph):
             self.color, self.radii, _, self.loss = self._run()
-        self.capacity = R.captured_capacity(self.device, self.P, *capacity_shape(self.rast))
+        self.capacity = self.slot.capacity
 
     def __call__(self):
         if self.exchange is not None and self.exchange.generation != self._exchange_generation:
@@ -133,9 +145,7 @@ class GraphedStep:
     def capacity_ok(self) -> bool:
         """After a synchronisation: no replay since the last check ran out of the instance capacity fixed at
         capture time (sticky device-side counter), and the last replay's published count fits too."""
-        if R.overflow_events(self.device) > 0:
-            return False
-        return self.capacity is None or self.num_rendered() <= self.capacity
+        return _steps_fit(self.device, [self])
 
 
 class FrameStreamer:
@@ -197,8 +207,9 @@ class FrameStreamer:
             s.synchronize()
 
     def capacity_ok(self) -> bool:
-        """After `synchronize()`: every frame since the last check fitted the instance capacity of the graphs."""
-        return R.overflow_events(self.device) == 0
+        """After `synchronize()`: every frame since the last check fitted the instance capacity of the graphs, and
+        so did each stream's last frame."""
+        return _steps_fit(self.device, self.steps)
 
     def recapture(self) -> None:
         for s, step in zip(self.streams, self.steps):

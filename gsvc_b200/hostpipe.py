@@ -37,18 +37,18 @@ from typing import Callable, Dict, Optional
 
 import torch
 
+from .graphed import GraphedStep, _packed_step, _steps_fit
 from .rasterizer import RasterizerError
-from .sharding import GRAD_LAYOUT, GRAD_WIDTH, packed_backward
-from .views import capacity_shape, render_params
+from .sharding import GRAD_LAYOUT, GRAD_WIDTH
 
 
 class HostStepPipeline:
     def __init__(self, P: int, device, slots: int = 2, use_graphs: bool = True, sharded: bool = False,
                  peer_copies: Optional[bool] = None):
-        """`use_graphs`: after one eager step per slot (which sizes the binning buffer), the slot's forward +
-        backward (8 kernels) is captured in a CUDA graph and replayed, so a step costs the host one graph launch
-        instead of ~10 launches and the autograd bookkeeping; `capacity_ok()` reports whether the instance capacity
-        fixed at capture time held (if not the slot is re-captured from an eager step)."""
+        """`use_graphs`: on a slot's first step its forward + backward (8 kernels) is captured in a
+        graphed.GraphedStep, whose eager warm-up sizes the binning buffer, and replayed from then on, so a step costs
+        the host one graph launch instead of ~10 launches and the autograd bookkeeping; `capacity_ok()` reports
+        whether the instance capacity fixed at capture time held (if not, call `recapture()`)."""
         if slots < 2:
             raise ValueError("need at least 2 slots to overlap copies with compute")
         self.P, self.slots = int(P), int(slots)
@@ -70,8 +70,8 @@ class HostStepPipeline:
         self.n_stepped = 0
         self.ready = deque()
         self.use_graphs = bool(use_graphs)
-        self.graphs = [None] * slots         # per slot: (key, CUDAGraph) once captured
-        self.eager_seen = [None] * slots     # per slot: key of the last eager step (capture needs one first)
+        self.graphs = [None] * slots         # per slot: its GraphedStep once captured
+        self.graph_keys = [None] * slots     # per slot: the (rasterizer, dL) its GraphedStep was captured with
         # host-side row sharding over the ranks of the default process group
         self.rank, self.world = 0, 1
         if sharded:
@@ -208,21 +208,15 @@ class HostStepPipeline:
         main.wait_event(self.in_ready[b])
         if self.d2h_done[b] is not None:
             main.wait_event(self.d2h_done[b])                 # the slot's gradient buffer has been read out
-        key = (id(rast), dL.data_ptr(), tuple(dL.shape))
-        g = self.graphs[b]
-        if g is not None and g[0] != key:
-            g = self.graphs[b] = None
-        if g is None and self.use_graphs and self.eager_seen[b] == key:
-            # second step on this slot with the same rasterizer and seed gradient: capture it
-            graph = torch.cuda.CUDAGraph()
-            with torch.cuda.graph(graph):
-                self._compute(b, rast, dL)
-            g = self.graphs[b] = (key, graph, rast)
-        if g is not None:
-            g[1].replay()
+        if self.use_graphs:
+            key = (id(rast), dL.data_ptr(), tuple(dL.shape))
+            if self.graphs[b] is None or self.graph_keys[b] != key:
+                self.graphs[b] = GraphedStep(rast, self.views(self.dev_flat[b]), dL, packed=self.dev_grads[b],
+                                             warmup=1)
+                self.graph_keys[b] = key
+            self.graphs[b]()
         else:
-            self.last_num_rendered = self._compute(b, rast, dL)
-            self.eager_seen[b] = key
+            _packed_step(rast, self.views(self.dev_flat[b]), dL, self.dev_grads[b])
         work = None
         if self.world > 1 and self.peer is not None:
             pass        # the gradients are exchanged on the copy-out stream below, without a collective kernel
@@ -257,24 +251,15 @@ class HostStepPipeline:
         self.n_stepped += 1
         return b
 
-    def _compute(self, b: int, rast, dL: torch.Tensor) -> int:
-        p = {k: v.requires_grad_(True) for k, v in self.views(self.dev_flat[b]).items()}
-        color, radii, n = render_params(rast, p)
-        with packed_backward(self.dev_grads[b]):
-            torch.autograd.grad(color, [p[k] for k, _ in GRAD_LAYOUT], grad_outputs=dL)
-        return n
-
-    def capacity_ok(self, rast) -> bool:
-        """After a synchronisation: did the instance capacity of the captured graphs hold the last replayed step?
-        (False: call `recapture()`; the gradients of that step are invalid.)"""
-        from . import rasterizer as R
-        if R.overflow_events(self.device) > 0:
-            return False
-        return R.captured_capacity_ok(self.device, self.P, *capacity_shape(rast))
+    def capacity_ok(self, rast=None) -> bool:
+        """After a synchronisation: did the instance capacity of the slots' captured steps hold every replay since
+        the last check?  (False: call `recapture()`; the gradients of those steps are invalid.)  `rast` is accepted
+        for existing callers and not used: each slot's step knows its own capacity."""
+        return _steps_fit(self.device, [g for g in self.graphs if g is not None])
 
     def recapture(self) -> None:
+        """Drop the slots' captured steps: each slot captures a new one on its next step."""
         self.graphs = [None] * self.slots
-        self.eager_seen = [None] * self.slots
 
     def grads(self, slot: int) -> torch.Tensor:
         """The [P,14] gradients of the step that returned `slot` (pinned host memory); blocks until they landed.

@@ -86,31 +86,6 @@ def _record_capacity(key_exact, key_density, P: int, num_rendered: int) -> None:
         _density_hint[key_density] = max(d, 0.97 * _density_hint.get(key_density, 0.0))
 
 
-_captured_caps: dict = {}
-
-
-def last_num_rendered() -> int:
-    """num_rendered most recently published by the device to this thread's pinned counter (after a
-    synchronize it is the value of the last forward, eager or replayed from a CUDA graph)."""
-    st = _count_slots
-    return int(st.slot[0].item()) & ((1 << 40) - 1) if hasattr(st, "slot") else 0
-
-
-def captured_capacity(device, P: int, H: int, W: int, n_views: Optional[int] = None) -> Optional[int]:
-    """The binning capacity the last CUDA-graph capture of this shape fixed (None: never captured).  `n_views`: for
-    a graph around views.rasterize_views; None is one view."""
-    key, _ = _capacity_keys(torch.device(device).index, P, H, W, 1 if n_views is None else n_views)
-    return _captured_caps.get(key)
-
-
-def captured_capacity_ok(device, P: int, H: int, W: int, n_views: Optional[int] = None) -> bool:
-    """After replaying a CUDA graph that contains the rasterizer (and synchronizing): did the binning capacity
-    fixed at capture time hold the instances of the last replay?  If not, the replay's image is invalid and
-    the step must be re-captured (or run eagerly).  `n_views`: for a graph around views.rasterize_views."""
-    cap = captured_capacity(device, P, H, W, n_views)
-    return cap is None or last_num_rendered() <= cap
-
-
 def overflow_events(device=None, reset: bool = True) -> int:
     """How many rasterizer launches on `device` ran out of instance capacity since the last reset (synchronises the
     current stream).  Only CUDA-graph replays can be affected: the eager call re-runs by itself."""
@@ -247,15 +222,25 @@ def _bytes(n: int, device) -> torch.Tensor:
 
 
 class CountSlot:
-    """A pinned, device-addressable 64-bit word the tile scan publishes `ticket << 40 | num_rendered` into."""
+    """A pinned, device-addressable 64-bit word the tile scan publishes `ticket << 40 | num_rendered` into.
+
+    `capacity` is the binning capacity a rasterizer call captured in a CUDA graph under this slot fixed (None until
+    such a capture); a replay has nobody to re-run it, so its owner checks `fits()` after a synchronisation.  When
+    one graph captures several rasterizer calls under one slot, the slot holds the last call's capacity and count:
+    the sticky device counter (overflow_events) still reports an overflow of the others."""
 
     def __init__(self):
         self.tensor = torch.zeros(1, dtype=torch.int64).pin_memory()
         self.ptr = self.tensor.data_ptr()
         self.ticket = 0
+        self.capacity = None
 
     def value(self) -> int:
         return int(self.tensor[0].item()) & ((1 << 40) - 1)
+
+    def fits(self) -> bool:
+        """After a synchronisation: the last published count fits the captured capacity (True before a capture)."""
+        return self.capacity is None or self.value() <= self.capacity
 
 
 @contextlib.contextmanager
@@ -263,7 +248,8 @@ def own_count_slot(slot: "CountSlot"):
     """Rasterizer calls of this thread inside the context publish their instance count to `slot` instead of the
     thread's shared one.  A CUDA graph bakes the slot's address into its scan kernel, so every captured graph gets a
     slot of its own (GraphedStep does this): replays on different streams no longer overwrite each other's count,
-    and the slot lives as long as the graph's owner, not as long as the capturing thread."""
+    the slot lives as long as the graph's owner, not as long as the capturing thread, and it records the capacity
+    the capture fixed."""
     st = _count_slots
     prev = getattr(st, "override", None)
     st.override = slot
@@ -274,16 +260,16 @@ def own_count_slot(slot: "CountSlot"):
 
 
 def _count_slot():
-    """One pinned count word per host thread (or the caller's own, see own_count_slot) + a ticket counter."""
+    """(the active CountSlot, its next ticket): one pinned count word per host thread, or the caller's own (see
+    own_count_slot)."""
     st = _count_slots
     slot = getattr(st, "override", None)
     if slot is None:
         if not hasattr(st, "own"):
             st.own = CountSlot()
-            st.slot = st.own.tensor      # (last_num_rendered reads it)
         slot = st.own
     slot.ticket = (slot.ticket % 0xFFFFFE) + 1
-    return slot.ptr, slot.ticket
+    return slot, slot.ticket
 
 
 def _require_cuda(t: torch.Tensor, what: str):
@@ -360,14 +346,15 @@ class _RasterizeViews(torch.autograd.Function):
             cap, hint = _predict_capacity(hint_key, dens_key, P)
             # CUDA-graph capture (torch.cuda.graph around the caller's step): nothing may wait on the device, so
             # the instance count of the last eager call stands in for num_rendered and the binning capacity is
-            # fixed generously; captured_capacity_ok() tells the caller after a replay whether it sufficed.
+            # fixed generously and recorded on the count slot; its fits() tells the caller after a replay whether it
+            # sufficed.
             capturing = torch.cuda.is_current_stream_capturing()
+            slot, ticket = _count_slot()
             if capturing:
                 if hint is None:
                     raise RasterizerError("run the rasterizer once eagerly with these shapes before capturing it "
                                           "in a CUDA graph (the binning capacity comes from that call)")
-                cap = int(hint * 1.5) + 65536
-                _captured_caps[hint_key] = cap
+                cap = slot.capacity = int(hint * 1.5) + 65536
             # one allocation for all native state: [geom | image | backward accumulators | binning]
             need_grad = any(ctx.needs_input_grad)
             n_geom = _align(L.gsvc_rast_geom_bytes(P * V, sh_M))
@@ -385,20 +372,19 @@ class _RasterizeViews(torch.autograd.Function):
             color = torch.empty((3, H, W) if single else (n_out, 3, H, W), dtype=_F32, device=device)
             radii = torch.empty((P,) if single else (V, P), dtype=torch.int32, device=device)
             stream = _stream_ptr(device)
-            slot, ticket = _count_slot()
             try:
                 L.gsvc_rast_count_overflows(1 if capturing else 0)   # a replay has nobody to re-run it; eager does
                 _lib.check(L.gsvc_rast_forward_views_launch(
                     nv.ref, V, nv.views, n_out, P, sh_M, _ptr(means3D_c), _ptr(sh_c), _ptr(col_c), _ptr(op_c),
                     _ptr(sc_c), _ptr(rot_c), _ptr(cov_c), geom_p, image_p, bin_p, cap, acc_p, color.data_ptr(),
-                    radii.data_ptr(), slot, ticket, stream), "gsvc_rast_forward_views_launch")
+                    radii.data_ptr(), slot.ptr, ticket, stream), "gsvc_rast_forward_views_launch")
                 # The reference API returns num_rendered as a Python int (renderer.py:90).  The scan kernel
                 # publishes it into pinned memory as soon as it is known, so this wait ends while the
                 # scatter / sort / blend kernels are still running: no stream synchronisation.
                 if capturing:
                     num_rendered = hint
                 else:
-                    num_rendered = _lib.check(L.gsvc_rast_wait_count(slot, ticket, stream), "gsvc_rast_wait_count")
+                    num_rendered = _lib.check(L.gsvc_rast_wait_count(slot.ptr, ticket, stream), "gsvc_rast_wait_count")
                 if num_rendered > 0xFFFFFFFF:
                     raise RasterizerError(f"num_rendered {num_rendered} exceeds 32-bit tile ranges")
                 capacity_stats["calls"] += 1
@@ -584,9 +570,9 @@ class GaussianRasterizer(nn.Module):
             if index_range is not None and lo == hi:
                 return idx[:0], (radii.zero_() if radii is not None else None)
             _lib.check(L.gsvc_rast_visible_filter_compact(ns.ref, P, _ptr(m), _ptr(s), _ptr(r), _ptr(c), _ptr(radii),
-                                                          _ptr(idx), scratch.data_ptr(), slot, ticket, lo, hi, stream),
-                       "gsvc_rast_visible_filter_compact")
-            count = _lib.check(L.gsvc_rast_wait_count(slot, ticket, stream), "gsvc_rast_wait_count")
+                                                          _ptr(idx), scratch.data_ptr(), slot.ptr, ticket, lo, hi,
+                                                          stream), "gsvc_rast_visible_filter_compact")
+            count = _lib.check(L.gsvc_rast_wait_count(slot.ptr, ticket, stream), "gsvc_rast_wait_count")
         return idx[:count], radii
 
     def forward(self, means3D, means2D, opacities, shs=None, colors_precomp=None, scales=None, rotations=None,

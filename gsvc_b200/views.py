@@ -149,10 +149,3 @@ def render_params(rast, p, means2D=None):
         means2D = torch.zeros_like(p["means3D"], requires_grad=True)
     return rast(means3D=p["means3D"], means2D=means2D, shs=None, colors_precomp=p["colors_precomp"],
                 opacities=p["opacities"], scales=p["scales"], rotations=p["rotations"], cov3D_precomp=None)
-
-
-def capacity_shape(rast):
-    """(H, W, n_views) of a GaussianRasterizer (one view) or a ViewBatch: the shape rasterizer.captured_capacity
-    takes after P."""
-    rs, n_views = (rast.settings[0], rast.n_views) if isinstance(rast, ViewBatch) else (rast.raster_settings, 1)
-    return int(rs.image_height), int(rs.image_width), n_views

@@ -568,9 +568,10 @@ def test_retain_graph_double_backward_is_consistent(cuda_device):
         assert (z - 2 * x).abs().max() <= ATOMIC_RTOL * z.abs().max()
 
 
-def test_cuda_graph_capture_and_replay(cuda_device):
+def test_cuda_graph_capture_and_replay_under_own_count_slot(cuda_device):
     """The whole forward+backward is capturable in a CUDA graph (no host wait while capturing); a replay on
-    updated inputs reproduces the eager result."""
+    updated inputs reproduces the eager result.  The capture records its capacity on the caller's count slot, and
+    the replay's count fits it."""
     from gsvc_b200 import rasterizer
     from gsvc_b200.rasterizer import GaussianRasterizer
     scene = make_scene(P=12000, W=192, H=128, F=192, seed=29)
@@ -594,36 +595,32 @@ def test_cuda_graph_capture_and_replay(cuda_device):
     torch.cuda.current_stream(cuda_device).wait_stream(side)
     torch.cuda.synchronize()
     graph = torch.cuda.CUDAGraph()
-    with torch.cuda.graph(graph):
+    slot = rasterizer.CountSlot()
+    with rasterizer.own_count_slot(slot), torch.cuda.graph(graph):
         color_g, radii_g, grads_g = step()
+    assert slot.capacity is not None and slot.capacity > 0
     # new values in the static input tensors, then replay
     with torch.no_grad():
         p["means3D"][:, :2] += 0.01
         p["opacities"].mul_(0.9)
+    rasterizer.overflow_events(cuda_device)            # clear whatever earlier tests left
     graph.replay()
     torch.cuda.synchronize()
-    assert rasterizer.captured_capacity_ok(cuda_device, 12000, 128, 192)
+    assert rasterizer.overflow_events(cuda_device) == 0 and slot.fits()
+    assert slot.value() > 0
     color_e, radii_e, grads_e = step()
     assert torch.equal(radii_g, radii_e)
     assert torch.equal(color_g, color_e)               # the forward is deterministic
     for a, b in zip(grads_g, grads_e):
         assert (a - b).abs().max() <= ATOMIC_RTOL * b.abs().max()
-    assert rasterizer.last_num_rendered() > 0
 
 
-def test_host_step_pipeline_matches_direct_call(cuda_device):
-    """gsvc_b200.hostpipe (pinned host params in, pinned host [P,14] grads out, copies pipelined over two slots)
-    returns, for every step of a sequence with changing parameters, exactly the gradients of the plain call."""
-    from gsvc_b200.hostpipe import HostStepPipeline
-    from gsvc_b200.rasterizer import GaussianRasterizer
+def _host_param_sets(g, P, n):
+    """`n` pinned [14*P] parameter sets (GRAD_LAYOUT order) of the Gaussians `g`, opacities and x positions changing
+    from one set to the next."""
     from gsvc_b200.sharding import GRAD_LAYOUT
-    P = 9000
-    scene = make_scene(P=P, W=160, H=96, F=160, seed=31)
-    rast = GaussianRasterizer(raster_settings=product_settings(scene, cuda_device))
-    dL = torch.randn((3, 96, 160), generator=torch.Generator().manual_seed(2)).to(cuda_device)
-    g = scene["gaussians"]
     hosts = []
-    for s in range(5):
+    for s in range(n):
         flat = torch.empty(14 * P, dtype=torch.float32).pin_memory()
         off = 0
         for k, w in GRAD_LAYOUT:
@@ -635,7 +632,11 @@ def test_host_step_pipeline_matches_direct_call(cuda_device):
             flat[off:off + w * P].copy_(v.reshape(-1))
             off += w * P
         hosts.append(flat)
-    pipe = HostStepPipeline(P, cuda_device, slots=2)
+    return hosts
+
+
+def _run_pipeline(pipe, rast, dL, hosts):
+    """One step per host parameter set, each set prefetched a step ahead: the [P,14] host gradients of every step."""
     got = []
     pipe.prefetch(hosts[0])
     for i in range(len(hosts)):
@@ -643,19 +644,71 @@ def test_host_step_pipeline_matches_direct_call(cuda_device):
             pipe.prefetch(hosts[i + 1])
         slot = pipe.step(rast, dL)
         got.append(pipe.grads(slot).clone())
-    with pytest.raises(Exception):
-        pipe.step(rast, dL)                     # nothing prefetched
-    assert pipe.graphs[0] is not None and pipe.graphs[1] is not None   # steps 2.. were CUDA-graph replays
-    assert pipe.capacity_ok(rast)
+    return got
+
+
+def _assert_pipeline_matches_direct_call(pipe, rast, dL, hosts, got):
+    """Each step's gradients are the plain drop-in call's on that parameter set, up to the order of the atomics."""
+    from gsvc_b200.sharding import GRAD_LAYOUT
     for flat, packed in zip(hosts, got):
-        p = {k: v.clone().to(cuda_device).requires_grad_(True) for k, v in pipe.views(flat).items()}
+        p = {k: v.clone().to(dL.device).requires_grad_(True) for k, v in pipe.views(flat).items()}
         m2d = torch.zeros_like(p["means3D"], requires_grad=True)
         color, _, _ = rast(means3D=p["means3D"], means2D=m2d, shs=None, colors_precomp=p["colors_precomp"],
                            opacities=p["opacities"], scales=p["scales"], rotations=p["rotations"], cov3D_precomp=None)
         grads = torch.autograd.grad(color, [p[k] for k, _ in GRAD_LAYOUT], grad_outputs=dL)
-        ref = torch.cat([x.reshape(P, -1) for x in grads], dim=1).cpu()
+        ref = torch.cat([x.reshape(pipe.P, -1) for x in grads], dim=1).cpu()
         assert ref.abs().max() > 0
         assert (packed - ref).abs().max() <= ATOMIC_RTOL * ref.abs().max()   # atomics order only
+
+
+def test_host_step_pipeline_matches_direct_call(cuda_device):
+    """gsvc_b200.hostpipe (pinned host params in, pinned host [P,14] grads out, copies pipelined over two slots)
+    returns, for every step of a sequence with changing parameters, exactly the gradients of the plain call."""
+    from gsvc_b200.hostpipe import HostStepPipeline
+    from gsvc_b200.rasterizer import GaussianRasterizer
+    P = 9000
+    scene = make_scene(P=P, W=160, H=96, F=160, seed=31)
+    rast = GaussianRasterizer(raster_settings=product_settings(scene, cuda_device))
+    dL = torch.randn((3, 96, 160), generator=torch.Generator().manual_seed(2)).to(cuda_device)
+    hosts = _host_param_sets(scene["gaussians"], P, 5)
+    pipe = HostStepPipeline(P, cuda_device, slots=2)
+    got = _run_pipeline(pipe, rast, dL, hosts)
+    with pytest.raises(Exception):
+        pipe.step(rast, dL)                     # nothing prefetched
+    assert pipe.graphs[0] is not None and pipe.graphs[1] is not None   # the steps were CUDA-graph replays
+    assert pipe.capacity_ok(rast)
+    _assert_pipeline_matches_direct_call(pipe, rast, dL, hosts, got)
+
+
+def test_host_step_pipeline_capacity_ignores_eager_calls(cuda_device):
+    """The pipeline's captured steps publish their instance counts to count slots of their own: an eager call on the
+    same thread that renders far more instances than the pipeline's capacity (same P and image size) does not make
+    `capacity_ok()` report an overflow the pipeline never had, and the next replays still equal the plain call."""
+    from gsvc_b200.hostpipe import HostStepPipeline
+    from gsvc_b200.rasterizer import GaussianRasterizer
+    P = 20000
+    scene = make_scene(P=P, W=256, H=160, F=256, seed=61)
+    rast = GaussianRasterizer(raster_settings=product_settings(scene, cuda_device))
+    dL = torch.randn((3, 160, 256), generator=torch.Generator().manual_seed(5)).to(cuda_device)
+    hosts = _host_param_sets(scene["gaussians"], P, 6)
+    pipe = HostStepPipeline(P, cuda_device, slots=2)
+    _run_pipeline(pipe, rast, dL, hosts[:4])        # two steps per slot: both slots have replayed their graph
+    torch.cuda.synchronize()
+    assert pipe.graphs[0] is not None and pipe.graphs[1] is not None
+    assert pipe.capacity_ok(rast)
+    g = {k: v.to(cuda_device) for k, v in scene["gaussians"].items()}
+    with torch.no_grad():
+        kw = dict(means2D=g["means3D"], shs=None, colors_precomp=g["colors_precomp"], opacities=g["opacities"],
+                  rotations=g["rotations"], cov3D_precomp=None)
+        _, _, n0 = rast(means3D=g["means3D"], scales=g["scales"], **kw)
+        _, _, n_big = rast(means3D=g["means3D"], scales=g["scales"] * 8.0, **kw)
+    torch.cuda.synchronize()
+    assert n_big > 1.5 * n0 + 65536                 # far past the capacity the pipeline's capture fixed
+    assert pipe.capacity_ok(rast)
+    got = _run_pipeline(pipe, rast, dL, hosts[4:])
+    torch.cuda.synchronize()
+    assert pipe.capacity_ok(rast)
+    _assert_pipeline_matches_direct_call(pipe, rast, dL, hosts[4:], got)
 
 
 def test_graphed_step_matches_eager(cuda_device):

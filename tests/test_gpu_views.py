@@ -193,7 +193,8 @@ def test_view_batch_validation(cuda_device):
 
 def test_frame_streamer_matches_single_frames(cuda_device):
     """graphed.FrameStreamer: independent frames replayed round-robin on several streams equal the frames rendered
-    one by one (bit-exact: same kernels), including when a stream's buffers are reused."""
+    one by one (bit-exact: same kernels), including when a stream's buffers are reused.  `capacity_ok()` holds for
+    them, and reports a frame that outgrows its stream's captured capacity."""
     from gsvc_b200.graphed import FrameStreamer
     from gsvc_b200.views import render_toast
     P, W, H, F = 8000, 160, 96, 160
@@ -215,6 +216,12 @@ def test_frame_streamer_matches_single_frames(cuda_device):
                                      rotations=params["rotations"])
             assert torch.equal(got[i], ref), f"frame {frames[i]}"
     assert not torch.equal(got[0], got[5])
+    assert streamer.capacity_ok()
+    with torch.no_grad():
+        params["scales"].mul_(8.0)                       # the static tensors the graphs read: every splat ~64x the tiles
+    streamer.render(sets[0].viewmatrix, sets[1].viewmatrix)
+    streamer.synchronize()
+    assert not streamer.capacity_ok()
 
 
 def test_densify_stats_equals_the_reference_expression(cuda_device):
