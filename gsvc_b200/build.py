@@ -27,6 +27,7 @@ SOURCES = {
     "preprocess_bwd.cu": [],
     "epilogue.cu": [],
     "loss.cu": [],
+    "quality.cu": [],
     "collective.cu": [],
     "api.cu": [],
 }

@@ -32,6 +32,7 @@ import torch
 
 from . import rasterizer as R
 from .loss import _check_lambda, photometric_loss
+from . import quality as Q
 from .rasterizer import RasterizerError
 from .sharding import GRAD_LAYOUT, GRAD_WIDTH, packed_backward
 from .views import ViewBatch, render_params
@@ -161,7 +162,16 @@ class FrameStreamer:
         streamer.synchronize()
 
     `render` returns the stream's static output tensor: it is overwritten n_streams frames later, so consume it
-    (on its stream, or after `wait`) before that."""
+    (on its stream, or after `wait`) before that.
+
+    Decode-and-evaluate: with a `target` frame and a `quality` output (3 fp32 values on the device, typically a row
+    of the caller's [F,3] tensor), the frame's PSNR / SSIM / MS-SSIM (gsvc_b200.quality) are computed on its stream
+    right after the replay, before the output tensor can be reused; one synchronisation at the end of the loop:
+
+        q = torch.empty(F, 3, device="cuda")
+        for i, (V_front, V_back) in enumerate(frames):
+            streamer.render(V_front, V_back, target=gt[i], quality=q[i])
+        streamer.synchronize()                                              # q: [F,3] psnr, ssim, ms_ssim"""
 
     def __init__(self, front, back, params: Dict[str, torch.Tensor], n_streams: int = 4, toast: bool = True):
         m = params["means3D"]
@@ -183,10 +193,16 @@ class FrameStreamer:
             self.steps.append(step)
             self.mats.append((vf, vb))
             self.events.append(None)
+        self.scratch = [None] * self.n          # per-stream scratch of the quality metrics, allocated on first use
         self.i = 0
 
-    def render(self, V_front: torch.Tensor, V_back: torch.Tensor) -> torch.Tensor:
+    def render(self, V_front: torch.Tensor, V_back: torch.Tensor, target: Optional[torch.Tensor] = None,
+               quality: Optional[torch.Tensor] = None) -> torch.Tensor:
         k = self.i % self.n
+        if (target is None) != (quality is None):
+            raise RasterizerError("render: give both target and quality, or neither")
+        if target is not None:
+            self._check_quality_args(self.steps[k].color, target, quality)
         self.i += 1
         s = self.streams[k]
         s.wait_stream(torch.cuda.current_stream(self.device))      # V_front / V_back may have just been produced
@@ -194,9 +210,27 @@ class FrameStreamer:
             self.mats[k][0].copy_(V_front, non_blocking=True)
             self.mats[k][1].copy_(V_back, non_blocking=True)
             color, _, _ = self.steps[k]()
+            if target is not None:
+                target.record_stream(s)
+                quality.record_stream(s)
+                N, _, H, W = color.shape
+                if self.scratch[k] is None:
+                    self.scratch[k] = R._bytes(Q.scratch_bytes(N, H, W), self.device)
+                y = R._dev_f32(target, self.device, "target").reshape(color.shape)
+                Q.quality_into(quality, color, y, self.scratch[k])
             self.events[k] = s.record_event()
         self._last = k
         return color[0] if color.shape[0] == 1 else color
+
+    def _check_quality_args(self, color, target, quality):
+        frame = color.shape[1:] if color.shape[0] == 1 else color.shape
+        if not isinstance(target, torch.Tensor) or target.device != self.device or target.shape != frame:
+            raise RasterizerError(f"render: target must be a tensor of shape {tuple(frame)} on {self.device}")
+        want = frame[:-3] + (3,)
+        if (not isinstance(quality, torch.Tensor) or quality.device != self.device or quality.shape != want
+                or quality.dtype != torch.float32 or not quality.is_contiguous()):
+            raise RasterizerError(f"render: quality must be a contiguous float32 tensor of shape {tuple(want)} "
+                                  f"on {self.device}")
 
     def wait(self, image: torch.Tensor = None) -> None:
         """Make the current stream wait for the most recently submitted frame."""

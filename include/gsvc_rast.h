@@ -404,6 +404,27 @@ GSVC_RAST_API int gsvc_rast_loss_backward(int32_t n_images, int32_t H, int32_t W
                                           const float *target, float lambda_dssim, const float *dL_dloss,
                                           float *dL_dimage, void *stream);
 
+/*
+ * Frame quality metrics (docs/SPEC.md "Evaluation metrics", decision U10): the PSNR / SSIM / MS-SSIM of an evaluation
+ * loop, on the device.  For each image n of x = image, y = target, both [n_images,3,H,W] fp32, with x clamped to
+ * [0, 1] on read and y read as given (data range 1):
+ *     psnr    = 10 log10(1 / mse), mse = mean (x - y)^2 over the image's 3*H*W values (summed in double); +inf if 0
+ *     ssim    = mean S, S as in the loss block above (zero padding of 5, 11x11 window, sigma 1.5)
+ *     ms_ssim = mean_c prod_{l<4} relu(cs_{l,c})^{w_l} * relu(ssim_{4,c})^{w_4},  w = (0.0448, 0.2856, 0.3001, 0.2363,
+ *               0.1333): pytorch_msssim's ms_ssim(data_range=1).  Per level l and channel c, cs and ssim are the means of
+ *               (2 sigma_xy + C2) / (sigma_x^2 + sigma_y^2 + C2) and of S over the VALID (unpadded) window positions;
+ *               level l+1 is avg_pool2d(level l, 2, stride 2, padding (h % 2, w % 2)) of x and y.  NaN unless
+ *               min(H, W) > 160.
+ *   gsvc_rast_quality  writes quality [n_images,3] = (psnr, ssim, ms_ssim) (device).  scratch:
+ *                      gsvc_rast_quality_scratch_bytes(n_images, H, W) bytes for the pooled levels 1-4 (a third of the
+ *                      pixels of an image pair) and the per-CTA partial sums, which are summed per image in a fixed
+ *                      order: the results are bit-reproducible.  Six launches (two when min(H, W) <= 160), no atomics,
+ *                      no host synchronisation.
+ */
+GSVC_RAST_API size_t gsvc_rast_quality_scratch_bytes(int32_t n_images, int32_t H, int32_t W);
+GSVC_RAST_API int gsvc_rast_quality(int32_t n_images, int32_t H, int32_t W, const float *image, const float *target,
+                                    float *quality /* [n_images,3]: psnr, ssim, ms_ssim */, void *scratch, void *stream);
+
 #ifdef __cplusplus
 }
 #endif
