@@ -28,6 +28,7 @@ SOURCES = {
     "epilogue.cu": [],
     "loss.cu": [],
     "quality.cu": [],
+    "export.cu": [],
     "collective.cu": [],
     "api.cu": [],
 }

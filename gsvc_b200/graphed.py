@@ -32,6 +32,7 @@ import torch
 
 from . import rasterizer as R
 from .loss import _check_lambda, photometric_loss
+from . import export as E
 from . import quality as Q
 from .rasterizer import RasterizerError
 from .sharding import GRAD_LAYOUT, GRAD_WIDTH, packed_backward
@@ -171,7 +172,28 @@ class FrameStreamer:
         q = torch.empty(F, 3, device="cuda")
         for i, (V_front, V_back) in enumerate(frames):
             streamer.render(V_front, V_back, target=gt[i], quality=q[i])
-        streamer.synchronize()                                              # q: [F,3] psnr, ssim, ms_ssim"""
+        streamer.synchronize()                                              # q: [F,3] psnr, ssim, ms_ssim
+
+    Decode-to-host: with `host_out`, a pinned contiguous uint8 CPU tensor shaped like the frame ([H,W,3] for a toast,
+    [n_out,H,W,3] otherwise), the frame is converted to 8-bit RGB on its stream after the replay (and after the
+    quality pass, if any) into one of 2 x n_streams device staging buffers, and copied from there into `host_out` on
+    one device-to-host stream: the copy waits for the conversion, and a staging buffer is converted into again only
+    after its previous copy.  The frame's own stream never waits for the link, so its next replay is not delayed by
+    the ~0.11 ms a 1080p frame takes to cross it.  `last_event()` is recorded after the copy; a decode-to-disk loop
+    keeps a ring of pinned buffers and waits on a buffer's event before it writes the frame out and reuses it:
+
+        ring = [torch.empty(H, W, 3, dtype=torch.uint8).pin_memory() for _ in range(R)]
+        done = [None] * R
+        for i, (V_front, V_back) in enumerate(frames):
+            j = i % R
+            if done[j] is not None:
+                done[j].synchronize(); write_png(ring[j])                   # frame i - R
+            streamer.render(V_front, V_back, host_out=ring[j])
+            done[j] = streamer.last_event()
+        streamer.synchronize()                                              # then write the last R frames
+
+    A replay that overflowed its capacity (`capacity_ok()` false after a synchronisation) leaves invalid quality values
+    and invalid host frames alike."""
 
     def __init__(self, front, back, params: Dict[str, torch.Tensor], n_streams: int = 4, toast: bool = True):
         m = params["means3D"]
@@ -194,15 +216,22 @@ class FrameStreamer:
             self.mats.append((vf, vb))
             self.events.append(None)
         self.scratch = [None] * self.n          # per-stream scratch of the quality metrics, allocated on first use
+        self.staging = [None] * (2 * self.n)    # uint8 frames of the host copies, frame f in f % 2n (its stream's)
+        self.copied = [None] * (2 * self.n)     # event after the last copy out of each staging buffer
+        self.copy_stream = None                 # the device-to-host stream, created on first use
+        self._last_event = None
         self.i = 0
 
     def render(self, V_front: torch.Tensor, V_back: torch.Tensor, target: Optional[torch.Tensor] = None,
-               quality: Optional[torch.Tensor] = None) -> torch.Tensor:
+               quality: Optional[torch.Tensor] = None, host_out: Optional[torch.Tensor] = None) -> torch.Tensor:
         k = self.i % self.n
         if (target is None) != (quality is None):
             raise RasterizerError("render: give both target and quality, or neither")
         if target is not None:
             self._check_quality_args(self.steps[k].color, target, quality)
+        if host_out is not None:
+            self._check_host_out(self.steps[k].color, host_out)
+        j = self.i % (2 * self.n)
         self.i += 1
         s = self.streams[k]
         s.wait_stream(torch.cuda.current_stream(self.device))      # V_front / V_back may have just been produced
@@ -218,8 +247,22 @@ class FrameStreamer:
                     self.scratch[k] = R._bytes(Q.scratch_bytes(N, H, W), self.device)
                 y = R._dev_f32(target, self.device, "target").reshape(color.shape)
                 Q.quality_into(quality, color, y, self.scratch[k])
+            if host_out is not None:
+                if self.copy_stream is None:
+                    self.copy_stream = torch.cuda.Stream(self.device)
+                if self.staging[j] is None:
+                    self.staging[j] = torch.empty(host_out.shape, dtype=torch.uint8, device=self.device)
+                if self.copied[j] is not None:
+                    s.wait_event(self.copied[j])
+                E.rgb8_into(self.staging[j], color)
             self.events[k] = s.record_event()
         self._last = k
+        self._last_event = self.events[k]
+        if host_out is not None:
+            self.copy_stream.wait_event(self.events[k])
+            with torch.cuda.stream(self.copy_stream):
+                host_out.copy_(self.staging[j], non_blocking=True)
+                self.copied[j] = self._last_event = self.copy_stream.record_event()
         return color[0] if color.shape[0] == 1 else color
 
     def _check_quality_args(self, color, target, quality):
@@ -232,12 +275,28 @@ class FrameStreamer:
             raise RasterizerError(f"render: quality must be a contiguous float32 tensor of shape {tuple(want)} "
                                   f"on {self.device}")
 
+    def _check_host_out(self, color, host_out):
+        frame = color.shape[1:] if color.shape[0] == 1 else color.shape
+        want = tuple(frame[:-3]) + (frame[-2], frame[-1], 3)
+        if not isinstance(host_out, torch.Tensor) or host_out.is_cuda:
+            raise RasterizerError("render: host_out must be a CPU tensor (pinned), the frame's destination on the host")
+        if not host_out.is_pinned():
+            raise RasterizerError("render: host_out must be pinned (a copy into pageable memory blocks the host)")
+        if host_out.dtype != torch.uint8 or tuple(host_out.shape) != want or not host_out.is_contiguous():
+            raise RasterizerError(f"render: host_out must be a contiguous uint8 tensor of shape {want}")
+
+    def last_event(self) -> torch.cuda.Event:
+        """The event recorded after everything `render` enqueued for the most recent frame, its host copy included."""
+        if self._last_event is None:
+            raise RasterizerError("last_event: no frame has been rendered yet")
+        return self._last_event
+
     def wait(self, image: torch.Tensor = None) -> None:
         """Make the current stream wait for the most recently submitted frame."""
         torch.cuda.current_stream(self.device).wait_event(self.events[self._last])
 
     def synchronize(self) -> None:
-        for s in self.streams:
+        for s in self.streams + ([self.copy_stream] if self.copy_stream is not None else []):
             s.synchronize()
 
     def capacity_ok(self) -> bool:

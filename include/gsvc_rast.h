@@ -425,6 +425,19 @@ GSVC_RAST_API size_t gsvc_rast_quality_scratch_bytes(int32_t n_images, int32_t H
 GSVC_RAST_API int gsvc_rast_quality(int32_t n_images, int32_t H, int32_t W, const float *image, const float *target,
                                     float *quality /* [n_images,3]: psnr, ssim, ms_ssim */, void *scratch, void *stream);
 
+/*
+ * 8-bit frame export (docs/SPEC.md "8-bit frame export", decision U11): composed frames to the bytes an image writer
+ * takes.  image is [n_images,3,H,W] fp32 (planar, as render_toast / the views chain write it); out is [n_images,H,W,3]
+ * uint8, RGB interleaved, row 0 first, device-addressable.  Every value x becomes
+ *     q = uint8(min(max(fl(fl(x * 255) + 0.5), 0), 255))      truncated; NaN -> 0, +inf -> 255, -inf -> 0
+ * with the product and the sum rounded separately (never fused): torchvision's save_image arithmetic.  One launch, no
+ * scratch, no atomics, no host synchronisation (capturable in a CUDA graph).  n_images, H, W >= 1, image and out non-
+ * NULL and n_images * H * W * 3 within a 64-bit index, else GSVC_RAST_ERR_INVALID before any CUDA work.  Fastest
+ * when H * W % 4 == 0, image is 16-byte and out 4-byte aligned; any other size or alignment is handled too.
+ */
+GSVC_RAST_API int gsvc_rast_frames_rgb8(int32_t n_images, int32_t H, int32_t W, const float *image,
+                                        uint8_t *out /* [n_images,H,W,3], device-addressable */, void *stream);
+
 #ifdef __cplusplus
 }
 #endif
