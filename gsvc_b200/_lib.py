@@ -82,6 +82,11 @@ SIGNATURES = {
                                            _vp]),
     "gsvc_rast_backward_views_exchange": (C.c_int, [_SP, _i32, _VP, _i32, _i32, _i32, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
                                                     _vp, _vp, _vp, _vp, _i32, _vp, _vp, _vp, C.POINTER(Exchange), _vp]),
+    "gsvc_rast_forward_ragged_launch": (C.c_int, [_SP, _i32, _VP, _i32, _vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
+                                                  _vp, _vp, _vp, _i64, _vp, _vp, _vp, _vp, C.c_uint32, _vp]),
+    "gsvc_rast_forward_ragged_render": (C.c_int, [_SP, _i32, _VP, _i32, _vp, _vp, _vp, _vp, _i64, _vp, _vp]),
+    "gsvc_rast_backward_ragged": (C.c_int, [_SP, _i32, _VP, _i32, _vp, _i32, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
+                                            _vp, _vp, _vp, _vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "gsvc_rast_export_keys": (C.c_int, [_SP, _i32, _i64, _vp, _vp, _vp, _vp, _vp, _vp]),
     "gsvc_rast_export_geom": (C.c_int, [_i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "gsvc_rast_export_image": (C.c_int, [_SP, _i32, _vp, _vp, _vp, _vp]),

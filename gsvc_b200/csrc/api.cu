@@ -82,6 +82,8 @@ static int make_settings_views(const gsvc_rast_settings* st, int n_views, const 
     d.bg = st->bg;
     d.sh_degree = st->sh_degree; d.sh_M = sh_M;
     d.n_views = n_views;
+    d.ragged = 0;
+    memset(&d.rows, 0, sizeof(d.rows));
     int used[MAX_VIEWS] = {0};
     d.accumulate = 0;
     memset(&d.vt, 0, sizeof(d.vt));
@@ -96,6 +98,25 @@ static int make_settings_views(const gsvc_rast_settings* st, int n_views, const 
     }
     for (int o = 0; o < n_out; o++)
         if (!used[o]) return fail(GSVC_RAST_ERR_INVALID, "output image %d has no view", o);
+    return 0;
+}
+
+// A ragged batch: the view map as above, then the views' own counts (n_views entries), summed into P.
+static int make_settings_ragged(const gsvc_rast_settings* st, int n_views, const gsvc_rast_view* views, int n_out,
+                                const int32_t* counts_host, int sh_M, DevSettings& d, int32_t& P)
+{
+    int rc = make_settings_views(st, n_views, views, n_out, sh_M, d);
+    if (rc) return rc;
+    if (!counts_host) return fail(GSVC_RAST_ERR_INVALID, "counts_host is NULL");
+    long long total = 0;
+    for (int v = 0; v < n_views; v++) {
+        if (counts_host[v] < 0) return fail(GSVC_RAST_ERR_INVALID, "count of view %d is %d, expected >= 0", v, counts_host[v]);
+        total += counts_host[v];
+        if (total > 0x7fffffffll) return fail(GSVC_RAST_ERR_INVALID, "the views' counts sum to more than 2^31 - 1 rows");
+        d.rows.off[v + 1] = (int)total;
+    }
+    d.ragged = 1;
+    P = (int32_t)total;
     return 0;
 }
 
@@ -288,10 +309,10 @@ static int forward_launch_core(const gsvc_rast_settings* st, const DevSettings& 
     if (!geom || !image || !out_color || (P > 0 && !radii))
         return fail(GSVC_RAST_ERR_INVALID, "geom/image/out_color/radii must be non-NULL");
     if (capacity > 0 && !binning) return fail(GSVC_RAST_ERR_INVALID, "binning is NULL");
-    if ((long long)P * d.n_views > 0x7fffffffll) return fail(GSVC_RAST_ERR_INVALID, "P * n_views exceeds 31 bits");
+    if (!d.ragged && (long long)P * d.n_views > 0x7fffffffll)
+        return fail(GSVC_RAST_ERR_INVALID, "P * n_views exceeds 31 bits");
     const bool dbg = st->debug != 0;
-    const int PV = (P < 1 ? 1 : P) * d.n_views;
-    GeomView g = geom_view(geom, PV, d.sh_M);
+    GeomView g = geom_view(geom, state_rows(d, P < 1 ? 1 : P), d.sh_M);
     ImageView im = image_view(image, d.W, d.H, d.n_views);
     PreInputs in{P, means3D, shs, colors_precomp, opacities, scales, rotations, cov3D_precomp, 0, P};
     if (d.accumulate)   // views that share an output image add into it
@@ -396,7 +417,7 @@ static int forward_render_core(const gsvc_rast_settings* st, const DevSettings& 
         return fail(GSVC_RAST_ERR_INVALID, "geom/image/binning/out_color must be non-NULL and capacity > 0");
     const bool dbg = st->debug != 0;
     // sh_M only affects the tail of the geom layout (clamp flags), which these stages never touch
-    GeomView g = geom_view(const_cast<void*>(geom), (P < 1 ? 1 : P) * d.n_views, 0);
+    GeomView g = geom_view(const_cast<void*>(geom), state_rows(d, P < 1 ? 1 : P), 0);
     ImageView im = image_view(image, d.W, d.H, d.n_views);
     // the scatter cursors were consumed by a previous attempt: reset them
     CK(cudaMemsetAsync(im.tile_cursor, 0, (size_t)d.gx * d.gy * d.n_views * sizeof(unsigned int), stream), "cursor reset");
@@ -478,12 +499,12 @@ static int backward_core(const gsvc_rast_settings* st, const DevSettings& d, int
     if (out.packed && (shs || cov3D_precomp))
         return fail(GSVC_RAST_ERR_INVALID, "dL_packed needs colors_precomp and the scale/rotation pair");
     const bool dbg = st->debug != 0;
-    GeomView g = geom_view(const_cast<void*>(geom), (P < 1 ? 1 : P) * d.n_views, d.sh_M);
+    GeomView g = geom_view(const_cast<void*>(geom), state_rows(d, P < 1 ? 1 : P), d.sh_M);
     ImageView im = image_view(const_cast<void*>(image), d.W, d.H, d.n_views);
     BinView b = bin_view(const_cast<void*>(binning), capacity);
     float4* acc = static_cast<float4*>(scratch);
     PreInputs in{P, means3D, shs, colors_precomp, nullptr, scales, rotations, cov3D_precomp, 0, P};
-    { StageScope t(ST_RENDER_BWD, stream); CK(launch_render_backward(d, P, g, im, b, capacity, dL_dout, acc, scratch_is_zero != 0, stream), "render_backward"); }
+    { StageScope t(ST_RENDER_BWD, stream); CK(launch_render_backward(d, state_rows(d, P), g, im, b, capacity, dL_dout, acc, scratch_is_zero != 0, stream), "render_backward"); }
     { StageScope t(ST_PREPROCESS_BWD, stream); CK(launch_preprocess_backward(d, in, radii, g, acc, out, ex, stream), "preprocess_backward"); }
     return 0;
 }
@@ -571,6 +592,53 @@ int gsvc_rast_backward_views_exchange(const gsvc_rast_settings* st, int32_t n_vi
     return backward_core(st, d, P, sh_M, capacity, means3D, shs, colors_precomp, scales, rotations, cov3D_precomp, radii,
                          geom, image, binning, scratch, scratch_is_zero, dL_dout, out, static_cast<cudaStream_t>(stream_),
                          ex);
+}
+
+int gsvc_rast_forward_ragged_launch(const gsvc_rast_settings* st, int32_t n_views, const gsvc_rast_view* views_host,
+                                    int32_t n_out, const int32_t* counts_host, int32_t sh_M, const float* means3D,
+                                    const float* shs, const float* colors_precomp, const float* opacities,
+                                    const float* scales, const float* rotations, const float* cov3D_precomp, void* geom,
+                                    void* image, void* binning, int64_t capacity, void* bwd_scratch, float* out_color,
+                                    int32_t* radii, uint64_t* count_slot_host, uint32_t ticket, void* stream_)
+{
+    DevSettings d;
+    int32_t P = 0;
+    int rc = make_settings_ragged(st, n_views, views_host, n_out, counts_host, shs ? sh_M : 0, d, P);
+    if (rc) return rc;
+    return forward_launch_core(st, d, n_out, P, sh_M, means3D, shs, colors_precomp, opacities, scales, rotations,
+                               cov3D_precomp, geom, image, binning, capacity, bwd_scratch, out_color, radii,
+                               count_slot_host, ticket, static_cast<cudaStream_t>(stream_));
+}
+
+int gsvc_rast_forward_ragged_render(const gsvc_rast_settings* st, int32_t n_views, const gsvc_rast_view* views_host,
+                                    int32_t n_out, const int32_t* counts_host, const void* geom, void* image,
+                                    void* binning, int64_t capacity, float* out_color, void* stream_)
+{
+    DevSettings d;
+    int32_t P = 0;
+    int rc = make_settings_ragged(st, n_views, views_host, n_out, counts_host, 0, d, P);
+    if (rc) return rc;
+    return forward_render_core(st, d, n_out, P, geom, image, binning, capacity, out_color,
+                               static_cast<cudaStream_t>(stream_));
+}
+
+int gsvc_rast_backward_ragged(const gsvc_rast_settings* st, int32_t n_views, const gsvc_rast_view* views_host,
+                              int32_t n_out, const int32_t* counts_host, int32_t sh_M, int64_t capacity,
+                              const float* means3D, const float* shs, const float* colors_precomp, const float* scales,
+                              const float* rotations, const float* cov3D_precomp, const int32_t* radii,
+                              const void* geom, const void* image, const void* binning, void* scratch,
+                              int32_t scratch_is_zero, const float* dL_dout, float* dL_dmeans3D, float* dL_dmeans2D,
+                              float* dL_dcolors, float* dL_dopacities, float* dL_dscales, float* dL_drotations,
+                              float* dL_dcov3D, float* dL_dshs, void* stream_)
+{
+    DevSettings d;
+    int32_t P = 0;
+    int rc = make_settings_ragged(st, n_views, views_host, n_out, counts_host, shs ? sh_M : 0, d, P);
+    if (rc) return rc;
+    BwdOutputs out{dL_dmeans3D, dL_dmeans2D, dL_dcolors, dL_dopacities, dL_dscales, dL_drotations, dL_dcov3D, dL_dshs,
+                   nullptr};
+    return backward_core(st, d, P, sh_M, capacity, means3D, shs, colors_precomp, scales, rotations, cov3D_precomp, radii,
+                         geom, image, binning, scratch, scratch_is_zero, dL_dout, out, static_cast<cudaStream_t>(stream_));
 }
 
 int gsvc_rast_export_keys(const gsvc_rast_settings* st, int32_t n_views, int64_t capacity, const void* image,

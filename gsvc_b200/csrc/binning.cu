@@ -127,17 +127,22 @@ cudaError_t read_overflow_events(unsigned int* host_value, bool reset, cudaStrea
     return e;
 }
 
+// RAGGED: view v's Gaussians are rows rows.off[v] .. rows.off[v+1]-1 (virtual Gaussian = row); the grid is
+// (ceil(max_v P_v / 256), n_views) and a CTA wholly past its view's rows leaves at once
+template <bool RAGGED>
 __global__ void __launch_bounds__(256) scatter_kernel(int P, int gx, int Tv, GeomView geo, ImageView im, BinView bin,
-                                                      unsigned long long cap, int count_events)
+                                                      unsigned long long cap, int count_events, ViewRows rows)
 {
     pdl_prologue();
+    const int v = blockIdx.y;                       // view of the batch: virtual Gaussian v*P + g, tiles v*Tv + t
+    const int Pv = RAGGED ? rows.off[v + 1] - rows.off[v] : P;
+    if (RAGGED && (int)(blockIdx.x * blockDim.x) >= Pv) return;
     const int g = blockIdx.x * blockDim.x + threadIdx.x;
     const int lane = threadIdx.x & 31;
-    const int v = blockIdx.y;                       // view of the batch: virtual Gaussian v*P + g, tiles v*Tv + t
-    const size_t gv = (size_t)v * P + g;
+    const size_t gv = RAGGED ? (size_t)rows.off[v] + g : (size_t)v * P + g;
     const int tbase = v * Tv;
     ushort4 r = make_ushort4(0, 0, 0, 0);
-    if (g < P) r = geo.rect[gv];
+    if (g < Pv) r = geo.rect[gv];
     const int w = (int)r.z - (int)r.x, h = (int)r.w - (int)r.y;
     const int area = (w > 0 && h > 0) ? w * h : 0;
     unsigned long long item = 0ull;
@@ -174,10 +179,12 @@ __global__ void __launch_bounds__(256) scatter_kernel(int P, int gx, int Tv, Geo
 cudaError_t launch_scatter(const DevSettings& s, int P, GeomView g, ImageView im, BinView b, long long cap,
                            bool count_overflow_events, cudaStream_t st)
 {
-    if (P <= 0) return cudaSuccess;
+    const int Pmax = max_view_rows(s, P);
+    if (Pmax <= 0) return cudaSuccess;
     count_launch();
-    return launch_pdl(scatter_kernel, dim3((P + 255) / 256, s.n_views), dim3(256), st, P, s.gx, s.gx * s.gy, g, im, b,
-                      (unsigned long long)cap, count_overflow_events ? 1 : 0);
+    return launch_pdl(s.ragged ? scatter_kernel<true> : scatter_kernel<false>, dim3((Pmax + 255) / 256, s.n_views),
+                      dim3(256), st, P, s.gx, s.gx * s.gy, g, im, b, (unsigned long long)cap,
+                      count_overflow_events ? 1 : 0, s.rows);
 }
 
 // ---- per-tile sort of the 64-bit composites -----------------------------------------------------

@@ -31,6 +31,13 @@ struct ViewTable {
     float weight[MAX_VIEWS];             // out[out_image] += weight * view  (1 for a plain view, 0.5 for a toast half)
 };
 
+// A per-view-set ("ragged") batch: every view has Gaussians of its own, concatenated in view order.  View v owns rows
+// off[v] .. off[v+1]-1 of the inputs, and the virtual Gaussian is the row itself (tiles stay v*Tv + t).  By value in the
+// launch parameters (68 bytes), so a ragged chain needs no device table.
+struct ViewRows {
+    int off[MAX_VIEWS + 1];
+};
+
 // Settings as the kernels see them (passed by value in the launch parameters).
 struct DevSettings {
     int W, H, gx, gy;
@@ -39,7 +46,20 @@ struct DevSettings {
     int sh_degree, sh_M;
     int n_views, accumulate;   // accumulate: several views share an output image (atomic adds onto a zeroed image)
     ViewTable vt;
+    int ragged;                // 0: one Gaussian set shared by every view (virtual Gaussian v*P + g); 1: `rows`
+    ViewRows rows;
 };
+
+// Rows of the per-Gaussian state (geom, accumulators, radii) of a call with P input Gaussians (the total of the views'
+// counts when ragged), and the most rows any one view has (the x extent of the per-view kernel grids).
+inline int state_rows(const DevSettings& d, int P) { return d.ragged ? P : P * d.n_views; }
+inline int max_view_rows(const DevSettings& d, int P)
+{
+    if (!d.ragged) return P;
+    int m = 0;
+    for (int v = 0; v < d.n_views; v++) m = d.rows.off[v + 1] - d.rows.off[v] > m ? d.rows.off[v + 1] - d.rows.off[v] : m;
+    return m;
+}
 
 // ---- per-Gaussian state ("geom") -------------------------------------------------------------
 //  feat0 = (pix.x, pix.y, rho_hi, B/C)   rho = B/A as rho_hi + rho_lo (fp64 quotient split into two floats); the two
@@ -335,7 +355,7 @@ __device__ __forceinline__ int warp_tiles_get(const WarpTiles& w, int idx, int g
 
 // ---- launch stages implemented in the .cu files ------------------------------------------------
 struct PreInputs {
-    int P;
+    int P;                     // Gaussians of the shared set, or rows of a ragged batch (all views)
     const float* means3D;
     const float* shs;
     const float* colors_precomp;
@@ -367,7 +387,7 @@ cudaError_t launch_scatter(const DevSettings& s, int P, GeomView g, ImageView im
 cudaError_t launch_sort_tiles(const DevSettings& s, ImageView im, BinView b, long long cap, cudaStream_t st);
 cudaError_t launch_render_forward(const DevSettings& s, GeomView g, ImageView im, BinView b, long long cap,
                                   float* out_color, cudaStream_t st);
-cudaError_t launch_render_backward(const DevSettings& s, int P, GeomView g, ImageView im, BinView b, long long cap,
+cudaError_t launch_render_backward(const DevSettings& s, int rows, GeomView g, ImageView im, BinView b, long long cap,
                                    const float* dL_dout, float4* acc, bool acc_is_zero, cudaStream_t st);
 struct BwdOutputs {
     float* dL_dmeans3D; float* dL_dmeans2D; float* dL_dcolors; float* dL_dopacities;   // dL_dmeans2D is [n_views,P,3]

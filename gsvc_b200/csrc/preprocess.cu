@@ -134,17 +134,21 @@ __global__ void __launch_bounds__(256) compact_write_kernel(int P, const unsigne
 
 // MODE 0: full preprocess + per-tile instance counting.  MODE 1: visible_filter (radii only).
 // MODE 2: visible_filter + stable compaction of the visible indices.
-template <int MODE>
+// RAGGED (MODE 0 only): every view has its own rows (s.rows); the grid is (ceil(max_v P_v / 256), n_views).
+template <int MODE, bool RAGGED = false>
 __global__ void __launch_bounds__(256) preprocess_kernel(DevSettings s, PreInputs in, int32_t* __restrict__ radii,
                                                          GeomView geo, unsigned int* __restrict__ tile_count,
                                                          float4* __restrict__ acc_to_zero, CompactOut co)
 {
     constexpr bool FILTER = MODE != 0;
     pdl_prologue();
+    // Gaussians of this view: the shared set's P, or the view's own count (a CTA wholly past it has nothing to do)
+    const int Pv = RAGGED ? s.rows.off[blockIdx.y + 1] - s.rows.off[blockIdx.y] : in.P;
+    if (RAGGED && (int)(blockIdx.x * blockDim.x) >= Pv) return;
     // Lanes past the end stay in the warp (they redo the last Gaussian with all stores masked) so that the
     // warp-wide tile walk at the end (and the block-wide compaction) runs converged.
     const int g_raw = blockIdx.x * blockDim.x + threadIdx.x;
-    bool valid = g_raw < in.P;
+    bool valid = g_raw < Pv;
     if (FILTER) {
         // Slab-ordered anchors (SURVEY.md §8f row f4; the reference's stream codec keeps them z-sorted in 0.01
         // intervals, utils/encodings.py:827-862): only indices in [range_lo, range_hi) can be inside the TSW slab.
@@ -161,18 +165,21 @@ __global__ void __launch_bounds__(256) preprocess_kernel(DevSettings s, PreInput
         }
     }
     const bool in_range = !FILTER || (g_raw >= in.range_lo && g_raw < in.range_hi);
-    const int g = valid ? (in_range ? g_raw : min(max(g_raw, in.range_lo), in.range_hi - 1)) : in.P - 1;
-    // view of the batch (grid.y): per-Gaussian state of view v lives at virtual index v*P + g, its tiles at v*Tv + t
+    const int g = valid ? (in_range ? g_raw : min(max(g_raw, in.range_lo), in.range_hi - 1)) : Pv - 1;
+    // view of the batch (grid.y)
     const int v = FILTER ? 0 : (int)blockIdx.y;
-    const size_t gv = (size_t)v * in.P + g;
-    const float p[3] = {__ldg(in.means3D + 3 * g), __ldg(in.means3D + 3 * g + 1), __ldg(in.means3D + 3 * g + 2)};
+    // row of the inputs: g of the shared set, or the view's own row off_v + g.  Per-Gaussian state of view v lives
+    // at virtual index v*P + g (shared) or at that row (ragged), its tiles at v*Tv + t
+    const int gp = RAGGED ? s.rows.off[v] + g : g;
+    const size_t gv = RAGGED ? (size_t)gp : (size_t)v * in.P + g;
+    const float p[3] = {__ldg(in.means3D + 3 * gp), __ldg(in.means3D + 3 * gp + 1), __ldg(in.means3D + 3 * gp + 2)};
     // scales / quaternion are fetched together with the position (one memory round trip per Gaussian, at the
     // price of 28 wasted bytes for the third of the Gaussians the slab test culls)
     float sc[3] = {0.f, 0.f, 0.f};
     float4 q_pre = make_float4(1.f, 0.f, 0.f, 0.f);
     if (!in.cov3D_precomp) {
-        sc[0] = __ldg(in.scales + 3 * g); sc[1] = __ldg(in.scales + 3 * g + 1); sc[2] = __ldg(in.scales + 3 * g + 2);
-        q_pre = ld_row4(in.rotations, (size_t)g);
+        sc[0] = __ldg(in.scales + 3 * gp); sc[1] = __ldg(in.scales + 3 * gp + 1); sc[2] = __ldg(in.scales + 3 * gp + 2);
+        q_pre = ld_row4(in.rotations, (size_t)gp);
     }
     // The CTA's view matrix (strided device tensor: 12 loads + 64-bit stride arithmetic per thread otherwise) is
     // fetched once by 12 threads and broadcast through shared memory; the Gaussian's own loads above are already
@@ -195,7 +202,7 @@ __global__ void __launch_bounds__(256) preprocess_kernel(DevSettings s, PreInput
         float cov[6];
         if (in.cov3D_precomp) {
 #pragma unroll
-            for (int k = 0; k < 6; k++) cov[k] = __ldg(in.cov3D_precomp + 6 * (size_t)g + k);
+            for (int k = 0; k < 6; k++) cov[k] = __ldg(in.cov3D_precomp + 6 * (size_t)gp + k);
         } else {
             cov3d_from_scale_rot(sc, s.scale_modifier, q_pre, cov);
         }
@@ -238,16 +245,16 @@ __global__ void __launch_bounds__(256) preprocess_kernel(DevSettings s, PreInput
     if (ok) {
         const float det_inv = 1.f / det;
         const float cA = c * det_inv, cB = -b * det_inv, cC = a * det_inv;
-        const float op = __ldg(in.opacities + g);
+        const float op = __ldg(in.opacities + gp);
         float rgb[3];
         if (in.colors_precomp) {
-            rgb[0] = __ldg(in.colors_precomp + 3 * g);
-            rgb[1] = __ldg(in.colors_precomp + 3 * g + 1);
-            rgb[2] = __ldg(in.colors_precomp + 3 * g + 2);
+            rgb[0] = __ldg(in.colors_precomp + 3 * gp);
+            rgb[1] = __ldg(in.colors_precomp + 3 * gp + 1);
+            rgb[2] = __ldg(in.colors_precomp + 3 * gp + 2);
         } else {
             uint8_t cl[3];
             const float campos[3] = {s.vt.campos[v][0], s.vt.campos[v][1], s.vt.campos[v][2]};
-            sh_to_rgb(s.sh_degree, in.shs + (size_t)g * s.sh_M * 3, p, campos, rgb, cl);
+            sh_to_rgb(s.sh_degree, in.shs + (size_t)gp * s.sh_M * 3, p, campos, rgb, cl);
             geo.clamped[3 * gv] = cl[0];
             geo.clamped[3 * gv + 1] = cl[1];
             geo.clamped[3 * gv + 2] = cl[2];
@@ -359,10 +366,12 @@ cudaError_t launch_preprocess(const DevSettings& s, const PreInputs& in, int32_t
     const size_t nbytes = reinterpret_cast<char*>(im.scan_partials + (T / 1024 + 2)) - reinterpret_cast<char*>(im.tile_count);
     cudaError_t e = cudaMemsetAsync(im.tile_count, 0, nbytes, st);
     if (e != cudaSuccess) return e;
-    if (in.P <= 0) return cudaSuccess;
+    const int Pmax = max_view_rows(s, in.P);
+    if (Pmax <= 0) return cudaSuccess;
     count_launch();
-    return launch_pdl(preprocess_kernel<0>, dim3((in.P + 255) / 256, s.n_views), dim3(256), st, s, in, radii, g,
-                      im.tile_count, acc_to_zero, CompactOut{});
+    return launch_pdl(s.ragged ? preprocess_kernel<0, true> : preprocess_kernel<0, false>,
+                      dim3((Pmax + 255) / 256, s.n_views), dim3(256), st, s, in, radii, g, im.tile_count, acc_to_zero,
+                      CompactOut{});
 }
 
 }  // namespace gsvc

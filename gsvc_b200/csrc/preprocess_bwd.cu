@@ -84,9 +84,13 @@ __device__ void sh_backward(int deg, int M, const float* sh, float* dsh, const f
     dmean[2] += (ddz - z * dot) / len;
 }
 
+// g: the parameter row.  Shared set (RAGGED false): the views' states at v*P + g, summed over the views.  Ragged: row g
+// belongs to `view` alone, and its state is at row g itself.
+template <bool RAGGED>
 __device__ __forceinline__ void gaussian_backward(const DevSettings& s, const PreInputs& in,
                                                   const int32_t* __restrict__ radii, const GeomView& geo,
-                                                  const float4* __restrict__ acc, const BwdOutputs& out, const int g)
+                                                  const float4* __restrict__ acc, const BwdOutputs& out, const int g,
+                                                  const int view)
 {
     float dmean[3] = {0.f, 0.f, 0.f}, dcol[3] = {0.f, 0.f, 0.f}, dop = 0.f;
     float dsc[3] = {0.f, 0.f, 0.f}, drot[4] = {0.f, 0.f, 0.f, 0.f}, dcov[6] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
@@ -96,9 +100,9 @@ __device__ __forceinline__ void gaussian_backward(const DevSettings& s, const Pr
     }
 
     // A batch of views shares the Gaussian parameters: their gradients are summed here, in view order, so the
-    // batch writes ONE dense gradient instead of n_views of them plus the adds.
-    for (int v = 0; v < s.n_views; v++) {
-    const size_t gv = (size_t)v * in.P + g;
+    // batch writes ONE dense gradient instead of n_views of them plus the adds.  A ragged row has one view: no sum.
+    for (int v = RAGGED ? view : 0; v < (RAGGED ? view + 1 : s.n_views); v++) {
+    const size_t gv = RAGGED ? (size_t)g : (size_t)v * in.P + g;
     const bool vis = radii[gv] > 0;
     float dm2[2] = {0.f, 0.f};
     if (vis) {
@@ -254,19 +258,27 @@ __device__ __forceinline__ void gaussian_backward(const DevSettings& s, const Pr
 // frame-sharded step and live in symmetric memory) the first ex.n_ex CTAs of the launch do not compute: they sum the rows
 // over the ranks chunk by chunk while the other CTAs are still producing the later chunks (collective.cuh), so the
 // launch ends with the all-reduced buffer in place and most of the transfer hidden under the computation.
+// RAGGED: grid (ceil(max_v P_v / 128), n_views), thread i of view v handles row off_v + i for i < P_v; never an exchange.
+template <bool RAGGED>
 __global__ void __launch_bounds__(256,2) preprocess_backward_kernel(DevSettings s, PreInputs in,
                                                                   const int32_t* __restrict__ radii, GeomView geo,
                                                                   const float4* __restrict__ acc, BwdOutputs out,
                                                                   ExchangeArgs ex)
 {
     pdl_prologue();
+    if (RAGGED) {
+        const int v = blockIdx.y, lo = s.rows.off[v];
+        const int i = blockIdx.x * blockDim.x + threadIdx.x;
+        if (i < s.rows.off[v + 1] - lo) gaussian_backward<true>(s, in, radii, geo, acc, out, lo + i, v);
+        return;
+    }
     if (ex.n_ex > 0 && (int)blockIdx.x < ex.n_ex) {
         exchange_role(ex);
         return;
     }
     const int cta = (int)blockIdx.x - ex.n_ex;
     const int g = cta * blockDim.x + threadIdx.x;
-    if (g < in.P) gaussian_backward(s, in, radii, geo, acc, out, g);
+    if (g < in.P) gaussian_backward<false>(s, in, radii, geo, acc, out, g, 0);
     if (ex.n_ex > 0) {
         // device-scope only: a system-scope fence in each of the ~P/128 CTAs cost 100 us per launch.  The chain to the
         // peers is closed by the coordinator CTA: it acquires the chunk's count (device scope), fences at system scope
@@ -282,8 +294,14 @@ cudaError_t launch_preprocess_backward(const DevSettings& s, const PreInputs& in
 {
     if (in.P <= 0) return cudaSuccess;
     count_launch();
+    if (s.ragged) {
+        const int Pmax = max_view_rows(s, in.P);
+        return launch_pdl(preprocess_backward_kernel<true>, dim3((Pmax + 127) / 128, s.n_views), dim3(128), st, s, in,
+                          radii, g, acc, out, ExchangeArgs{});
+    }
     const int n_compute = (in.P + 127) / 128;
-    return launch_pdl(preprocess_backward_kernel, dim3(n_compute + ex.n_ex), dim3(128), st, s, in, radii, g, acc, out, ex);
+    return launch_pdl(preprocess_backward_kernel<false>, dim3(n_compute + ex.n_ex), dim3(128), st, s, in, radii, g, acc,
+                      out, ex);
 }
 
 // Densification statistic at the rasterizer boundary (scene/gaussian_model.py:1298-1314 `training_statis`, called

@@ -572,15 +572,15 @@ render_backward_kernel(DevSettings s, GeomView geo, ImageView im, BinView bin, u
 }
 
 
-cudaError_t launch_render_backward(const DevSettings& s, int P, GeomView g, ImageView im, BinView b, long long cap,
+cudaError_t launch_render_backward(const DevSettings& s, int rows, GeomView g, ImageView im, BinView b, long long cap,
                                    const float* dL_dout, float4* acc, bool acc_is_zero, cudaStream_t st)
 {
     if (!acc_is_zero) {
-        cudaError_t e = cudaMemsetAsync(acc, 0, (size_t)P * s.n_views * 48, st);
+        cudaError_t e = cudaMemsetAsync(acc, 0, (size_t)rows * 48, st);
         if (e != cudaSuccess) return e;
     }
     const int T = s.gx * s.gy * s.n_views;
-    if (T <= 0 || P <= 0) return cudaSuccess;
+    if (T <= 0 || rows <= 0) return cudaSuccess;
     count_launch();
     return launch_pdl(render_backward_kernel, dim3(T), dim3(BWD_THREADS), st, s, g, im, b, (unsigned long long)cap,
                       dL_dout, reinterpret_cast<float*>(acc));

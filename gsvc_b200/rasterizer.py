@@ -13,7 +13,9 @@ plumbing.  There is no CPU / eager fallback: CPU tensors raise.
 
 The drop-in call and views.rasterize_views share one autograd Function: a drop-in call is a batch of
 one view through the batched entry points (gsvc_rast_forward_views_launch, + gsvc_rast_forward_views_render
-on overflow; gsvc_rast_backward_views), the same kernels and buffer sizes as the single-view entry points.
+on overflow; gsvc_rast_backward_views), the same kernels and buffer sizes as the single-view entry points.  A batch
+over per-view Gaussian sets (rasterize_views(..., counts=...)) goes through the same Function and the
+gsvc_rast_*_ragged entry points.
 """
 from __future__ import annotations
 
@@ -47,14 +49,16 @@ class GaussianRasterizationSettings(NamedTuple):
 
 # Instance-capacity prediction, so that the binning buffer can be sized — and scatter / sort / blend launched — before
 # the instance count of THIS call is known (no mid-pipeline host synchronisation):
-#   _capacity_hint[(device, P, H, W, V)]    the last num_rendered seen for exactly this shape (CUDA-graph capture
-#                                           requires it: a replay's capacity is fixed);
-#   _density_hint[(device, H, W, V)]        instances per INPUT Gaussian at this image size, a slowly decaying
+#   _capacity_hint[(device, P, H, W, V, ragged)]  the last num_rendered seen for exactly this shape (CUDA-graph
+#                                           capture requires it: a replay's capacity is fixed);
+#   _density_hint[(device, H, W, V, ragged)]  instances per INPUT Gaussian at this image size, a slowly decaying
 #                                           maximum.  The reference's render() hands over a different P on every
 #                                           call (the Gaussians of the anchors visible in THAT view,
 #                                           ortho_gaussian_renderer/renderer.py:28-37), so an exact-shape hint never
 #                                           hits there; the density of instances per Gaussian, however, is a
 #                                           property of the scene's scale distribution and moves slowly.
+#                                           A shared set's input Gaussian is drawn in every view, a ragged batch's
+#                                           row in one: the two densities differ by about V, hence the mode in keys.
 _capacity_hint: dict = {}
 _density_hint: dict = {}
 _count_slots = threading.local()
@@ -63,9 +67,10 @@ _count_slots = threading.local()
 capacity_stats = {"calls": 0, "rerendered": 0, "cold": 0}
 
 
-def _capacity_keys(dev: Optional[int], P: int, H: int, W: int, n_views: int):
-    """(exact-shape key, density key) of a call of `n_views` views on device index `dev`; a drop-in call is one view."""
-    return (dev, P, H, W, n_views), (dev, H, W, n_views)
+def _capacity_keys(dev: Optional[int], P: int, H: int, W: int, n_views: int, ragged: bool = False):
+    """(exact-shape key, density key) of a call of `n_views` views on device index `dev`; a drop-in call is one view.
+    `ragged`: the views have Gaussian sets of their own (P is then the total of their counts)."""
+    return (dev, P, H, W, n_views, ragged), (dev, H, W, n_views, ragged)
 
 
 def _predict_capacity(key_exact, key_density, P: int):
@@ -307,25 +312,30 @@ def _check_modes(scales, rotations, cov3D_precomp, colours=None):
         raise Exception("Please provide exactly one of either scale/rotation pair or precomputed 3D covariance!")
 
 
-def _snapshot_settings(rs, batch) -> tuple:
+def _snapshot_settings(rs, batch, counts=None) -> tuple:
     """The settings part of a debug snapshot: upstream's tuple(raster_settings) for a drop-in call, the views and
-    their image map for a batch."""
+    their image map for a batch (and the views' counts for a ragged one)."""
     if batch is None:
         return (tuple(rs),)
-    return ([tuple(x) for x in batch.settings], batch.out_image, batch.flip_x, batch.weight)
+    return ([tuple(x) for x in batch.settings], batch.out_image, batch.flip_x, batch.weight, counts)
 
 
 class _RasterizeViews(torch.autograd.Function):
     """One kernel chain over the views of `batch` (a views.ViewBatch), or over the single view `rs` of a drop-in call
     (`batch` None).  A drop-in call differs in two things only: its outputs have upstream's shapes (image [3,H,W],
-    radii [P], means2D gradient [P,3]), and its backward never carries the exchange of sharding.packed_backward."""
+    radii [P], means2D gradient [P,3]), and its backward never carries the exchange of sharding.packed_backward.
+    `counts` (a batch only; tuple of n_views ints, validated by views.rasterize_views): the inputs are the views' own
+    Gaussian sets concatenated in view order; radii and the means2D gradient then have one row per input row, and
+    the backward never takes a packed_backward target."""
 
     @staticmethod
-    def forward(ctx, means3D, means2D, sh, colors_precomp, opacities, scales, rotations, cov3Ds_precomp, rs, batch):
+    def forward(ctx, means3D, means2D, sh, colors_precomp, opacities, scales, rotations, cov3Ds_precomp, rs, batch,
+                counts=None):
         L = _lib.lib()
         _require_cuda(means3D, "means3D")
         device = means3D.device
         single = batch is None
+        ragged = counts is not None
         with _on_device(device):
             # the reference builds new settings on every render(): the drop-in's descriptor is built per call
             nv = _NativeViews(None, device, rs) if single else batch.native(device)
@@ -342,7 +352,9 @@ class _RasterizeViews(torch.autograd.Function):
             sh_M = sh_c.shape[1] if sh_c is not None else 0
             H, W = int(rs.image_height), int(rs.image_width)
 
-            hint_key, dens_key = _capacity_keys(device.index, P, H, W, V)
+            rows = P if ragged else P * V      # rows of the per-Gaussian state
+            counts_c = (C.c_int32 * V)(*counts) if ragged else None
+            hint_key, dens_key = _capacity_keys(device.index, P, H, W, V, ragged)
             cap, hint = _predict_capacity(hint_key, dens_key, P)
             # CUDA-graph capture (torch.cuda.graph around the caller's step): nothing may wait on the device, so
             # the instance count of the last eager call stands in for num_rendered and the binning capacity is
@@ -357,9 +369,9 @@ class _RasterizeViews(torch.autograd.Function):
                 cap = slot.capacity = int(hint * 1.5) + 65536
             # one allocation for all native state: [geom | image | backward accumulators | binning]
             need_grad = any(ctx.needs_input_grad)
-            n_geom = _align(L.gsvc_rast_geom_bytes(P * V, sh_M))
+            n_geom = _align(L.gsvc_rast_geom_bytes(rows, sh_M))
             n_img = _align(L.gsvc_rast_image_bytes_views(W, H, V))
-            n_acc = _align(L.gsvc_rast_backward_scratch_bytes(P * V)) if need_grad else 0
+            n_acc = _align(L.gsvc_rast_backward_scratch_bytes(rows)) if need_grad else 0
             n_bin = L.gsvc_rast_binning_bytes(cap) if cap > 0 else 0
             state = _bytes(n_geom + n_img + n_acc + n_bin, device)
             base = state.data_ptr()
@@ -370,14 +382,20 @@ class _RasterizeViews(torch.autograd.Function):
             # outputs allocated in the caller's shape: indexing a batch of one would put a select node (and its
             # image-sized zero fill) into every backward
             color = torch.empty((3, H, W) if single else (n_out, 3, H, W), dtype=_F32, device=device)
-            radii = torch.empty((P,) if single else (V, P), dtype=torch.int32, device=device)
+            radii = torch.empty((P,) if single or ragged else (V, P), dtype=torch.int32, device=device)
             stream = _stream_ptr(device)
             try:
                 L.gsvc_rast_count_overflows(1 if capturing else 0)   # a replay has nobody to re-run it; eager does
-                _lib.check(L.gsvc_rast_forward_views_launch(
-                    nv.ref, V, nv.views, n_out, P, sh_M, _ptr(means3D_c), _ptr(sh_c), _ptr(col_c), _ptr(op_c),
-                    _ptr(sc_c), _ptr(rot_c), _ptr(cov_c), geom_p, image_p, bin_p, cap, acc_p, color.data_ptr(),
-                    radii.data_ptr(), slot.ptr, ticket, stream), "gsvc_rast_forward_views_launch")
+                if ragged:
+                    _lib.check(L.gsvc_rast_forward_ragged_launch(
+                        nv.ref, V, nv.views, n_out, counts_c, sh_M, _ptr(means3D_c), _ptr(sh_c), _ptr(col_c),
+                        _ptr(op_c), _ptr(sc_c), _ptr(rot_c), _ptr(cov_c), geom_p, image_p, bin_p, cap, acc_p,
+                        color.data_ptr(), radii.data_ptr(), slot.ptr, ticket, stream), "gsvc_rast_forward_ragged_launch")
+                else:
+                    _lib.check(L.gsvc_rast_forward_views_launch(
+                        nv.ref, V, nv.views, n_out, P, sh_M, _ptr(means3D_c), _ptr(sh_c), _ptr(col_c), _ptr(op_c),
+                        _ptr(sc_c), _ptr(rot_c), _ptr(cov_c), geom_p, image_p, bin_p, cap, acc_p, color.data_ptr(),
+                        radii.data_ptr(), slot.ptr, ticket, stream), "gsvc_rast_forward_views_launch")
                 # The reference API returns num_rendered as a Python int (renderer.py:90).  The scan kernel
                 # publishes it into pinned memory as soon as it is known, so this wait ends while the
                 # scatter / sort / blend kernels are still running: no stream synchronisation.
@@ -395,19 +413,24 @@ class _RasterizeViews(torch.autograd.Function):
                     cap = max(num_rendered, 1)
                     binning = _bytes(L.gsvc_rast_binning_bytes(cap), device)
                     bin_p = binning.data_ptr()
-                    _lib.check(L.gsvc_rast_forward_views_render(nv.ref, V, nv.views, n_out, P, geom_p, image_p, bin_p,
-                                                                cap, color.data_ptr(), stream),
-                               "gsvc_rast_forward_views_render")
+                    if ragged:
+                        _lib.check(L.gsvc_rast_forward_ragged_render(nv.ref, V, nv.views, n_out, counts_c, geom_p,
+                                                                     image_p, bin_p, cap, color.data_ptr(), stream),
+                                   "gsvc_rast_forward_ragged_render")
+                    else:
+                        _lib.check(L.gsvc_rast_forward_views_render(nv.ref, V, nv.views, n_out, P, geom_p, image_p,
+                                                                    bin_p, cap, color.data_ptr(), stream),
+                                   "gsvc_rast_forward_views_render")
                 if not capturing:
                     _record_capacity(hint_key, dens_key, P, num_rendered)
             except Exception:
                 if rs.debug:
                     torch.save((means3D, sh, colors_precomp, opacities, scales, rotations, cov3Ds_precomp)
-                               + _snapshot_settings(rs, batch), "snapshot_fw.dump")
+                               + _snapshot_settings(rs, batch, counts), "snapshot_fw.dump")
                     print("\nAn error occured in forward. Please forward snapshot_fw.dump for debugging.")
                 raise
 
-        ctx.rs, ctx.batch, ctx.nv = rs, batch, nv
+        ctx.rs, ctx.batch, ctx.nv, ctx.counts, ctx.counts_c = rs, batch, nv, counts, counts_c
         ctx.sh_M, ctx.capacity = sh_M, cap
         ctx.offsets = (n_geom, n_img, n_acc)
         ctx.save_for_backward(means3D_c, sh_c, col_c, sc_c, rot_c, cov_c, radii, state, binning)
@@ -417,11 +440,12 @@ class _RasterizeViews(torch.autograd.Function):
     @staticmethod
     def backward(ctx, grad_out_color, _grad_radii=None, _grad_num=None):
         L = _lib.lib()
-        nv, single = ctx.nv, ctx.batch is None
+        nv, single, ragged = ctx.nv, ctx.batch is None, ctx.counts is not None
         V, n_out = nv.n_views, nv.n_out
         means3D, sh, col, sc, rot, cov, radii, state, binning = ctx.saved_tensors
         device = means3D.device
         P = means3D.shape[0]
+        rows = P if ragged else P * V
         n_geom, n_img, n_acc = ctx.offsets
         base = state.data_ptr()
         bin_p = binning.data_ptr() if binning is not None else base + n_geom + n_img + n_acc
@@ -430,16 +454,17 @@ class _RasterizeViews(torch.autograd.Function):
             # frame-sharded training: write (means3D, colours, opacity, scales, rotation) gradients straight into
             # the caller's [P,14] all-reduce buffer (gsvc_b200.sharding.packed_backward) and return views of it.  A
             # drop-in backward takes the buffer only: packed_backward leaves that buffer un-reduced for the caller's
-            # exchange.run(), so carrying the exchange too would sum it twice.
-            packed, exchange = _packed_target.take_with_exchange(P, device, col is not None and sc is not None,
-                                                                 carry=not single)
+            # exchange.run(), so carrying the exchange too would sum it twice.  A ragged backward has one gradient
+            # per row, not per Gaussian of a shared set: it never takes the buffer, like a call that does not fit it.
+            packed, exchange = _packed_target.take_with_exchange(P, device, col is not None and sc is not None
+                                                                 and not ragged, carry=not single)
             if exchange is not None and (P % 2 or sh is not None or cov is not None):
                 raise RasterizerError("a backward that carries the exchange needs an even P, colors_precomp and the "
                                       "scale / rotation pair")
             # one allocation for every gradient (contiguous slices) and the accumulator scratch
-            widths = (3, 3 * V, 1, 3 if col is not None else 0, ctx.sh_M * 3 if sh is not None else 0,
+            widths = (3, 3 if ragged else 3 * V, 1, 3 if col is not None else 0, ctx.sh_M * 3 if sh is not None else 0,
                       3 if sc is not None else 0, 4 if rot is not None else 0, 6 if cov is not None else 0)
-            n_scratch = 0 if n_acc else L.gsvc_rast_backward_scratch_bytes(P * V) // 4
+            n_scratch = 0 if n_acc else L.gsvc_rast_backward_scratch_bytes(rows) // 4
             # the accumulators inside the forward state were zeroed by the preprocess kernel; a backward
             # dirties them, so a second backward over the same graph (retain_graph) asks for a clear
             acc_clean = 1 if (n_acc and not getattr(ctx, "acc_dirty", False)) else 0
@@ -459,6 +484,13 @@ class _RasterizeViews(torch.autograd.Function):
                         _ptr(sc), _ptr(rot), _ptr(cov), _ptr(radii), base, base + n_geom, bin_p, scratch_p, acc_clean,
                         _ptr(g_out), _ptr(g_means2D), _ptr(packed), C.byref(exchange.exchange_struct()),
                         _stream_ptr(device)), "gsvc_rast_backward_views_exchange")
+                elif ragged:
+                    _lib.check(L.gsvc_rast_backward_ragged(
+                        nv.ref, V, nv.views, n_out, ctx.counts_c, ctx.sh_M, ctx.capacity, _ptr(means3D), _ptr(sh),
+                        _ptr(col), _ptr(sc), _ptr(rot), _ptr(cov), _ptr(radii), base, base + n_geom, bin_p, scratch_p,
+                        acc_clean, _ptr(g_out), _ptr(g_means3D), _ptr(g_means2D), _ptr(g_col), _ptr(g_opac),
+                        _ptr(g_sc), _ptr(g_rot), _ptr(g_cov), _ptr(g_sh), _stream_ptr(device)),
+                        "gsvc_rast_backward_ragged")
                 else:
                     _lib.check(L.gsvc_rast_backward_views(
                         nv.ref, V, nv.views, n_out, P, ctx.sh_M, ctx.capacity, _ptr(means3D), _ptr(sh), _ptr(col),
@@ -469,16 +501,16 @@ class _RasterizeViews(torch.autograd.Function):
             except Exception:
                 if ctx.rs.debug:
                     torch.save((means3D, sh, col, sc, rot, cov, radii, grad_out_color)
-                               + _snapshot_settings(ctx.rs, ctx.batch), "snapshot_bw.dump")
+                               + _snapshot_settings(ctx.rs, ctx.batch, ctx.counts), "snapshot_bw.dump")
                     print("\nAn error occured in backward. Writing snapshot_bw.dump for debugging.\n")
                 raise
         v = lambda t, *shape: None if t is None else t.view(*shape)
-        m2d = (P, 3) if single else (V, P, 3)
+        m2d = (P, 3) if single or ragged else (V, P, 3)
         if packed is not None:
             return (packed[:, 0:3], v(g_means2D, *m2d), None, packed[:, 3:6], packed[:, 6:7], packed[:, 7:10],
-                    packed[:, 10:14], None, None, None)
+                    packed[:, 10:14], None, None, None, None)
         return (v(g_means3D, P, 3), v(g_means2D, *m2d), v(g_sh, P, ctx.sh_M, 3), v(g_col, P, 3), v(g_opac, P, 1),
-                v(g_sc, P, 3), v(g_rot, P, 4), v(g_cov, P, 6), None, None)
+                v(g_sc, P, 3), v(g_rot, P, 4), v(g_cov, P, 6), None, None, None)
 
 
 # upstream passes an absent input to rasterize_gaussians as torch.Tensor([]); one shared instance, never written,
@@ -486,13 +518,14 @@ class _RasterizeViews(torch.autograd.Function):
 _EMPTY = torch.Tensor([])
 
 
-def _rasterize(rs, batch, means3D, means2D, opacities, shs, colors_precomp, scales, rotations, cov3D_precomp):
+def _rasterize(rs, batch, means3D, means2D, opacities, shs, colors_precomp, scales, rotations, cov3D_precomp,
+               counts=None):
     """GaussianRasterizer.forward / views.rasterize_views: upstream's input checks, then absent inputs as the empty
     tensor upstream's rasterize_gaussians takes."""
     _check_modes(scales, rotations, cov3D_precomp, (shs, colors_precomp))
     opt = lambda t: _EMPTY if t is None else t
     return _RasterizeViews.apply(means3D, opt(means2D), opt(shs), opt(colors_precomp), opacities, opt(scales),
-                                 opt(rotations), opt(cov3D_precomp), rs, batch)
+                                 opt(rotations), opt(cov3D_precomp), rs, batch, counts)
 
 
 def rasterize_gaussians(means3D, means2D, sh, colors_precomp, opacities, scales, rotations, cov3Ds_precomp,

@@ -1,12 +1,10 @@
-"""Batched views of one Gaussian set — the "toast" of SURVEY.md §8f row f1.
+"""Batched views — the "toast" of SURVEY.md §8f row f1.
 
 The reference renders every frame twice (front view, then the x-mirrored back view), flips the
 second image and averages the two (/root/reference/pipeline/train.py:353-387,
 utils/report_utils.py:303-314); a training iteration does that for two frames, i.e. FOUR complete
-rasterizer calls plus flip / add / scale passes.  Views that SHARE a Gaussian set can be batched (decode /
-evaluation of a fixed set; the front / back pair of one frame when the generator ran once for both — in training
-the reference regenerates the neural Gaussians per render() call, so there the per-call path is the comparable
-one, see DESIGN.md §5).  Here a batch of up to 16
+rasterizer calls plus flip / add / scale passes.  Views that SHARE a Gaussian set (decode / evaluation of a fixed
+set) and views with sets of their own (below) are both batched.  For a shared set a batch of up to 16
 views is ONE kernel chain (virtual Gaussian v*P+g, virtual tile v*T+t): one preprocess, one scan,
 one scatter, one sort, one blend forward, one blend backward, one per-Gaussian backward that SUMS
 the views' parameter gradients (what autograd accumulates across the reference's calls), and the
@@ -16,13 +14,28 @@ flip + average is folded into the blend's epilogue / the backward's prologue.
                                        scales=..., rotations=...)               # images [2,3,H,W]
     image, radii, n = render_toast(front, back, means3D=..., ...)               # (img_f + flip(img_b)) / 2
 
+Views with Gaussian sets of their OWN (what the reference's training iteration and decode loop render: every
+render() call regenerates its neural Gaussians, guassian.py:147-246) are one chain as well: pass the sets
+concatenated in view order and `counts=[P_0, ..., P_{V-1}]`.  Row off_v + g (off_v = P_0 + ... + P_{v-1}) is then
+Gaussian g of view v, drawn in view v only; radii and the means2D gradient have one row per input row, and every
+row's parameter gradient is its own view's (nothing is summed):
+
+    images, radii, n = rasterize_views(ViewBatch.toasts([(f0, b0), (f1, b1)]), means3D=torch.cat(xyz_per_view),
+                                       ..., counts=[len(x) for x in xyz_per_view])    # radii [sum P_v]
+
+Each view's image, radii and instance count are bit-identical to a GaussianRasterizer call on that view's own set.
+sharding.densify_stats needs nothing new for such a batch: one view per row is its n_views=1 form over the
+sum(P_v) rows (radii [sum P_v], means2D gradient [sum P_v, 3]).  A ragged backward never takes a
+sharding.packed_backward target: it is treated like a call that does not fit the target.
+
 Semantics per view are exactly those of `GaussianRasterizer`: both go through the one autograd Function of
-rasterizer.py and the gsvc_rast_*_views entry points, a `GaussianRasterizer` call being a batch of one.
+rasterizer.py and the gsvc_rast_*_views / *_ragged entry points, a `GaussianRasterizer` call being a batch of one.
 This module keeps the batch itself (ViewBatch: validation, the image map, its cached native descriptor).
 There is no CPU fallback.
 """
 from __future__ import annotations
 
+import operator
 import weakref
 from typing import Optional, Sequence
 
@@ -115,26 +128,52 @@ class ViewBatch:
         return cls(settings, out_image=out, flip_x=flip, weight=w)
 
 
+def _check_counts(counts, n_views: int, rows: int) -> tuple:
+    """The views' counts of a ragged call as a tuple of ints: one per view, each >= 0, summing to the input rows."""
+    try:
+        c = tuple(operator.index(x) for x in counts)
+    except TypeError as e:
+        raise RasterizerError(f"counts must be a sequence of ints, got {counts!r}") from e
+    if len(c) != n_views:
+        raise RasterizerError(f"counts needs one entry per view: {n_views} views, got {len(c)} counts")
+    if any(x < 0 for x in c):
+        raise RasterizerError(f"counts must be >= 0, got {list(c)}")
+    if sum(c) != rows:
+        raise RasterizerError(f"counts sum to {sum(c)}, but the inputs have {rows} rows (means3D.shape[0])")
+    return c
+
+
 def rasterize_views(views, means3D, opacities, means2D=None, shs=None, colors_precomp=None, scales=None,
-                    rotations=None, cov3D_precomp=None):
+                    rotations=None, cov3D_precomp=None, counts=None):
     """Rasterize every view of `views` (a ViewBatch, or a sequence of GaussianRasterizationSettings = one image
     per view) in one kernel chain.
 
     Returns (images [n_out,3,H,W], radii [n_views,P] int32, num_rendered: int, the total over the views).
     Differentiable like GaussianRasterizer; parameter gradients are summed over the views.  `means2D`
-    (optional, [n_views,P,3], requires_grad) receives each view's screen-space gradient (columns 0,1)."""
+    (optional, [n_views,P,3], requires_grad) receives each view's screen-space gradient (columns 0,1).
+
+    `counts` (optional, n_views ints >= 0 summing to means3D.shape[0]): every view has a Gaussian set of its own,
+    the inputs are those sets concatenated in view order (see the module docstring).  radii is then [sum P_v],
+    `means2D` [sum P_v, 3], and each row's gradients are those of its own view; num_rendered is still the total."""
     batch = views if isinstance(views, ViewBatch) else ViewBatch(list(views))
-    if means2D is not None and tuple(means2D.shape) != (batch.n_views, means3D.shape[0], 3):
-        raise RasterizerError(f"means2D must be [n_views, P, 3] = {(batch.n_views, means3D.shape[0], 3)}, "
+    P = means3D.shape[0]
+    if counts is not None:
+        counts = _check_counts(counts, batch.n_views, P)
+        if means2D is not None and tuple(means2D.shape) != (P, 3):
+            raise RasterizerError(f"means2D of a ragged batch must be [sum P_v, 3] = {(P, 3)}, "
+                                  f"got {tuple(means2D.shape)}")
+    elif means2D is not None and tuple(means2D.shape) != (batch.n_views, P, 3):
+        raise RasterizerError(f"means2D must be [n_views, P, 3] = {(batch.n_views, P, 3)}, "
                               f"got {tuple(means2D.shape)}")
     return _rasterize(batch.settings[0], batch, means3D, means2D, opacities, shs, colors_precomp, scales, rotations,
-                      cov3D_precomp)
+                      cov3D_precomp, counts)
 
 
 def render_toast(front: GaussianRasterizationSettings, back: GaussianRasterizationSettings, means3D, opacities,
-                 **kw):
-    """One frame as the reference composes it (train.py:353-375): (front + flip_x(back)) / 2 → [3,H,W]."""
-    images, radii, n = rasterize_views(ViewBatch.toast(front, back), means3D, opacities, **kw)
+                 counts=None, **kw):
+    """One frame as the reference composes it (train.py:353-375): (front + flip_x(back)) / 2 → [3,H,W].
+    `counts=[P_front, P_back]`: the two views have Gaussian sets of their own, concatenated (rasterize_views)."""
+    images, radii, n = rasterize_views(ViewBatch.toast(front, back), means3D, opacities, counts=counts, **kw)
     return images[0], radii, n
 
 

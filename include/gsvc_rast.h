@@ -220,6 +220,40 @@ GSVC_RAST_API int gsvc_rast_backward_views(const gsvc_rast_settings *st, int32_t
                              float *dL_dcov3D, float *dL_dshs, float *dL_packed, void *stream);
 
 /*
+ * Batched views over per-view Gaussian sets ("ragged" batches, docs/SPEC.md "Binning").  The reference regenerates its
+ * neural Gaussians on every render() call (ortho_gaussian_renderer/guassian.py:147-246: per-view visibility mask,
+ * embeddings from the view's camera, training noise), so every view of a training iteration or a decoded frame has a
+ * set of its own, of its own size.  These entry points take the views' sets concatenated in view order: counts_host
+ * [n_views] (host memory, each >= 0, sum <= 2^31 - 1) in place of P, view v owning rows off_v .. off_v + counts[v] - 1,
+ * off_v = counts[0] + ... + counts[v-1].  Row r is rendered in its own view only; the virtual Gaussian is r itself
+ * (point_list and export_keys carry r), tiles are v*T+t as for the shared-set batch, and the view map is the same.
+ * Per view, the image, radii and instance count are bit-identical to a single-view call on that view's own set.
+ * Every per-Gaussian array has sum(counts) rows: inputs, radii [sum], dL_dmeans2D [sum,3] and every parameter gradient,
+ * each row its own view's gradient (nothing is summed over views).  Sizes: geom gsvc_rast_geom_bytes(sum, sh_M), image
+ * gsvc_rast_image_bytes_views(W,H,n_views), scratch gsvc_rast_backward_scratch_bytes(sum).  No packed gradient and no
+ * exchange.  Other arguments as the _views entry points.
+ */
+GSVC_RAST_API int gsvc_rast_forward_ragged_launch(const gsvc_rast_settings *st, int32_t n_views,
+                             const gsvc_rast_view *views_host, int32_t n_out, const int32_t *counts_host, int32_t sh_M,
+                             const float *means3D, const float *shs, const float *colors_precomp,
+                             const float *opacities, const float *scales, const float *rotations,
+                             const float *cov3D_precomp, void *geom, void *image, void *binning, int64_t capacity,
+                             void *bwd_scratch, float *out_color, int32_t *radii, uint64_t *count_slot_host,
+                             uint32_t ticket, void *stream);
+GSVC_RAST_API int gsvc_rast_forward_ragged_render(const gsvc_rast_settings *st, int32_t n_views,
+                             const gsvc_rast_view *views_host, int32_t n_out, const int32_t *counts_host,
+                             const void *geom, void *image, void *binning, int64_t capacity, float *out_color,
+                             void *stream);
+GSVC_RAST_API int gsvc_rast_backward_ragged(const gsvc_rast_settings *st, int32_t n_views, const gsvc_rast_view *views_host,
+                             int32_t n_out, const int32_t *counts_host, int32_t sh_M, int64_t capacity,
+                             const float *means3D, const float *shs, const float *colors_precomp, const float *scales,
+                             const float *rotations, const float *cov3D_precomp, const int32_t *radii,
+                             const void *geom, const void *image, const void *binning, void *scratch,
+                             int32_t scratch_is_zero, const float *dL_dout, float *dL_dmeans3D, float *dL_dmeans2D,
+                             float *dL_dcolors, float *dL_dopacities, float *dL_dscales, float *dL_drotations,
+                             float *dL_dcov3D, float *dL_dshs, void *stream);
+
+/*
  * Densification statistic of the step at the rasterizer boundary.  The reference calls
  * GaussianModel.training_statis once per rendered view (pipeline/train.py:559-565); per view it takes the norm of
  * the screen-space gradient of the Gaussians that were drawn — `torch.norm(viewspace_points.grad[radii > 0, :2])`,
