@@ -106,6 +106,9 @@ SIGNATURES = {
     "gsvc_rast_quality_scratch_bytes": (_sz, [_i32, _i32, _i32]),
     "gsvc_rast_quality": (C.c_int, [_i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp]),
     "gsvc_rast_frames_rgb8": (C.c_int, [_i32, _i32, _i32, _vp, _vp, _vp]),
+    "gsvc_rast_loss_forward_rgb8": (C.c_int, [_i32, _i32, _i32, _vp, _vp, _i32, _vp, C.c_float, _vp, _vp, _vp]),
+    "gsvc_rast_loss_backward_rgb8": (C.c_int, [_i32, _i32, _i32, _vp, _vp, _i32, _vp, C.c_float, _vp, _vp, _vp]),
+    "gsvc_rast_quality_rgb8": (C.c_int, [_i32, _i32, _i32, _vp, _vp, _i32, _vp, _vp, _vp, _vp]),
 }
 
 STAGES = ("preprocess", "tile_scan", "scatter", "sort_tiles", "render_forward", "render_backward",

@@ -62,17 +62,18 @@ __device__ __forceinline__ void vpass(const float* h, int hrows, int cols, int i
 }
 
 // the shift of a CTA: x and y at its tile centre, clamped into the image
-__device__ __forceinline__ void tile_shift(const float* x, const float* y, int H, int W, int ty, int tx, float& kx,
-                                           float& ky)
+template <class Y>
+__device__ __forceinline__ void tile_shift(const float* x, Y y, int H, int W, int ty, int tx, float& kx, float& ky)
 {
     const int r = min(ty * T + T / 2, H - 1), c = min(tx * T + T / 2, W - 1);
     kx = __ldg(x + (size_t)r * W + c);
-    ky = __ldg(y + (size_t)r * W + c);
+    ky = y((size_t)r * W + c);
 }
 
+// Tgt: PlanarTarget (fp32) or Rgb8Target (ssim.cuh); a CTA whose target frame is out of range leaves a NaN partial
+template <class Tgt>
 __global__ void __launch_bounds__(THREADS) loss_forward_kernel(int H, int W, const float* __restrict__ image,
-                                                                 const float* __restrict__ target,
-                                                                 double2* __restrict__ partials)
+                                                                 Tgt target, double2* __restrict__ partials)
 {
     __shared__ float s_x[F_SW * F_SW], s_y[F_SW * F_SW];
     __shared__ float s_h[5 * F_HR * T];
@@ -80,7 +81,11 @@ __global__ void __launch_bounds__(THREADS) loss_forward_kernel(int H, int W, con
     const int tx = blockIdx.x, ty = blockIdx.y, plane = blockIdx.z;      // plane = n * 3 + c
     const size_t off = (size_t)plane * H * W;
     const float* x = image + off;
-    const float* y = target + off;
+    typename Tgt::Plane y;
+    if (!target.plane(plane, H, W, y)) {
+        if (threadIdx.x == 0) partials[((size_t)plane * gridDim.y + ty) * gridDim.x + tx] = make_double2(NAN, NAN);
+        return;
+    }
     stage(x, y, H, W, ty * T - R, tx * T - R, F_SW, F_SW, s_x, s_y);
     __syncthreads();
     hpass_moments(s_x, s_y, F_HR, T, F_SW, s_h);
@@ -101,7 +106,7 @@ __global__ void __launch_bounds__(THREADS) loss_forward_kernel(int H, int W, con
             const float b1 = mux * mux + muy * muy + C1, b2 = mo[2][u] + mo[3][u] + C2;
             sum_s += (a1 * a2) / (b1 * b2);
             const size_t o = (size_t)gr * W + gc;
-            sum_l1 += fabsf(__ldg(x + o) - __ldg(y + o));
+            sum_l1 += fabsf(__ldg(x + o) - y(o));
         }
     }
 #pragma unroll
@@ -140,8 +145,10 @@ __global__ void __launch_bounds__(THREADS) loss_reduce_kernel(int per_image, dou
     }
 }
 
+// a CTA whose target frame is out of range writes zeros over its tile
+template <class Tgt>
 __global__ void __launch_bounds__(THREADS) loss_backward_kernel(int H, int W, const float* __restrict__ image,
-                                                                  const float* __restrict__ target, float lambda,
+                                                                  Tgt target, float lambda,
                                                                   const float* __restrict__ dL_dloss,
                                                                   float* __restrict__ dL_dimage)
 {
@@ -152,7 +159,13 @@ __global__ void __launch_bounds__(THREADS) loss_backward_kernel(int H, int W, co
     const int tx = blockIdx.x, ty = blockIdx.y, plane = blockIdx.z;
     const size_t off = (size_t)plane * H * W;
     const float* x = image + off;
-    const float* y = target + off;
+    typename Tgt::Plane y;
+    if (!target.plane(plane, H, W, y)) {
+        const int j = threadIdx.x % T, i0 = (threadIdx.x / T) * RUN, gc = tx * T + j;
+        for (int u = 0; u < RUN && gc < W && ty * T + i0 + u < H; u++)
+            dL_dimage[off + (size_t)(ty * T + i0 + u) * W + gc] = 0.0f;
+        return;
+    }
     float kx, ky;
     tile_shift(x, y, H, W, ty, tx, kx, ky);
     const int mr0 = ty * T - R, mc0 = tx * T - R;        // image coordinates of map element (0, 0)
@@ -234,7 +247,7 @@ __global__ void __launch_bounds__(THREADS) loss_backward_kernel(int H, int W, co
         const int gr = ty * T + i0 + u;
         if (gr >= H) break;
         const size_t o = (size_t)gr * W + gc;
-        const float vx = __ldg(x + o), vy = __ldg(y + o);
+        const float vx = __ldg(x + o), vy = y(o);
         const float d = vx - vy;
         const float sgn = d > 0.0f ? 1.0f : (d < 0.0f ? -1.0f : 0.0f);   // torch.sign: 0 where x == y
         const float dss = sm[0][u] + 2.0f * (vx - kx) * sm[1][u] + (vy - ky) * sm[2][u];
@@ -242,7 +255,8 @@ __global__ void __launch_bounds__(THREADS) loss_backward_kernel(int H, int W, co
     }
 }
 
-// the backward's 71 KB of shared memory: opted into once per device (an attribute, no stream work)
+// the backward's 71 KB of shared memory: opted into once per device and instantiation (an attribute, no stream work)
+template <class Tgt>
 static cudaError_t prepare_backward()
 {
     static std::atomic<unsigned long long> done{0};          // bit per device
@@ -251,7 +265,7 @@ static cudaError_t prepare_backward()
     if (e != cudaSuccess) return e;
     const unsigned long long bit = 1ull << (dev & 63);
     if (done.load() & bit) return cudaSuccess;
-    e = cudaFuncSetAttribute(loss_backward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)B_SMEM_BYTES);
+    e = cudaFuncSetAttribute(loss_backward_kernel<Tgt>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)B_SMEM_BYTES);
     if (e == cudaSuccess) done.fetch_or(bit);
     return e;
 }
@@ -260,7 +274,7 @@ static cudaError_t prepare_backward()
 
 int fail(int code, const char* fmt, ...);
 
-static int loss_check(int32_t n, int32_t H, int32_t W, const float* image, const float* target, float lambda)
+static int loss_check(int32_t n, int32_t H, int32_t W, const float* image, const void* target, float lambda)
 {
     if (!image || !target) return fail(GSVC_RAST_ERR_INVALID, "image / target is NULL");
     if (n < 1 || H < 1 || W < 1) return fail(GSVC_RAST_ERR_INVALID, "n_images, H and W must be >= 1, got %d, %d, %d", n, H, W);
@@ -271,6 +285,47 @@ static int loss_check(int32_t n, int32_t H, int32_t W, const float* image, const
     if ((double)n * 3.0 * (double)H * (double)W >= 9.0e18)
         return fail(GSVC_RAST_ERR_INVALID, "size too large: n_images * 3 * H * W overflows a 64-bit index");
     return GSVC_RAST_OK;
+}
+
+// the frame cube of an 8-bit target (SPEC U12), after the size rules of the call it goes with
+int rgb8_target_check(int32_t n, int32_t H, int32_t W, int32_t n_frames, const int32_t* frame_index)
+{
+    if (n_frames < 1) return fail(GSVC_RAST_ERR_INVALID, "n_frames must be >= 1, got %d", n_frames);
+    if (!frame_index && n > n_frames)
+        return fail(GSVC_RAST_ERR_INVALID, "frame_index is NULL (image n against frame n) but n_images %d > n_frames %d",
+                    n, n_frames);
+    if ((double)n_frames * 3.0 * (double)H * (double)W >= 9.0e18)
+        return fail(GSVC_RAST_ERR_INVALID, "size too large: n_frames * H * W * 3 overflows a 64-bit index");
+    return GSVC_RAST_OK;
+}
+
+template <class Tgt>
+static int loss_forward(int32_t n_images, int32_t H, int32_t W, const float* image, Tgt target, float lambda_dssim,
+                        float* loss, void* scratch, cudaStream_t st)
+{
+    const dim3 grid((W + loss::T - 1) / loss::T, (H + loss::T - 1) / loss::T, n_images * 3);
+    double2* partials = static_cast<double2*>(scratch);
+    count_launch(2);
+    loss::loss_forward_kernel<<<grid, loss::THREADS, 0, st>>>(H, W, image, target, partials);
+    loss::loss_reduce_kernel<<<n_images, loss::THREADS, 0, st>>>((int)(3 * grid.x * grid.y),
+                                                                  1.0 / (3.0 * (double)H * (double)W), lambda_dssim,
+                                                                  partials, loss);
+    const cudaError_t e = cudaGetLastError();
+    return e == cudaSuccess ? GSVC_RAST_OK : fail(GSVC_RAST_ERR_CUDA, "loss_forward: %s", cudaGetErrorString(e));
+}
+
+template <class Tgt>
+static int loss_backward(int32_t n_images, int32_t H, int32_t W, const float* image, Tgt target, float lambda_dssim,
+                         const float* dL_dloss, float* dL_dimage, cudaStream_t st)
+{
+    cudaError_t e = loss::prepare_backward<Tgt>();
+    if (e != cudaSuccess) return fail(GSVC_RAST_ERR_CUDA, "loss_backward: %s", cudaGetErrorString(e));
+    const dim3 grid((W + loss::T - 1) / loss::T, (H + loss::T - 1) / loss::T, n_images * 3);
+    count_launch();
+    loss::loss_backward_kernel<<<grid, loss::THREADS, loss::B_SMEM_BYTES, st>>>(H, W, image, target, lambda_dssim,
+                                                                                 dL_dloss, dL_dimage);
+    e = cudaGetLastError();
+    return e == cudaSuccess ? GSVC_RAST_OK : fail(GSVC_RAST_ERR_CUDA, "loss_backward: %s", cudaGetErrorString(e));
 }
 
 }  // namespace gsvc
@@ -292,16 +347,8 @@ int gsvc_rast_loss_forward(int32_t n_images, int32_t H, int32_t W, const float* 
     int rc = loss_check(n_images, H, W, image, target, lambda_dssim);
     if (rc != GSVC_RAST_OK) return rc;
     if (!loss || !scratch) return fail(GSVC_RAST_ERR_INVALID, "loss / scratch is NULL");
-    cudaStream_t st = static_cast<cudaStream_t>(stream_);
-    const dim3 grid((W + loss::T - 1) / loss::T, (H + loss::T - 1) / loss::T, n_images * 3);
-    double2* partials = static_cast<double2*>(scratch);
-    count_launch(2);
-    loss::loss_forward_kernel<<<grid, loss::THREADS, 0, st>>>(H, W, image, target, partials);
-    loss::loss_reduce_kernel<<<n_images, loss::THREADS, 0, st>>>((int)(3 * grid.x * grid.y),
-                                                                  1.0 / (3.0 * (double)H * (double)W), lambda_dssim,
-                                                                  partials, loss);
-    const cudaError_t e = cudaGetLastError();
-    return e == cudaSuccess ? GSVC_RAST_OK : fail(GSVC_RAST_ERR_CUDA, "loss_forward: %s", cudaGetErrorString(e));
+    return loss_forward(n_images, H, W, image, ssim::PlanarTarget{target}, lambda_dssim, loss, scratch,
+                        static_cast<cudaStream_t>(stream_));
 }
 
 int gsvc_rast_loss_backward(int32_t n_images, int32_t H, int32_t W, const float* image, const float* target,
@@ -310,15 +357,32 @@ int gsvc_rast_loss_backward(int32_t n_images, int32_t H, int32_t W, const float*
     int rc = loss_check(n_images, H, W, image, target, lambda_dssim);
     if (rc != GSVC_RAST_OK) return rc;
     if (!dL_dloss || !dL_dimage) return fail(GSVC_RAST_ERR_INVALID, "dL_dloss / dL_dimage is NULL");
-    cudaStream_t st = static_cast<cudaStream_t>(stream_);
-    cudaError_t e = loss::prepare_backward();
-    if (e != cudaSuccess) return fail(GSVC_RAST_ERR_CUDA, "loss_backward: %s", cudaGetErrorString(e));
-    const dim3 grid((W + loss::T - 1) / loss::T, (H + loss::T - 1) / loss::T, n_images * 3);
-    count_launch();
-    loss::loss_backward_kernel<<<grid, loss::THREADS, loss::B_SMEM_BYTES, st>>>(H, W, image, target, lambda_dssim,
-                                                                                 dL_dloss, dL_dimage);
-    e = cudaGetLastError();
-    return e == cudaSuccess ? GSVC_RAST_OK : fail(GSVC_RAST_ERR_CUDA, "loss_backward: %s", cudaGetErrorString(e));
+    return loss_backward(n_images, H, W, image, ssim::PlanarTarget{target}, lambda_dssim, dL_dloss, dL_dimage,
+                         static_cast<cudaStream_t>(stream_));
+}
+
+int gsvc_rast_loss_forward_rgb8(int32_t n_images, int32_t H, int32_t W, const float* image, const uint8_t* frames,
+                                int32_t n_frames, const int32_t* frame_index, float lambda_dssim, float* loss,
+                                void* scratch, void* stream_)
+{
+    int rc = loss_check(n_images, H, W, image, frames, lambda_dssim);
+    if (rc == GSVC_RAST_OK) rc = rgb8_target_check(n_images, H, W, n_frames, frame_index);
+    if (rc != GSVC_RAST_OK) return rc;
+    if (!loss || !scratch) return fail(GSVC_RAST_ERR_INVALID, "loss / scratch is NULL");
+    return loss_forward(n_images, H, W, image, ssim::Rgb8Target{frames, frame_index, n_frames}, lambda_dssim, loss, scratch,
+                        static_cast<cudaStream_t>(stream_));
+}
+
+int gsvc_rast_loss_backward_rgb8(int32_t n_images, int32_t H, int32_t W, const float* image, const uint8_t* frames,
+                                 int32_t n_frames, const int32_t* frame_index, float lambda_dssim,
+                                 const float* dL_dloss, float* dL_dimage, void* stream_)
+{
+    int rc = loss_check(n_images, H, W, image, frames, lambda_dssim);
+    if (rc == GSVC_RAST_OK) rc = rgb8_target_check(n_images, H, W, n_frames, frame_index);
+    if (rc != GSVC_RAST_OK) return rc;
+    if (!dL_dloss || !dL_dimage) return fail(GSVC_RAST_ERR_INVALID, "dL_dloss / dL_dimage is NULL");
+    return loss_backward(n_images, H, W, image, ssim::Rgb8Target{frames, frame_index, n_frames}, lambda_dssim, dL_dloss,
+                         dL_dimage, static_cast<cudaStream_t>(stream_));
 }
 
 }  // extern "C"

@@ -14,6 +14,8 @@
 
 #include <math.h>
 
+#include <type_traits>
+
 namespace gsvc {
 
 namespace quality {
@@ -58,9 +60,10 @@ static Layout layout(int n, int H, int W)
 // One 32x32 tile of one plane of an h x w level.  L0: x is clamped on read and the all-pixel sums are formed.
 // partials[cta] = (sum (x - y)^2, sum S, interior sum S, interior sum cs); xo / yo (nullptr after the last level):
 // the ceil(h/2) x ceil(w/2) pooled images, avg_pool2d(2, 2, padding = (h % 2, w % 2), count_include_pad).
-template <bool L0>
-__global__ void __launch_bounds__(THREADS) quality_level_kernel(int h, int w, const float* __restrict__ xi,
-                                                                  const float* __restrict__ yi,
+// Tgt: PlanarTarget, or Rgb8Target at level 0 (ssim.cuh).  A CTA whose target frame is out of range leaves NaN
+// partials and NaN pooled values, so every level of its image is NaN.
+template <bool L0, class Tgt>
+__global__ void __launch_bounds__(THREADS) quality_level_kernel(int h, int w, const float* __restrict__ xi, Tgt yi,
                                                                   double4* __restrict__ partials,
                                                                   float* __restrict__ xo, float* __restrict__ yo)
 {
@@ -71,7 +74,21 @@ __global__ void __launch_bounds__(THREADS) quality_level_kernel(int h, int w, co
     const int tx = blockIdx.x, ty = blockIdx.y, plane = blockIdx.z;      // plane = n * 3 + c
     const size_t off = (size_t)plane * h * w;
     const int r0 = ty * T - R, c0 = tx * T - R;                          // image coordinates of stage (0, 0)
-    stage<L0>(xi + off, yi + off, h, w, r0, c0, F_SW, F_SW, s_x, s_y);
+    typename Tgt::Plane y;
+    if (!yi.plane(plane, h, w, y)) {
+        if (xo) {
+            const int ho = (h + 1) / 2, wo = (w + 1) / 2;
+            const int oi = ty * PT + threadIdx.x / PT, oj = tx * PT + threadIdx.x % PT;
+            if (oi < ho && oj < wo) {
+                const size_t o = (size_t)plane * ho * wo + (size_t)oi * wo + oj;
+                xo[o] = NAN;
+                yo[o] = NAN;
+            }
+        }
+        if (threadIdx.x == 0) partials[((size_t)plane * gridDim.y + ty) * gridDim.x + tx] = make_double4(NAN, NAN, NAN, NAN);
+        return;
+    }
+    stage<L0>(xi + off, y, h, w, r0, c0, F_SW, F_SW, s_x, s_y);
     __syncthreads();
     hpass_moments(s_x, s_y, F_HR, T, F_SW, s_h);
     if (xo) {                                   // pooled level: one output per thread from the stage
@@ -149,7 +166,9 @@ struct ReduceArgs {
 };
 
 // One CTA per image: every (channel, level) sum in a fixed order (strided per thread, butterfly per warp, warps in
-// index order), then PSNR, SSIM and MS-SSIM in double.
+// index order), then PSNR, SSIM and MS-SSIM in double.  NAN_ROWS (8-bit targets, whose values are finite): a NaN
+// level-0 sum marks an out-of-range frame, and the whole row is NaN (MS-SSIM's clamp at 0 would otherwise hide it).
+template <bool NAN_ROWS>
 __global__ void __launch_bounds__(THREADS) quality_reduce_kernel(ReduceArgs a, float* __restrict__ quality)
 {
     __shared__ double s_w[4][THREADS / 32];
@@ -197,6 +216,7 @@ __global__ void __launch_bounds__(THREADS) quality_reduce_kernel(ReduceArgs a, f
         }
         ms /= 3.0;
     }
+    if (NAN_ROWS && isnan(ss)) ms = (double)NAN;
     float* out = quality + (size_t)blockIdx.x * 3;
     out[0] = (float)psnr;
     out[1] = (float)(ss / a.count);
@@ -207,7 +227,9 @@ __global__ void __launch_bounds__(THREADS) quality_reduce_kernel(ReduceArgs a, f
 
 int fail(int code, const char* fmt, ...);
 
-static int quality_check(int32_t n, int32_t H, int32_t W, const float* image, const float* target, const float* out,
+int rgb8_target_check(int32_t n, int32_t H, int32_t W, int32_t n_frames, const int32_t* frame_index);   // loss.cu
+
+static int quality_check(int32_t n, int32_t H, int32_t W, const float* image, const void* target, const float* out,
                          const void* scratch)
 {
     if (!image || !target) return fail(GSVC_RAST_ERR_INVALID, "image / target is NULL");
@@ -220,24 +242,12 @@ static int quality_check(int32_t n, int32_t H, int32_t W, const float* image, co
     return GSVC_RAST_OK;
 }
 
-}  // namespace gsvc
-
-using namespace gsvc;
-
-extern "C" {
-
-size_t gsvc_rast_quality_scratch_bytes(int32_t n_images, int32_t H, int32_t W)
+template <class Tgt>
+static int quality_run(int32_t n_images, int32_t H, int32_t W, const float* image, Tgt target, float* quality,
+                       void* scratch, cudaStream_t st)
 {
-    return quality::layout(n_images < 1 ? 1 : n_images, H < 1 ? 1 : H, W < 1 ? 1 : W).bytes;
-}
-
-int gsvc_rast_quality(int32_t n_images, int32_t H, int32_t W, const float* image, const float* target, float* quality,
-                      void* scratch, void* stream_)
-{
-    int rc = quality_check(n_images, H, W, image, target, quality, scratch);
-    if (rc != GSVC_RAST_OK) return rc;
     using namespace quality;
-    cudaStream_t st = static_cast<cudaStream_t>(stream_);
+    constexpr bool rgb8 = !std::is_same<Tgt, PlanarTarget>::value;
     const Layout L = layout(n_images, H, W);
     char* base = static_cast<char*>(scratch);
     const int levels = (H < MS_MIN_SIDE || W < MS_MIN_SIDE) ? 1 : LEVELS;   // no pyramid without MS-SSIM
@@ -256,16 +266,45 @@ int gsvc_rast_quality(int32_t n_images, int32_t H, int32_t W, const float* image
         float* xo = l + 1 < levels ? reinterpret_cast<float*>(base + L.img_x[l + 1]) : nullptr;
         float* yo = l + 1 < levels ? reinterpret_cast<float*>(base + L.img_y[l + 1]) : nullptr;
         if (l == 0)
-            e = launch_pdl(quality_level_kernel<true>, grid, dim3(THREADS), st, H, W, image, target, part, xo, yo);
+            e = launch_pdl(quality_level_kernel<true, Tgt>, grid, dim3(THREADS), st, H, W, image, target, part, xo, yo);
         else
-            e = launch_pdl(quality_level_kernel<false>, grid, dim3(THREADS), st, L.h[l], L.w[l],
+            e = launch_pdl(quality_level_kernel<false, PlanarTarget>, grid, dim3(THREADS), st, L.h[l], L.w[l],
                            reinterpret_cast<const float*>(base + L.img_x[l]),
-                           reinterpret_cast<const float*>(base + L.img_y[l]), part, xo, yo);
+                           PlanarTarget{reinterpret_cast<const float*>(base + L.img_y[l])}, part, xo, yo);
     }
-    if (e == cudaSuccess) e = launch_pdl(quality_reduce_kernel, dim3(n_images), dim3(THREADS), st, ra, quality);
+    if (e == cudaSuccess) e = launch_pdl(quality_reduce_kernel<rgb8>, dim3(n_images), dim3(THREADS), st, ra, quality);
     count_launch(levels + 1);
     if (e == cudaSuccess) e = cudaGetLastError();
     return e == cudaSuccess ? GSVC_RAST_OK : fail(GSVC_RAST_ERR_CUDA, "quality: %s", cudaGetErrorString(e));
+}
+
+}  // namespace gsvc
+
+using namespace gsvc;
+
+extern "C" {
+
+size_t gsvc_rast_quality_scratch_bytes(int32_t n_images, int32_t H, int32_t W)
+{
+    return quality::layout(n_images < 1 ? 1 : n_images, H < 1 ? 1 : H, W < 1 ? 1 : W).bytes;
+}
+
+int gsvc_rast_quality(int32_t n_images, int32_t H, int32_t W, const float* image, const float* target, float* quality,
+                      void* scratch, void* stream_)
+{
+    int rc = quality_check(n_images, H, W, image, target, quality, scratch);
+    if (rc != GSVC_RAST_OK) return rc;
+    return quality_run(n_images, H, W, image, ssim::PlanarTarget{target}, quality, scratch, static_cast<cudaStream_t>(stream_));
+}
+
+int gsvc_rast_quality_rgb8(int32_t n_images, int32_t H, int32_t W, const float* image, const uint8_t* frames,
+                           int32_t n_frames, const int32_t* frame_index, float* quality, void* scratch, void* stream_)
+{
+    int rc = quality_check(n_images, H, W, image, frames, quality, scratch);
+    if (rc == GSVC_RAST_OK) rc = rgb8_target_check(n_images, H, W, n_frames, frame_index);
+    if (rc != GSVC_RAST_OK) return rc;
+    return quality_run(n_images, H, W, image, ssim::Rgb8Target{frames, frame_index, n_frames}, quality, scratch,
+                       static_cast<cudaStream_t>(stream_));
 }
 
 }  // extern "C"

@@ -10,6 +10,13 @@
 // (the law of total variance): every sum is of non-negative or centred terms, exact to fp32 rounding at any level of
 // the image, flat regions included.
 //
+// Targets (SPEC U12).  A kernel reads its target through a reader type: PlanarTarget is the fp32 [N,3,H,W] tensor,
+// Rgb8Target an 8-bit [F,H,W,3] frame cube with an optional device frame index (image n is compared with frame
+// index[n], frame n without one).  Every thread of a CTA reads its plane's index word (one broadcast load per warp,
+// no barrier before the staging can start); a CTA whose index is outside [0, F) reads no target byte, and its kernel
+// writes NaN (forward, quality) or zero (backward) for it instead.  A byte q reads as fl(q / 255), the one correctly
+// rounded division of torchvision's to_tensor.
+//
 // Every .cu file is compiled as its own whole-program module, so each includer gets its own copy of c_g.
 #pragma once
 
@@ -35,11 +42,48 @@ __constant__ float c_g[11] = {0x1.0d956cp-10f, 0x1.f1fe02p-8f, 0x1.26eb18p-5f, 0
                               0x1.106560p-2f, 0x1.b43c40p-3f, 0x1.bff0fep-4f, 0x1.26eb18p-5f, 0x1.f1fe02p-8f,
                               0x1.0d956cp-10f};
 
+// fp32 targets, planar like the images: the plane of CTA plane p starts at y + p * H * W
+struct PlanarTarget {
+    const float* y;
+    struct Plane {
+        const float* y;
+        __device__ __forceinline__ float operator()(size_t o) const { return __ldg(y + o); }
+    };
+    __device__ __forceinline__ bool plane(int p, int H, int W, Plane& out) const
+    {
+        out.y = y + (size_t)p * H * W;
+        return true;
+    }
+};
+
+// 8-bit targets: frames [n_frames, H, W, 3] (RGB interleaved, any alignment), index [N] int32 or nullptr
+struct Rgb8Target {
+    const uint8_t* frames;
+    const int32_t* index;
+    int n_frames;
+    struct Plane {
+        const uint8_t* q;                       // channel c of the frame: pixel o at q[3 o]
+        __device__ __forceinline__ float operator()(size_t o) const
+        {
+            return __fdiv_rn((float)__ldg(q + 3 * o), 255.0f);
+        }
+    };
+    // false (for every thread of the CTA) when the frame of plane p's image is outside [0, n_frames)
+    __device__ __forceinline__ bool plane(int p, int H, int W, Plane& out) const
+    {
+        const int n = p / 3;
+        const int f = index ? __ldg(index + n) : n;
+        if (f < 0 || f >= n_frames) return false;
+        out.q = frames + (size_t)f * H * W * 3 + (p - n * 3);
+        return true;
+    }
+};
+
 // Stage rows [r0, r0+rows) x cols [c0, c0+cols) of x and y (0 outside the image: the zero padding) into sx / sy.
-// CLAMP_X: x is read clamped to [0, 1].
-template <bool CLAMP_X = false>
-__device__ __forceinline__ void stage(const float* __restrict__ x, const float* __restrict__ y, int H, int W, int r0,
-                                      int c0, int rows, int cols, float* sx, float* sy)
+// CLAMP_X: x is read clamped to [0, 1].  y: a target plane reader (PlanarTarget::Plane, Rgb8Target::Plane).
+template <bool CLAMP_X = false, class Y>
+__device__ __forceinline__ void stage(const float* __restrict__ x, Y y, int H, int W, int r0, int c0, int rows,
+                                      int cols, float* sx, float* sy)
 {
     for (int e = threadIdx.x; e < rows * cols; e += THREADS) {
         const int r = e / cols, c = e - r * cols;
@@ -48,7 +92,7 @@ __device__ __forceinline__ void stage(const float* __restrict__ x, const float* 
         if (gr >= 0 && gr < H && gc >= 0 && gc < W) {
             const size_t o = (size_t)gr * W + gc;
             vx = __ldg(x + o);
-            vy = __ldg(y + o);
+            vy = y(o);
             if (CLAMP_X) vx = fminf(fmaxf(vx, 0.0f), 1.0f);
         }
         sx[e] = vx;

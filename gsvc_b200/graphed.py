@@ -20,6 +20,13 @@ L1 + D-SSIM loss (gsvc_b200.loss) against it and back-propagates, so the whole s
     target.copy_(frames)                                # this iteration's target frames, in place
     color, radii, grads = step()                        # step.loss: the per-image losses of this replay
 
+or against the video's 8-bit frames kept resident on the device (SPEC U12), picked per replay by a static index:
+
+    idx = torch.zeros(n_out, dtype=torch.int32, device="cuda")
+    step = GraphedStep(batch, params, None, loss_target=cube, loss_index=idx)     # cube [F,H,W,3] uint8
+    idx.copy_(pair, non_blocking=True)                  # this iteration's frame numbers, 4 bytes per image, in place
+    color, radii, grads = step()
+
 The binning capacity is fixed at capture time from an eager warm-up (+50 % + 64 Ki instances) and recorded on the
 step's own count slot; `capacity_ok()` compares it with the instance count the device published there for the last
 replay.
@@ -39,17 +46,32 @@ from .sharding import GRAD_LAYOUT, GRAD_WIDTH, packed_backward
 from .views import ViewBatch, render_params
 
 
-def _packed_step(rast, params, dL, packed, exchange=None, loss_target=None, lambda_dssim=0.2):
+def _packed_step(rast, params, dL, packed, exchange=None, loss_target=None, lambda_dssim=0.2, loss_index=None):
     """Forward + backward of `rast` on the GRAD_LAYOUT dict `params`, the gradients written into `packed`
     (sharding.packed_backward); the backward is seeded with `dL`, or with the mean of photometric_loss(image,
-    loss_target) when a target is given.  Returns (color, radii, num_rendered, per-image loss or None)."""
+    loss_target, index=loss_index) when a target is given.  Returns (color, radii, num_rendered, per-image loss or
+    None)."""
     leaves = {k: params[k].detach().requires_grad_(True) for k, _ in GRAD_LAYOUT}
     color, radii, n = render_params(rast, leaves)
-    loss = None if loss_target is None else photometric_loss(color, loss_target, lambda_dssim)
+    loss = None if loss_target is None else photometric_loss(color, loss_target, lambda_dssim, index=loss_index)
     with packed_backward(packed, exchange=exchange):
         torch.autograd.grad(color if loss is None else loss.mean(), [leaves[k] for k, _ in GRAD_LAYOUT],
                             grad_outputs=dL)
     return color, radii, n, loss
+
+
+def _check_rgb8_loss_target(target, index, device):
+    """A uint8 loss target of a captured step: nothing that photometric_loss would convert (a copy baked into the
+    graph would not see the caller's in-place writes).  Shapes are checked against the image by the warm-up."""
+    if not target.is_contiguous():
+        raise RasterizerError("a uint8 loss_target must be contiguous (the graph reads it in place)")
+    if index is not None:
+        if target.dim() != 4:
+            raise RasterizerError(f"with loss_index, loss_target must be a [F,H,W,3] cube, got {tuple(target.shape)}")
+        if (not isinstance(index, torch.Tensor) or index.device != device or index.dtype != torch.int32
+                or index.dim() != 1 or not index.is_contiguous()):
+            raise RasterizerError(f"loss_index must be a contiguous int32 [n_out] tensor on {device} (the graph reads "
+                                  "it in place)")
 
 
 def _steps_fit(device, steps) -> bool:
@@ -63,7 +85,8 @@ def _steps_fit(device, steps) -> bool:
 class GraphedStep:
     def __init__(self, rast, params: Dict[str, torch.Tensor], dL: Optional[torch.Tensor],
                  packed: Optional[torch.Tensor] = None, warmup: int = 2, exchange=None,
-                 loss_target: Optional[torch.Tensor] = None, lambda_dssim: float = 0.2):
+                 loss_target: Optional[torch.Tensor] = None, lambda_dssim: float = 0.2,
+                 loss_index: Optional[torch.Tensor] = None):
         """`rast`: a GaussianRasterizer (one view, dL [3,H,W]) or a views.ViewBatch (all its views in one chain,
         dL [n_out,3,H,W], gradients summed over the views).  `dL` None: forward only.  `packed`: optional [P,14]
         buffer the backward writes (sharding.GRAD_LAYOUT); allocated here if omitted.  `exchange`: a
@@ -72,20 +95,27 @@ class GraphedStep:
         `loss_target`: a static CUDA tensor shaped like the rendered image ([3,H,W] / [n_out,3,H,W]) instead of `dL`:
         the step then evaluates photometric_loss(image, loss_target, lambda_dssim) into the static `self.loss` (0-dim /
         [n_out]) and back-propagates the MEAN of the per-image losses.  Write each iteration's targets into it in
-        place."""
+        place.  8-bit targets (SPEC U12): `loss_target` a contiguous uint8 [H,W,3] / [n_out,H,W,3] tensor, or a
+        contiguous uint8 [F,H,W,3] cube with `loss_index`, a contiguous int32 [n_out] CUDA tensor: the graph reads both
+        in place, so an in-place write of the index picks the next replay's frames."""
         self.rast, self.params, self.dL = rast, params, dL
         m = params["means3D"]
         if not m.is_cuda:
             raise RasterizerError("GraphedStep needs CUDA tensors: gsvc_b200 has no CPU fallback")
         self.device, self.P = m.device, int(m.shape[0])
         self.loss_target, self.lambda_dssim, self.loss = loss_target, lambda_dssim, None
+        self.loss_index = loss_index
+        if loss_index is not None and (loss_target is None or loss_target.dtype != torch.uint8):
+            raise RasterizerError("loss_index picks frames of a uint8 loss_target cube: pass both")
         if loss_target is not None:
             if dL is not None:
                 raise RasterizerError("pass either dL (a fixed seed gradient) or loss_target (the step's own loss)")
             _check_lambda(lambda_dssim)
             if not isinstance(loss_target, torch.Tensor) or loss_target.device != self.device:
                 raise RasterizerError(f"loss_target must be a tensor on {self.device}")
-            if loss_target.dtype != torch.float32 or not loss_target.is_contiguous():
+            if loss_target.dtype == torch.uint8:
+                _check_rgb8_loss_target(loss_target, loss_index, self.device)
+            elif loss_target.dtype != torch.float32 or not loss_target.is_contiguous():
                 # a converted copy would be baked into the graph: in-place updates of the caller's tensor would be lost
                 raise RasterizerError("loss_target must be a contiguous fp32 tensor (the graph reads it in place)")
         self.backward = dL is not None or loss_target is not None
@@ -114,7 +144,8 @@ class GraphedStep:
         if not self.backward:
             with torch.no_grad():
                 return (*render_params(self.rast, p, means2D=p["means3D"]), None)   # no gradient: any tensor serves
-        return _packed_step(self.rast, p, self.dL, self.packed, self.exchange, self.loss_target, self.lambda_dssim)
+        return _packed_step(self.rast, p, self.dL, self.packed, self.exchange, self.loss_target, self.lambda_dssim,
+                            self.loss_index)
 
     def recapture(self) -> None:
         """(Re)build the graph: eager warm-up on a side stream (sets the capacity hint), then capture."""
@@ -192,6 +223,25 @@ class FrameStreamer:
             done[j] = streamer.last_event()
         streamer.synchronize()                                              # then write the last R frames
 
+    Evaluate against the source video's 8-bit frames (SPEC U12): `target` may be a uint8 frame ([H,W,3] for a toast,
+    [n_out,H,W,3] otherwise, contiguous), on the device (e.g. `cube[i]` of a resident cube) or in pinned host memory.
+    A host frame is copied on one host-to-device stream into one of 2 x n_streams device staging buffers, enqueued
+    before the frame's replay so that the copy runs under the render; the frame's stream waits for it only before its
+    quality pass, and a staging buffer is uploaded into again only after the quality pass that read it.  Pageable host
+    memory is refused (the copy would block the host).  `last_event()` follows the quality pass, so it covers the
+    upload: a caller streaming frames from disk refills its ring of pinned input buffers after a buffer's event:
+
+        ring = [torch.empty(H, W, 3, dtype=torch.uint8).pin_memory() for _ in range(R)]
+        done = [None] * R
+        for i, (V_front, V_back) in enumerate(frames):
+            j = i % R
+            if done[j] is not None:
+                done[j].synchronize()                                       # frame i - R has been read
+            ring[j].copy_(source_frame(i))                                  # e.g. np.array(PIL.Image.open(...))
+            streamer.render(V_front, V_back, target=ring[j], quality=q[i])
+            done[j] = streamer.last_event()
+        streamer.synchronize()
+
     A replay that overflowed its capacity (`capacity_ok()` false after a synchronisation) leaves invalid quality values
     and invalid host frames alike."""
 
@@ -219,6 +269,9 @@ class FrameStreamer:
         self.staging = [None] * (2 * self.n)    # uint8 frames of the host copies, frame f in f % 2n (its stream's)
         self.copied = [None] * (2 * self.n)     # event after the last copy out of each staging buffer
         self.copy_stream = None                 # the device-to-host stream, created on first use
+        self.t_staging = [None] * (2 * self.n)  # uint8 host targets uploaded for frame f in f % 2n
+        self.t_read = [None] * (2 * self.n)     # event after the quality pass that last read each of them
+        self.upload_stream = None               # the host-to-device stream, created on first use
         self._last_event = None
         self.i = 0
 
@@ -227,7 +280,10 @@ class FrameStreamer:
         k = self.i % self.n
         if (target is None) != (quality is None):
             raise RasterizerError("render: give both target and quality, or neither")
-        if target is not None:
+        rgb8 = isinstance(target, torch.Tensor) and target.dtype == torch.uint8
+        if rgb8:
+            self._check_rgb8_target(self.steps[k].color, target, quality)
+        elif target is not None:
             self._check_quality_args(self.steps[k].color, target, quality)
         if host_out is not None:
             self._check_host_out(self.steps[k].color, host_out)
@@ -235,11 +291,24 @@ class FrameStreamer:
         self.i += 1
         s = self.streams[k]
         s.wait_stream(torch.cuda.current_stream(self.device))      # V_front / V_back may have just been produced
+        uploaded = self._upload(j, target) if rgb8 and not target.is_cuda else None
         with torch.cuda.stream(s):
             self.mats[k][0].copy_(V_front, non_blocking=True)
             self.mats[k][1].copy_(V_back, non_blocking=True)
             color, _, _ = self.steps[k]()
-            if target is not None:
+            if rgb8:
+                quality.record_stream(s)
+                N, _, H, W = color.shape
+                if self.scratch[k] is None:
+                    self.scratch[k] = R._bytes(Q.scratch_bytes(N, H, W), self.device)
+                if uploaded is not None:
+                    s.wait_event(uploaded)
+                    frames = self.t_staging[j]
+                else:
+                    target.record_stream(s)
+                    frames = target
+                Q.quality_rgb8_into(quality.view(N, 3), color, frames.view(N, H, W, 3), None, self.scratch[k])
+            elif target is not None:
                 target.record_stream(s)
                 quality.record_stream(s)
                 N, _, H, W = color.shape
@@ -256,6 +325,8 @@ class FrameStreamer:
                     s.wait_event(self.copied[j])
                 E.rgb8_into(self.staging[j], color)
             self.events[k] = s.record_event()
+        if uploaded is not None:
+            self.t_read[j] = self.events[k]
         self._last = k
         self._last_event = self.events[k]
         if host_out is not None:
@@ -269,11 +340,40 @@ class FrameStreamer:
         frame = color.shape[1:] if color.shape[0] == 1 else color.shape
         if not isinstance(target, torch.Tensor) or target.device != self.device or target.shape != frame:
             raise RasterizerError(f"render: target must be a tensor of shape {tuple(frame)} on {self.device}")
+        self._check_quality_out(frame, quality)
+
+    def _check_quality_out(self, frame, quality):
         want = frame[:-3] + (3,)
         if (not isinstance(quality, torch.Tensor) or quality.device != self.device or quality.shape != want
                 or quality.dtype != torch.float32 or not quality.is_contiguous()):
             raise RasterizerError(f"render: quality must be a contiguous float32 tensor of shape {tuple(want)} "
                                   f"on {self.device}")
+
+    def _check_rgb8_target(self, color, target, quality):
+        frame = color.shape[1:] if color.shape[0] == 1 else color.shape
+        want = tuple(frame[:-3]) + (frame[-2], frame[-1], 3)
+        if tuple(target.shape) != want or not target.is_contiguous():
+            raise RasterizerError(f"render: a uint8 target must be a contiguous tensor of shape {want}, got "
+                                  f"{tuple(target.shape)}")
+        if target.is_cuda:
+            if target.device != self.device:
+                raise RasterizerError(f"render: target is on {target.device}, expected {self.device} or pinned host memory")
+        elif not target.is_pinned():
+            raise RasterizerError("render: a host target must be pinned (a copy from pageable memory blocks the host)")
+        self._check_quality_out(frame, quality)
+
+    def _upload(self, j, target):
+        """Enqueue the copy of pinned host frame `target` into staging buffer j; returns the event after it."""
+        if self.upload_stream is None:
+            self.upload_stream = torch.cuda.Stream(self.device)
+        if self.t_staging[j] is None:
+            self.t_staging[j] = torch.empty(target.shape, dtype=torch.uint8, device=self.device)
+        u = self.upload_stream
+        if self.t_read[j] is not None:
+            u.wait_event(self.t_read[j])            # the quality pass that read this buffer last
+        with torch.cuda.stream(u):
+            self.t_staging[j].copy_(target, non_blocking=True)
+            return u.record_event()
 
     def _check_host_out(self, color, host_out):
         frame = color.shape[1:] if color.shape[0] == 1 else color.shape
@@ -286,7 +386,8 @@ class FrameStreamer:
             raise RasterizerError(f"render: host_out must be a contiguous uint8 tensor of shape {want}")
 
     def last_event(self) -> torch.cuda.Event:
-        """The event recorded after everything `render` enqueued for the most recent frame, its host copy included."""
+        """The event recorded after everything `render` enqueued for the most recent frame, its host copy and the
+        upload of a host target included (the quality pass waits for the upload; this event follows both)."""
         if self._last_event is None:
             raise RasterizerError("last_event: no frame has been rendered yet")
         return self._last_event
@@ -296,7 +397,7 @@ class FrameStreamer:
         torch.cuda.current_stream(self.device).wait_event(self.events[self._last])
 
     def synchronize(self) -> None:
-        for s in self.streams + ([self.copy_stream] if self.copy_stream is not None else []):
+        for s in self.streams + [t for t in (self.copy_stream, self.upload_stream) if t is not None]:
             s.synchronize()
 
     def capacity_ok(self) -> bool:

@@ -9,12 +9,15 @@ reduction, deterministic, without host synchronisation and capturable in a CUDA 
 
 `image` is clamped to [0, 1] on read (the evaluation clamp), `gt` is used as given.  MS-SSIM is NaN when
 min(H, W) <= 160 (pytorch_msssim refuses such images); PSNR is +inf for identical images.  No gradient.
+
+`gt` may be the source video's 8-bit frames (SPEC U12, gsvc_b200.targets): uint8 [H,W,3] / [N,H,W,3], or a [F,H,W,3]
+cube with `index=` ([N] integer, on the device).  An index outside [0, F) gives that image a NaN row.
 """
 from __future__ import annotations
 
 import torch
 
-from . import _lib
+from . import _lib, targets as T8
 from .rasterizer import RasterizerError, _bytes, _dev_f32, _on_device, _require_cuda, _stream_ptr
 
 
@@ -43,11 +46,28 @@ def quality_into(out: torch.Tensor, images: torch.Tensor, targets: torch.Tensor,
                                             scratch.data_ptr(), _stream_ptr(images.device)), "gsvc_rast_quality")
 
 
-def frame_quality(images: torch.Tensor, targets: torch.Tensor) -> torch.Tensor:
+def quality_rgb8_into(out: torch.Tensor, images: torch.Tensor, frames: torch.Tensor, index, scratch: torch.Tensor) -> None:
+    """quality_into with 8-bit targets: `frames` uint8 [F,H,W,3] contiguous, `index` int32 [N] contiguous or None
+    (image n against frame n, N <= F), both on the images' device."""
+    N, _, H, W = images.shape
+    _lib.check(_lib.lib().gsvc_rast_quality_rgb8(N, H, W, images.data_ptr(), frames.data_ptr(), frames.shape[0],
+                                                 None if index is None else index.data_ptr(), out.data_ptr(),
+                                                 scratch.data_ptr(), _stream_ptr(images.device)),
+               "gsvc_rast_quality_rgb8")
+
+
+def frame_quality(images: torch.Tensor, targets: torch.Tensor, index: torch.Tensor = None) -> torch.Tensor:
     """(PSNR, SSIM, MS-SSIM) of each image against its target.
 
     `images`, `targets`: [3,H,W] (returns [3]) or [N,3,H,W] (returns [N,3]) CUDA tensors on the same device, cast to
-    fp32 and made contiguous.  The result is fp32 on that device and carries no gradient."""
+    fp32 and made contiguous.  The result is fp32 on that device and carries no gradient.
+
+    8-bit targets (SPEC U12): `targets` uint8 [H,W,3] / [N,H,W,3], or a [F,H,W,3] cube with `index` (integer [N] on
+    the device); bit for bit the fp32 result with `gsvc_b200.targets.to_float(frames, index)`."""
+    if T8.is_rgb8(targets):
+        return _frame_quality_rgb8(images, targets, index)
+    if index is not None:
+        raise RasterizerError("index selects frames of a uint8 target cube; these targets are not uint8")
     _check(images, targets)
     single = images.dim() == 3
     device = images.device
@@ -59,4 +79,23 @@ def frame_quality(images: torch.Tensor, targets: torch.Tensor) -> torch.Tensor:
         N, _, H, W = x.shape
         out = torch.empty((N, 3), dtype=torch.float32, device=device)
         quality_into(out, x, y, _bytes(scratch_bytes(N, H, W), device))
+    return out[0] if single else out
+
+
+def _frame_quality_rgb8(images, targets, index):
+    if not isinstance(images, torch.Tensor):
+        raise RasterizerError("images must be a tensor")
+    _require_cuda(images, "images")
+    if images.dim() not in (3, 4) or images.shape[-3] != 3 or images.numel() == 0:
+        raise RasterizerError(f"expected [3,H,W] or [N,3,H,W] images with N, H, W >= 1, got {tuple(images.shape)}")
+    single = images.dim() == 3
+    device = images.device
+    with torch.no_grad(), _on_device(device):
+        x = _dev_f32(images.detach(), device, "images")
+        if single:
+            x = x.unsqueeze(0)
+        frames, _, idx = T8.check(x, targets, index, single)
+        N, _, H, W = x.shape
+        out = torch.empty((N, 3), dtype=torch.float32, device=device)
+        quality_rgb8_into(out, x, frames, idx, _bytes(scratch_bytes(N, H, W), device))
     return out[0] if single else out

@@ -472,6 +472,31 @@ GSVC_RAST_API int gsvc_rast_quality(int32_t n_images, int32_t H, int32_t W, cons
 GSVC_RAST_API int gsvc_rast_frames_rgb8(int32_t n_images, int32_t H, int32_t W, const float *image,
                                         uint8_t *out /* [n_images,H,W,3], device-addressable */, void *stream);
 
+/*
+ * 8-bit source frames as targets (docs/SPEC.md "8-bit source frames", decision U12): the loss and quality calls above
+ * with the target read from a cube of 8-bit frames instead of an fp32 [n_images,3,H,W] tensor.  frames is
+ * [n_frames,H,W,3] uint8, RGB interleaved, row 0 first (what frames_rgb8 writes and np.array(PIL.Image) holds), device-
+ * addressable, any alignment.  Image n is compared with frame frame_index[n] (frame_index: [n_images] int32 on the
+ * device, read by the kernels, so a captured graph picks new frames through an in-place write), or with frame n when
+ * frame_index is NULL (then n_images <= n_frames).  A byte q reads as y = fl(q / 255), one correctly rounded division
+ * (torchvision's to_tensor): every result equals the fp32 call's with that target, bit for bit.  An index outside
+ * [0, n_frames) is never dereferenced: that image's loss and quality row are NaN and its dL_dimage is 0; the other
+ * images are unaffected.  Scratch sizes, launch counts and the size and lambda rules are those of the fp32 calls; a
+ * NULL pointer, n_frames < 1, a NULL frame_index with n_images > n_frames or n_frames * H * W * 3 beyond a 64-bit index
+ * is GSVC_RAST_ERR_INVALID too, before any CUDA work.
+ */
+GSVC_RAST_API int gsvc_rast_loss_forward_rgb8(int32_t n_images, int32_t H, int32_t W, const float *image,
+                                              const uint8_t *frames /* [n_frames,H,W,3] */, int32_t n_frames,
+                                              const int32_t *frame_index /* [n_images] device, or NULL */,
+                                              float lambda_dssim, float *loss, void *scratch, void *stream);
+GSVC_RAST_API int gsvc_rast_loss_backward_rgb8(int32_t n_images, int32_t H, int32_t W, const float *image,
+                                               const uint8_t *frames, int32_t n_frames, const int32_t *frame_index,
+                                               float lambda_dssim, const float *dL_dloss, float *dL_dimage,
+                                               void *stream);
+GSVC_RAST_API int gsvc_rast_quality_rgb8(int32_t n_images, int32_t H, int32_t W, const float *image,
+                                         const uint8_t *frames, int32_t n_frames, const int32_t *frame_index,
+                                         float *quality /* [n_images,3] */, void *scratch, void *stream);
+
 #ifdef __cplusplus
 }
 #endif
