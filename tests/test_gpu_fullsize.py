@@ -97,6 +97,8 @@ def test_config2_1080p_200k_forward_backward_vs_oracle(cuda_device, needle_mix):
 
 
 def test_config4_1080p_1M_forward_vs_oracle_and_stage_properties(cuda_device):
+    """BASELINE config 4: with more than 160 instances per tile the sort takes its dense path (sort_tiles_kernel<true>);
+    integer stages, forward and every visible Gaussian's gradient against the referee oracle behind it."""
     from gsvc_b200.rasterizer import RasterState
     cfg, g, rs, st = build(4, cuda_device)
     fo = oracle_forward(st, g)
@@ -104,26 +106,42 @@ def test_config4_1080p_1M_forward_vs_oracle_and_stage_properties(cuda_device):
     state = RasterState(rs, gd["means3D"], gd["opacities"], colors_precomp=gd["colors_precomp"], scales=gd["scales"],
                         rotations=gd["rotations"])
     assert state.num_rendered == fo["num_rendered"]
+    assert state.num_rendered / (((cfg["W"] + 15) // 16) * ((cfg["H"] + 15) // 16)) > 160
     check_forward(fo, state.color)
     check_stage_properties(state, cfg)
     keys, pl, ranges = state.export_keys()
     assert np.array_equal(pl.cpu().numpy().view(np.uint32), fo["bin"]["point_list"])     # bit-exact order at 3M+ instances
+    del state, keys, pl, ranges
+    gd, m2d, color, radii, n = run(rs, g, cuda_device, True)
+    assert n == fo["num_rendered"] and np.array_equal(radii.cpu().numpy(), fo["radii"])
+    check_forward(fo, color)
+    dL = parity.masked_dL(fo, torch.randn(color.shape, generator=torch.Generator().manual_seed(4)))
+    color.backward(torch.as_tensor(dL).to(cuda_device))
+    go = parity.oracle_backward(fo, dL)
+    got = {k: gd[k].grad for k in parity.GRAD_NAMES}
+    got["means2D"] = m2d.grad
+    parity.check_grads(fo, go, got)
 
 
 def test_config5_4k_2M_stress(cuda_device):
-    """4K, 2M Gaussians: 15-bit tile ids, multi-CTA scan (32 CTAs), scratch sized from the measured R."""
+    """4K, 2M Gaussians: 15-bit tile ids, multi-CTA scan (32 CTAs), scratch sized from the measured R; every visible
+    Gaussian's gradient against the referee oracle."""
     from gsvc_b200.rasterizer import RasterState
     cfg, g, rs, st = build(5, cuda_device)
     fo = oracle_forward(st, g)
     gd, m2d, color, radii, n = run(rs, g, cuda_device, True)
     assert n == fo["num_rendered"] and np.array_equal(radii.cpu().numpy(), fo["radii"])
     check_forward(fo, color)
+    names = ("means3D", "scales", "rotations", "opacities", "colors_precomp")
+    ins = [gd[k] for k in names]
+    dL = parity.masked_dL(fo, torch.randn(color.shape, generator=torch.Generator().manual_seed(55)))
+    got = dict(zip(names + ("means2D",), torch.autograd.grad(color, ins + [m2d], retain_graph=True,
+                                                             grad_outputs=torch.as_tensor(dL).to(cuda_device))))
+    parity.check_grads(fo, parity.oracle_backward(fo, dL), got)
     # backward: linearity in dL/dimage and exact zeros for culled Gaussians
     gen = torch.Generator().manual_seed(5)
     d1 = torch.randn(color.shape, generator=gen).to(cuda_device)
     d2 = torch.randn(color.shape, generator=gen).to(cuda_device)
-    names = ("means3D", "scales", "rotations", "opacities", "colors_precomp")
-    ins = [gd[k] for k in names]
     ga = torch.autograd.grad(color, ins, grad_outputs=d1, retain_graph=True)
     gb = torch.autograd.grad(color, ins, grad_outputs=d2, retain_graph=True)
     gc = torch.autograd.grad(color, ins, grad_outputs=d1 + 2 * d2)

@@ -411,13 +411,9 @@ def test_two_host_threads_on_their_own_streams(cuda_device):
 def test_heavy_tile_uses_global_sort_fallback(cuda_device):
     """> 4096 instances on one tile: the per-tile sort leaves shared memory; order must stay exact."""
     from gsvc_b200.rasterizer import RasterState
-    scene = make_scene(P=6000, W=64, H=48, F=64, seed=13)
+    from tests.deep_scenes import heavy_scene
+    scene = heavy_scene()                            # a seventh of the Gaussians tie in depth: order by Gaussian id
     gs = scene["gaussians"]
-    gs["means3D"][:, 0] = 0.02 * torch.randn(6000, generator=torch.Generator().manual_seed(1))
-    gs["means3D"][:, 1] = 0.02 * torch.randn(6000, generator=torch.Generator().manual_seed(2))
-    gs["means3D"][:, 2] = scene["frame"].z + 0.04 * (torch.rand(6000, generator=torch.Generator().manual_seed(3)) - 0.5)
-    gs["means3D"][::7, 2] = gs["means3D"][0, 2]      # exact depth ties: order falls back to the Gaussian id
-    gs["opacities"][:] = 0.02 + 0.02 * gs["opacities"]
     fo = _oracle_forward(scene)
     lens = fo["bin"]["ranges"][:, 1].astype(np.int64) - fo["bin"]["ranges"][:, 0]
     assert lens.max() > 4096
