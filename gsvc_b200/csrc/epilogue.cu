@@ -29,6 +29,16 @@ struct EpiIn {
     const float* bound_max;      // [3]
 };
 
+// The position before the clamp, rounded as the reference rounds it: fl(an + fl(fl(go + no) * gs)).  No FMA: a fused
+// v differs in the last bit, and next to a bound that flips the clamp and its gradient mask (docs/SPEC.md U13).
+__device__ __forceinline__ float position(float an, float go, float no, float gs)
+{
+    return __fadd_rn(an, __fmul_rn(__fadd_rn(go, no), gs));
+}
+
+// F.normalize's denominator: clamp_min(||q||, 1e-12), NaN propagating like clamp_min (fmaxf would return the eps).
+__device__ __forceinline__ float normalize_denom(float norm) { return norm < 1e-12f ? 1e-12f : norm; }
+
 __global__ void __launch_bounds__(256) epi_mark_kernel(EpiIn in, float* __restrict__ nop_full,
                                                        uint8_t* __restrict__ selection, unsigned int* __restrict__ ballots,
                                                        unsigned int* __restrict__ cta_count)
@@ -95,12 +105,11 @@ __global__ void __launch_bounds__(256) epi_write_kernel(EpiIn in, const unsigned
         color_out[3 * (size_t)j + c] = __ldg(in.color + e * 3 + c);
         const float sg = 1.0f / (1.0f + expf(-__ldg(sr + c)));                 // torch.sigmoid
         scaling_out[3 * (size_t)j + c] = __ldg(gs + 3 + c) * sg;
-        const float off = (__ldg(go + c) + __ldg(no + c)) * __ldg(gs + c);
-        const float v = __ldg(an + c) + off;
-        xyz[3 * (size_t)j + c] = fminf(fmaxf(v, __ldg(in.bound_min + c)), __ldg(in.bound_max + c));   // torch.clamp
+        const float v = position(__ldg(an + c), __ldg(go + c), __ldg(no + c), __ldg(gs + c));
+        xyz[3 * (size_t)j + c] = v != v ? v : fminf(fmaxf(v, __ldg(in.bound_min + c)), __ldg(in.bound_max + c));   // torch.clamp
     }
     const float q0 = __ldg(sr + 3), q1 = __ldg(sr + 4), q2 = __ldg(sr + 5), q3 = __ldg(sr + 6);
-    const float nrm = fmaxf(sqrtf(q0 * q0 + q1 * q1 + q2 * q2 + q3 * q3), 1e-12f);       // F.normalize, eps 1e-12
+    const float nrm = normalize_denom(sqrtf(q0 * q0 + q1 * q1 + q2 * q2 + q3 * q3));
     rot_out[4 * (size_t)j] = q0 / nrm; rot_out[4 * (size_t)j + 1] = q1 / nrm;
     rot_out[4 * (size_t)j + 2] = q2 / nrm; rot_out[4 * (size_t)j + 3] = q3 / nrm;
 }
@@ -143,20 +152,23 @@ __global__ void __launch_bounds__(128) epi_backward_kernel(EpiIn in, const int32
                 const float ds = __ldg(g.dscaling + 3 * (size_t)j + c);
                 d_sr[c] = ds * gs[3 + c] * sg * (1.0f - sg);
                 d_gs[3 + c] += ds * sg;
-                const float osum = __ldg(in.grid_offsets + (row * K + k) * 3 + c) + __ldg(in.neural_offset + e * 3 + c);
-                const float v = an[c] + osum * gs[c];
-                const float gx = (v >= lo[c] && v <= hi[c]) ? __ldg(g.dxyz + 3 * (size_t)j + c) : 0.f;   // clamp passes inside
+                const float go = __ldg(in.grid_offsets + (row * K + k) * 3 + c), no = __ldg(in.neural_offset + e * 3 + c);
+                const float osum = go + no;
+                const float v = position(an[c], go, no, gs[c]);            // the forward's v, bit for bit
+                const float gx = (v >= lo[c] && v <= hi[c]) ? __ldg(g.dxyz + 3 * (size_t)j + c) : 0.f;   // clamp passes on [lo, hi]
                 d_an[c] += gx;
                 d_no[c] = gx * gs[c];
                 d_gs[c] += gx * osum;
             }
             const float q[4] = {__ldg(sr + 3), __ldg(sr + 4), __ldg(sr + 5), __ldg(sr + 6)};
-            const float nrm = fmaxf(sqrtf(q[0] * q[0] + q[1] * q[1] + q[2] * q[2] + q[3] * q[3]), 1e-12f);
+            const float norm = sqrtf(q[0] * q[0] + q[1] * q[1] + q[2] * q[2] + q[3] * q[3]);
+            const float nrm = normalize_denom(norm);
             float dr[4], dot = 0.f;
 #pragma unroll
             for (int c = 0; c < 4; c++) { dr[c] = __ldg(g.drot + 4 * (size_t)j + c); dot += dr[c] * (q[c] / nrm); }
+            // below eps clamp_min passes no gradient to the norm: q / eps is linear in q
 #pragma unroll
-            for (int c = 0; c < 4; c++) d_sr[3 + c] = (dr[c] - (q[c] / nrm) * dot) / nrm;
+            for (int c = 0; c < 4; c++) d_sr[3 + c] = norm < 1e-12f ? dr[c] / nrm : (dr[c] - (q[c] / nrm) * dot) / nrm;
         }
         g.d_neural_opacity[e] = d_op * m;
         g.d_masks[e] = d_op * nop;

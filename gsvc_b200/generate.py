@@ -115,8 +115,13 @@ class _Epilogue(torch.autograd.Function):
         device = nop.device
         total = n_vis * K
         with torch.cuda.device(device):
-            z = lambda t, *shape: (torch.zeros(shape, dtype=_F32, device=device) if t is None else _c(t, device, "grad"))
-            dx, dc, do, ds, dr = z(d_xyz, M, 3), z(d_color, M, 3), z(d_opacity, M, 1), z(d_scaling, M, 3), z(d_rot, M, 4)
+            # an absent cotangent is zeros; with M = 0 none is read (every rank is -1), but the C-ABI takes non-NULL
+            # pointers, which empty tensors do not have: one row of zeros stands in
+            z = lambda t, *shape: (torch.zeros(shape, dtype=_F32, device=device) if t is None or M == 0 else
+                                   _c(t, device, "grad"))
+            m1 = max(M, 1)
+            dx, dc, do, ds, dr = z(d_xyz, m1, 3), z(d_color, m1, 3), z(d_opacity, m1, 1), z(d_scaling, m1, 3), \
+                z(d_rot, m1, 4)
             dn = None if d_nop_full is None else _c(d_nop_full, device, "grad")
             g_nop = torch.empty((max(total, 1),), dtype=_F32, device=device)
             g_col = torch.empty((max(total, 1) * 3,), dtype=_F32, device=device)
