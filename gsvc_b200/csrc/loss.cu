@@ -12,7 +12,9 @@
 // Backward (recompute, nothing stored by the forward): per pixel p of image n
 //     dSbar/dx(p) = 1/(3HW) sum_q w(q-p) [dS/dmu_x(q) + 2 x(p) dS/dExx(q) + y(p) dS/dExy(q)]
 // where dS/dmu_x contains -2 mu_x dS/dExx - mu_y dS/dExy: on flat patches the sum cancels like the variance.  The
-// CTA therefore takes a shift k (x and y at its tile centre) and correlates the three maps
+// CTA therefore takes a shift k (x and y at its tile centre, clamped into [0, 1] so that a NaN or infinite centre
+// leaves k finite and the NaN of the gradient where float64 autograd has it, within 10 px of the bad value) and
+// correlates the three maps
 //     a(q) = dS/dmu_x|direct - 2 (mu_x(q) - kx) e(q) - (mu_y(q) - ky) f(q),   e = dS/dExx,   f = dS/dExy
 // then dSbar/dx(p) = (A(p) + 2 (x(p) - kx) E(p) + (y(p) - ky) F(p)) / (3HW) with A, E, F the window sums of a, e, f.  The maps are recomputed over the tile plus a 5-pixel ring (moments from a
 // 10-pixel halo of x and y): about 2.5x the forward's FMAs, but only x and y are read and dL/dx written once.
@@ -61,13 +63,14 @@ __device__ __forceinline__ void vpass(const float* h, int hrows, int cols, int i
     }
 }
 
-// the shift of a CTA: x and y at its tile centre, clamped into the image
+// the shift of a CTA: x and y at its tile centre (clamped into the image), each clamped into [0, 1].  Any finite k
+// gives the same value; a NaN or infinite centre would make every map value of the tile NaN (fmaxf maps NaN to 0).
 template <class Y>
 __device__ __forceinline__ void tile_shift(const float* x, Y y, int H, int W, int ty, int tx, float& kx, float& ky)
 {
     const int r = min(ty * T + T / 2, H - 1), c = min(tx * T + T / 2, W - 1);
-    kx = __ldg(x + (size_t)r * W + c);
-    ky = y((size_t)r * W + c);
+    kx = fminf(fmaxf(__ldg(x + (size_t)r * W + c), 0.0f), 1.0f);
+    ky = fminf(fmaxf(y((size_t)r * W + c), 0.0f), 1.0f);
 }
 
 // Tgt: PlanarTarget (fp32) or Rgb8Target (ssim.cuh); a CTA whose target frame is out of range leaves a NaN partial

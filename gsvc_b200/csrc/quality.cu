@@ -14,8 +14,6 @@
 
 #include <math.h>
 
-#include <type_traits>
-
 namespace gsvc {
 
 namespace quality {
@@ -166,9 +164,8 @@ struct ReduceArgs {
 };
 
 // One CTA per image: every (channel, level) sum in a fixed order (strided per thread, butterfly per warp, warps in
-// index order), then PSNR, SSIM and MS-SSIM in double.  NAN_ROWS (8-bit targets, whose values are finite): a NaN
-// level-0 sum marks an out-of-range frame, and the whole row is NaN (MS-SSIM's clamp at 0 would otherwise hide it).
-template <bool NAN_ROWS>
+// index order), then PSNR, SSIM and MS-SSIM in double.  The relu of MS-SSIM keeps NaN, as pytorch_msssim's does: a NaN
+// in x or y, or a target frame out of range, makes the MS-SSIM entry NaN.
 __global__ void __launch_bounds__(THREADS) quality_reduce_kernel(ReduceArgs a, float* __restrict__ quality)
 {
     __shared__ double s_w[4][THREADS / 32];
@@ -210,13 +207,12 @@ __global__ void __launch_bounds__(THREADS) quality_reduce_kernel(ReduceArgs a, f
             double prod = 1.0;
             for (int l = 0; l < LEVELS; l++) {
                 const double m = s_tot[c][l][l == LEVELS - 1 ? 2 : 3] / a.valid[l];   // cs of levels 0-3, ssim of 4
-                prod *= pow(fmax(m, 0.0), wt[l]);
+                prod *= pow(m > 0.0 || isnan(m) ? m : 0.0, wt[l]);
             }
             ms += prod;
         }
         ms /= 3.0;
     }
-    if (NAN_ROWS && isnan(ss)) ms = (double)NAN;
     float* out = quality + (size_t)blockIdx.x * 3;
     out[0] = (float)psnr;
     out[1] = (float)(ss / a.count);
@@ -247,7 +243,6 @@ static int quality_run(int32_t n_images, int32_t H, int32_t W, const float* imag
                        void* scratch, cudaStream_t st)
 {
     using namespace quality;
-    constexpr bool rgb8 = !std::is_same<Tgt, PlanarTarget>::value;
     const Layout L = layout(n_images, H, W);
     char* base = static_cast<char*>(scratch);
     const int levels = (H < MS_MIN_SIDE || W < MS_MIN_SIDE) ? 1 : LEVELS;   // no pyramid without MS-SSIM
@@ -272,7 +267,7 @@ static int quality_run(int32_t n_images, int32_t H, int32_t W, const float* imag
                            reinterpret_cast<const float*>(base + L.img_x[l]),
                            PlanarTarget{reinterpret_cast<const float*>(base + L.img_y[l])}, part, xo, yo);
     }
-    if (e == cudaSuccess) e = launch_pdl(quality_reduce_kernel<rgb8>, dim3(n_images), dim3(THREADS), st, ra, quality);
+    if (e == cudaSuccess) e = launch_pdl(quality_reduce_kernel, dim3(n_images), dim3(THREADS), st, ra, quality);
     count_launch(levels + 1);
     if (e == cudaSuccess) e = cudaGetLastError();
     return e == cudaSuccess ? GSVC_RAST_OK : fail(GSVC_RAST_ERR_CUDA, "quality: %s", cudaGetErrorString(e));

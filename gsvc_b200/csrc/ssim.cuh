@@ -80,7 +80,8 @@ struct Rgb8Target {
 };
 
 // Stage rows [r0, r0+rows) x cols [c0, c0+cols) of x and y (0 outside the image: the zero padding) into sx / sy.
-// CLAMP_X: x is read clamped to [0, 1].  y: a target plane reader (PlanarTarget::Plane, Rgb8Target::Plane).
+// CLAMP_X: x is read clamped to [0, 1] as torch.clamp does it: NaN stays NaN, +-Inf become 1 / 0.
+// y: a target plane reader (PlanarTarget::Plane, Rgb8Target::Plane).
 template <bool CLAMP_X = false, class Y>
 __device__ __forceinline__ void stage(const float* __restrict__ x, Y y, int H, int W, int r0, int c0, int rows,
                                       int cols, float* sx, float* sy)
@@ -93,7 +94,7 @@ __device__ __forceinline__ void stage(const float* __restrict__ x, Y y, int H, i
             const size_t o = (size_t)gr * W + gc;
             vx = __ldg(x + o);
             vy = y(o);
-            if (CLAMP_X) vx = fminf(fmaxf(vx, 0.0f), 1.0f);
+            if (CLAMP_X) vx = vx < 0.0f ? 0.0f : (vx > 1.0f ? 1.0f : vx);
         }
         sx[e] = vx;
         sy[e] = vy;

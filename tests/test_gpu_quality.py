@@ -25,26 +25,38 @@ def _fused(x, y):
     return frame_quality(x, y)
 
 
+def _masks_equal(a, b):
+    return torch.equal(torch.isnan(a), torch.isnan(b)) and torch.equal(torch.isposinf(a), torch.isposinf(b)) \
+        and torch.equal(torch.isneginf(a), torch.isneginf(b))
+
+
 def check(x, y):
-    """x, y [N,3,H,W] CUDA.  Compares with the float64 oracle (run on the GPU); returns whether MS-SSIM qualified."""
+    """x, y [N,3,H,W] CUDA.  Compares with the float64 oracle (run on the GPU); returns whether MS-SSIM qualified.
+    NaN and infinities of each metric must be the oracle's; the bars hold on the finite entries."""
     from gsvc_b200.loss import photometric_loss
     N, _, H, W = x.shape
     q = _fused(x, y).double().cpu()
     xd, yd = x.double(), y.double()
-    ref = torch.stack([quality_oracle.psnr(xd, yd), quality_oracle.ssim(xd, yd)], dim=1).cpu()
+    ref = quality_oracle.frame_quality(xd, yd).cpu()
+    for k in range(3):
+        assert _masks_equal(q[:, k], ref[:, k]), (k, q[:, k], ref[:, k])
     finite = torch.isfinite(ref[:, 0])
-    assert torch.equal(torch.isfinite(q[:, 0]), finite), (q[:, 0], ref[:, 0])
     if finite.any():
         assert (q[finite, 0] - ref[finite, 0]).abs().max().item() <= PSNR_TOL, (q[:, 0], ref[:, 0])
-    assert (q[:, 1] - ref[:, 1]).abs().max().item() <= SSIM_TOL, (q[:, 1], ref[:, 1])
-    one_minus_loss = 1.0 - photometric_loss(x.float().clamp(0.0, 1.0), y.float(), 1.0).double().cpu()
-    assert (q[:, 1] - one_minus_loss).abs().max().item() <= SSIM_TOL
+    fs = torch.isfinite(ref[:, 1])
+    if fs.any():
+        assert (q[fs, 1] - ref[fs, 1]).abs().max().item() <= SSIM_TOL, (q[:, 1], ref[:, 1])
+        one_minus_loss = 1.0 - photometric_loss(x.float().clamp(0.0, 1.0), y.float(), 1.0).double().cpu()
+        assert (q[fs, 1] - one_minus_loss[fs]).abs().max().item() <= SSIM_TOL
     if min(H, W) < quality_oracle.MIN_SIDE:
         assert torch.isnan(q[:, 2]).all()
         return False
+    fm = torch.isfinite(ref[:, 2])
+    if not fm.any():
+        return False
     a = quality_oracle.ms_ssim_args(xd, yd)
     ms_ref, per_c = quality_oracle.ms_ssim_from_args(a)
-    a, ms_ref, per_c = a.cpu(), ms_ref.cpu(), per_c.cpu()
+    a, ms_ref, per_c, q = a.cpu()[fm], ms_ref.cpu()[fm], per_c.cpu()[fm], q[fm]
     w = torch.tensor(quality_oracle.WEIGHTS, dtype=torch.float64)
     zero = (a <= -1e-5).any(dim=-1)                                   # [N,3]
     regular = (a >= 1e-4).all(dim=-1)
@@ -115,6 +127,36 @@ def test_sizes(cuda_device, hw):
     x = torch.rand((1, 3) + hw, generator=_gen(hw[0] + hw[1])).to(cuda_device)
     y = _noisy(x, 0.05, 11)
     assert check(x, y) == (min(hw) > 160)
+
+
+@pytest.mark.parametrize("where", ["x centre", "x corner", "y"])
+def test_nan_is_not_black(cuda_device, where):
+    """A NaN in the rendered frame (at a level-0 tile centre, in a corner) or in an fp32 target makes that image's
+    PSNR, SSIM and MS-SSIM NaN, as torch.clamp and pytorch_msssim's relu keep it; the other image is unchanged."""
+    x = torch.rand((2, 3, 171, 333), generator=_gen(30)).to(cuda_device)
+    y = _noisy(x, 0.05, 31)
+    ok = _fused(x, y)
+    t = x if where.startswith("x") else y
+    t[1, 1][(0, 0) if where == "x corner" else (16, 48)] = math.nan
+    q = _fused(x, y)
+    assert torch.isnan(q[1]).all() and torch.equal(q[0], ok[0])
+    check(x, y)
+
+
+def test_infinities(cuda_device):
+    """+-Inf in x clamp to 1 / 0 (finite metrics within the bars); +Inf in y gives PSNR -inf, SSIM and MS-SSIM NaN."""
+    x = torch.rand((2, 3, 171, 333), generator=_gen(32)).to(cuda_device)
+    y = _noisy(x, 0.05, 33)
+    xi = x.clone()
+    xi[0, 0, 16, 48] = math.inf
+    xi[1, 2, 100, 7] = -math.inf
+    assert check(xi, y)
+    assert torch.isfinite(_fused(xi, y)).all()
+    yi = y.clone()
+    yi[1, 0, 16, 48] = math.inf
+    check(x, yi)
+    q = _fused(x, yi).cpu()
+    assert q[1, 0] == -math.inf and torch.isnan(q[1, 1:]).all() and torch.isfinite(q[0]).all()
 
 
 def test_closed_forms(cuda_device):
