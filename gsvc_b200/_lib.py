@@ -82,11 +82,22 @@ SIGNATURES = {
                                            _vp]),
     "gsvc_rast_backward_views_exchange": (C.c_int, [_SP, _i32, _VP, _i32, _i32, _i32, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
                                                     _vp, _vp, _vp, _vp, _i32, _vp, _vp, _vp, C.POINTER(Exchange), _vp]),
+    # deterministic twins (docs/SPEC.md U14): the twin's arguments, then (partials, partials_bytes) before the stream
+    "gsvc_rast_backward_partials_bytes": (_sz, [_i64]),
+    "gsvc_rast_backward_views_det": (C.c_int, [_SP, _i32, _VP, _i32, _i32, _i32, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
+                                               _vp, _vp, _vp, _vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
+                                               _vp, _sz, _vp]),
+    "gsvc_rast_backward_views_exchange_det": (C.c_int, [_SP, _i32, _VP, _i32, _i32, _i32, _i64, _vp, _vp, _vp, _vp, _vp, _vp,
+                                                        _vp, _vp, _vp, _vp, _vp, _i32, _vp, _vp, _vp, C.POINTER(Exchange),
+                                                        _vp, _sz, _vp]),
     "gsvc_rast_forward_ragged_launch": (C.c_int, [_SP, _i32, _VP, _i32, _vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
                                                   _vp, _vp, _vp, _i64, _vp, _vp, _vp, _vp, C.c_uint32, _vp]),
     "gsvc_rast_forward_ragged_render": (C.c_int, [_SP, _i32, _VP, _i32, _vp, _vp, _vp, _vp, _i64, _vp, _vp]),
     "gsvc_rast_backward_ragged": (C.c_int, [_SP, _i32, _VP, _i32, _vp, _i32, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
                                             _vp, _vp, _vp, _vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "gsvc_rast_backward_ragged_det": (C.c_int, [_SP, _i32, _VP, _i32, _vp, _i32, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
+                                                _vp, _vp, _vp, _vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
+                                                _sz, _vp]),
     "gsvc_rast_export_keys": (C.c_int, [_SP, _i32, _i64, _vp, _vp, _vp, _vp, _vp, _vp]),
     "gsvc_rast_export_geom": (C.c_int, [_i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "gsvc_rast_export_image": (C.c_int, [_SP, _i32, _vp, _vp, _vp, _vp]),

@@ -181,6 +181,7 @@ size_t gsvc_rast_image_bytes_views(int32_t W, int32_t H, int32_t n_views)
 }
 size_t gsvc_rast_binning_bytes(int64_t cap) { return bin_bytes(cap < 1 ? 1 : cap); }
 size_t gsvc_rast_backward_scratch_bytes(int32_t P) { return bwd_scratch_bytes(P < 1 ? 1 : P); }
+size_t gsvc_rast_backward_partials_bytes(int64_t capacity) { return det_partials_bytes(capacity < 1 ? 1 : capacity); }
 int64_t gsvc_rast_launch_count(int32_t reset)
 {
     return reset ? g_launches.exchange(0) : g_launches.load();
@@ -487,7 +488,8 @@ static int backward_core(const gsvc_rast_settings* st, const DevSettings& d, int
                          const float* means3D, const float* shs, const float* colors_precomp, const float* scales,
                          const float* rotations, const float* cov3D_precomp, const int32_t* radii, const void* geom,
                          const void* image, const void* binning, void* scratch, int32_t scratch_is_zero,
-                         const float* dL_dout, BwdOutputs out, cudaStream_t stream, ExchangeArgs ex = ExchangeArgs{})
+                         const float* dL_dout, BwdOutputs out, cudaStream_t stream, ExchangeArgs ex = ExchangeArgs{},
+                         bool det = false, void* partials = nullptr, size_t partials_bytes = 0)
 {
     int rc = check_inputs(P, sh_M, st->sh_degree, means3D, shs, colors_precomp, reinterpret_cast<const float*>(1), scales,
                           rotations, cov3D_precomp, true);
@@ -498,13 +500,25 @@ static int backward_core(const gsvc_rast_settings* st, const DevSettings& d, int
     if (capacity <= 0 || !binning) return fail(GSVC_RAST_ERR_INVALID, "binning is NULL or capacity <= 0");
     if (out.packed && (shs || cov3D_precomp))
         return fail(GSVC_RAST_ERR_INVALID, "dL_packed needs colors_precomp and the scale/rotation pair");
+    if (det && !partials) return fail(GSVC_RAST_ERR_INVALID, "partials is NULL");
+    if (det && partials_bytes < det_partials_bytes(capacity))
+        return fail(GSVC_RAST_ERR_INVALID, "partials holds %zu bytes, capacity %lld needs %zu",
+                    partials_bytes, (long long)capacity, det_partials_bytes(capacity));
     const bool dbg = st->debug != 0;
     GeomView g = geom_view(const_cast<void*>(geom), state_rows(d, P < 1 ? 1 : P), d.sh_M);
     ImageView im = image_view(const_cast<void*>(image), d.W, d.H, d.n_views);
     BinView b = bin_view(const_cast<void*>(binning), capacity);
     float4* acc = static_cast<float4*>(scratch);
     PreInputs in{P, means3D, shs, colors_precomp, nullptr, scales, rotations, cov3D_precomp, 0, P};
-    { StageScope t(ST_RENDER_BWD, stream); CK(launch_render_backward(d, state_rows(d, P), g, im, b, capacity, dL_dout, acc, scratch_is_zero != 0, stream), "render_backward"); }
+    if (det) {
+        StageScope t(ST_RENDER_BWD, stream);
+        CK(launch_render_backward_det(d, P, state_rows(d, P), g, im, b, capacity, dL_dout, acc, partials, stream),
+           "render_backward_det");
+    } else {
+        StageScope t(ST_RENDER_BWD, stream);
+        CK(launch_render_backward(d, state_rows(d, P), g, im, b, capacity, dL_dout, acc, scratch_is_zero != 0, stream),
+           "render_backward");
+    }
     { StageScope t(ST_PREPROCESS_BWD, stream); CK(launch_preprocess_backward(d, in, radii, g, acc, out, ex, stream), "preprocess_backward"); }
     return 0;
 }
@@ -527,14 +541,15 @@ int gsvc_rast_backward(const gsvc_rast_settings* st, int32_t P, int32_t sh_M, in
                          geom, image, binning, scratch, scratch_is_zero, dL_dout, out, static_cast<cudaStream_t>(stream_));
 }
 
-int gsvc_rast_backward_views(const gsvc_rast_settings* st, int32_t n_views, const gsvc_rast_view* views_host,
+static int backward_views_impl(const gsvc_rast_settings* st, int32_t n_views, const gsvc_rast_view* views_host,
                              int32_t n_out, int32_t P, int32_t sh_M, int64_t capacity, const float* means3D,
                              const float* shs, const float* colors_precomp, const float* scales,
                              const float* rotations, const float* cov3D_precomp, const int32_t* radii,
                              const void* geom, const void* image, const void* binning, void* scratch,
                              int32_t scratch_is_zero, const float* dL_dout, float* dL_dmeans3D, float* dL_dmeans2D,
                              float* dL_dcolors, float* dL_dopacities, float* dL_dscales, float* dL_drotations,
-                             float* dL_dcov3D, float* dL_dshs, float* dL_packed, void* stream_)
+                             float* dL_dcov3D, float* dL_dshs, float* dL_packed, bool det, void* partials,
+                             size_t partials_bytes, void* stream_)
 {
     DevSettings d;
     int rc = make_settings_views(st, n_views, views_host, n_out, shs ? sh_M : 0, d);
@@ -542,16 +557,18 @@ int gsvc_rast_backward_views(const gsvc_rast_settings* st, int32_t n_views, cons
     BwdOutputs out{dL_dmeans3D, dL_dmeans2D, dL_dcolors, dL_dopacities, dL_dscales, dL_drotations, dL_dcov3D, dL_dshs,
                    dL_packed};
     return backward_core(st, d, P, sh_M, capacity, means3D, shs, colors_precomp, scales, rotations, cov3D_precomp, radii,
-                         geom, image, binning, scratch, scratch_is_zero, dL_dout, out, static_cast<cudaStream_t>(stream_));
+                         geom, image, binning, scratch, scratch_is_zero, dL_dout, out, static_cast<cudaStream_t>(stream_),
+                         ExchangeArgs{}, det, partials, partials_bytes);
 }
 
-int gsvc_rast_backward_views_exchange(const gsvc_rast_settings* st, int32_t n_views, const gsvc_rast_view* views_host,
+static int backward_views_exchange_impl(const gsvc_rast_settings* st, int32_t n_views, const gsvc_rast_view* views_host,
                                       int32_t n_out, int32_t P, int32_t sh_M, int64_t capacity, const float* means3D,
                                       const float* shs, const float* colors_precomp, const float* scales,
                                       const float* rotations, const float* cov3D_precomp, const int32_t* radii,
                                       const void* geom, const void* image, const void* binning, void* scratch,
                                       int32_t scratch_is_zero, const float* dL_dout, float* dL_dmeans2D,
-                                      float* dL_packed, const gsvc_rast_exchange* x, void* stream_)
+                                      float* dL_packed, const gsvc_rast_exchange* x, bool det, void* partials,
+                                      size_t partials_bytes, void* stream_)
 {
     if (!x) return fail(GSVC_RAST_ERR_INVALID, "exchange is NULL");
     if (!dL_packed) return fail(GSVC_RAST_ERR_INVALID, "the exchange sums the packed [P,14] rows: dL_packed is NULL");
@@ -591,7 +608,7 @@ int gsvc_rast_backward_views_exchange(const gsvc_rast_settings* st, int32_t n_vi
     BwdOutputs out{nullptr, dL_dmeans2D, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, dL_packed};
     return backward_core(st, d, P, sh_M, capacity, means3D, shs, colors_precomp, scales, rotations, cov3D_precomp, radii,
                          geom, image, binning, scratch, scratch_is_zero, dL_dout, out, static_cast<cudaStream_t>(stream_),
-                         ex);
+                         ex, det, partials, partials_bytes);
 }
 
 int gsvc_rast_forward_ragged_launch(const gsvc_rast_settings* st, int32_t n_views, const gsvc_rast_view* views_host,
@@ -622,6 +639,89 @@ int gsvc_rast_forward_ragged_render(const gsvc_rast_settings* st, int32_t n_view
                                static_cast<cudaStream_t>(stream_));
 }
 
+static int backward_ragged_impl(const gsvc_rast_settings* st, int32_t n_views, const gsvc_rast_view* views_host,
+                              int32_t n_out, const int32_t* counts_host, int32_t sh_M, int64_t capacity,
+                              const float* means3D, const float* shs, const float* colors_precomp, const float* scales,
+                              const float* rotations, const float* cov3D_precomp, const int32_t* radii,
+                              const void* geom, const void* image, const void* binning, void* scratch,
+                              int32_t scratch_is_zero, const float* dL_dout, float* dL_dmeans3D, float* dL_dmeans2D,
+                              float* dL_dcolors, float* dL_dopacities, float* dL_dscales, float* dL_drotations,
+                              float* dL_dcov3D, float* dL_dshs, bool det, void* partials, size_t partials_bytes,
+                              void* stream_)
+{
+    DevSettings d;
+    int32_t P = 0;
+    int rc = make_settings_ragged(st, n_views, views_host, n_out, counts_host, shs ? sh_M : 0, d, P);
+    if (rc) return rc;
+    BwdOutputs out{dL_dmeans3D, dL_dmeans2D, dL_dcolors, dL_dopacities, dL_dscales, dL_drotations, dL_dcov3D, dL_dshs,
+                   nullptr};
+    return backward_core(st, d, P, sh_M, capacity, means3D, shs, colors_precomp, scales, rotations, cov3D_precomp, radii,
+                         geom, image, binning, scratch, scratch_is_zero, dL_dout, out, static_cast<cudaStream_t>(stream_),
+                         ExchangeArgs{}, det, partials, partials_bytes);
+}
+
+// ---- the backward entry points Python calls, atomic and deterministic (docs/SPEC.md U14): twins over one implementation
+
+int gsvc_rast_backward_views(const gsvc_rast_settings* st, int32_t n_views, const gsvc_rast_view* views_host,
+                             int32_t n_out, int32_t P, int32_t sh_M, int64_t capacity, const float* means3D,
+                             const float* shs, const float* colors_precomp, const float* scales,
+                             const float* rotations, const float* cov3D_precomp, const int32_t* radii,
+                             const void* geom, const void* image, const void* binning, void* scratch,
+                             int32_t scratch_is_zero, const float* dL_dout, float* dL_dmeans3D, float* dL_dmeans2D,
+                             float* dL_dcolors, float* dL_dopacities, float* dL_dscales, float* dL_drotations,
+                             float* dL_dcov3D, float* dL_dshs, float* dL_packed, void* stream_)
+{
+    return backward_views_impl(st, n_views, views_host, n_out, P, sh_M, capacity, means3D, shs, colors_precomp, scales,
+                               rotations, cov3D_precomp, radii, geom, image, binning, scratch, scratch_is_zero, dL_dout,
+                               dL_dmeans3D, dL_dmeans2D, dL_dcolors, dL_dopacities, dL_dscales, dL_drotations, dL_dcov3D,
+                               dL_dshs, dL_packed, false, nullptr, 0, stream_);
+}
+
+int gsvc_rast_backward_views_det(const gsvc_rast_settings* st, int32_t n_views, const gsvc_rast_view* views_host,
+                                 int32_t n_out, int32_t P, int32_t sh_M, int64_t capacity, const float* means3D,
+                                 const float* shs, const float* colors_precomp, const float* scales,
+                                 const float* rotations, const float* cov3D_precomp, const int32_t* radii,
+                                 const void* geom, const void* image, const void* binning, void* scratch,
+                                 int32_t scratch_is_zero, const float* dL_dout, float* dL_dmeans3D, float* dL_dmeans2D,
+                                 float* dL_dcolors, float* dL_dopacities, float* dL_dscales, float* dL_drotations,
+                                 float* dL_dcov3D, float* dL_dshs, float* dL_packed, void* partials,
+                                 size_t partials_bytes, void* stream_)
+{
+    return backward_views_impl(st, n_views, views_host, n_out, P, sh_M, capacity, means3D, shs, colors_precomp, scales,
+                               rotations, cov3D_precomp, radii, geom, image, binning, scratch, scratch_is_zero, dL_dout,
+                               dL_dmeans3D, dL_dmeans2D, dL_dcolors, dL_dopacities, dL_dscales, dL_drotations, dL_dcov3D,
+                               dL_dshs, dL_packed, true, partials, partials_bytes, stream_);
+}
+
+int gsvc_rast_backward_views_exchange(const gsvc_rast_settings* st, int32_t n_views, const gsvc_rast_view* views_host,
+                                      int32_t n_out, int32_t P, int32_t sh_M, int64_t capacity, const float* means3D,
+                                      const float* shs, const float* colors_precomp, const float* scales,
+                                      const float* rotations, const float* cov3D_precomp, const int32_t* radii,
+                                      const void* geom, const void* image, const void* binning, void* scratch,
+                                      int32_t scratch_is_zero, const float* dL_dout, float* dL_dmeans2D,
+                                      float* dL_packed, const gsvc_rast_exchange* x, void* stream_)
+{
+    return backward_views_exchange_impl(st, n_views, views_host, n_out, P, sh_M, capacity, means3D, shs, colors_precomp,
+                                        scales, rotations, cov3D_precomp, radii, geom, image, binning, scratch,
+                                        scratch_is_zero, dL_dout, dL_dmeans2D, dL_packed, x, false, nullptr, 0, stream_);
+}
+
+int gsvc_rast_backward_views_exchange_det(const gsvc_rast_settings* st, int32_t n_views,
+                                          const gsvc_rast_view* views_host, int32_t n_out, int32_t P, int32_t sh_M,
+                                          int64_t capacity, const float* means3D, const float* shs,
+                                          const float* colors_precomp, const float* scales, const float* rotations,
+                                          const float* cov3D_precomp, const int32_t* radii, const void* geom,
+                                          const void* image, const void* binning, void* scratch,
+                                          int32_t scratch_is_zero, const float* dL_dout, float* dL_dmeans2D,
+                                          float* dL_packed, const gsvc_rast_exchange* x, void* partials,
+                                          size_t partials_bytes, void* stream_)
+{
+    return backward_views_exchange_impl(st, n_views, views_host, n_out, P, sh_M, capacity, means3D, shs, colors_precomp,
+                                        scales, rotations, cov3D_precomp, radii, geom, image, binning, scratch,
+                                        scratch_is_zero, dL_dout, dL_dmeans2D, dL_packed, x, true, partials,
+                                        partials_bytes, stream_);
+}
+
 int gsvc_rast_backward_ragged(const gsvc_rast_settings* st, int32_t n_views, const gsvc_rast_view* views_host,
                               int32_t n_out, const int32_t* counts_host, int32_t sh_M, int64_t capacity,
                               const float* means3D, const float* shs, const float* colors_precomp, const float* scales,
@@ -631,14 +731,26 @@ int gsvc_rast_backward_ragged(const gsvc_rast_settings* st, int32_t n_views, con
                               float* dL_dcolors, float* dL_dopacities, float* dL_dscales, float* dL_drotations,
                               float* dL_dcov3D, float* dL_dshs, void* stream_)
 {
-    DevSettings d;
-    int32_t P = 0;
-    int rc = make_settings_ragged(st, n_views, views_host, n_out, counts_host, shs ? sh_M : 0, d, P);
-    if (rc) return rc;
-    BwdOutputs out{dL_dmeans3D, dL_dmeans2D, dL_dcolors, dL_dopacities, dL_dscales, dL_drotations, dL_dcov3D, dL_dshs,
-                   nullptr};
-    return backward_core(st, d, P, sh_M, capacity, means3D, shs, colors_precomp, scales, rotations, cov3D_precomp, radii,
-                         geom, image, binning, scratch, scratch_is_zero, dL_dout, out, static_cast<cudaStream_t>(stream_));
+    return backward_ragged_impl(st, n_views, views_host, n_out, counts_host, sh_M, capacity, means3D, shs,
+                                colors_precomp, scales, rotations, cov3D_precomp, radii, geom, image, binning, scratch,
+                                scratch_is_zero, dL_dout, dL_dmeans3D, dL_dmeans2D, dL_dcolors, dL_dopacities,
+                                dL_dscales, dL_drotations, dL_dcov3D, dL_dshs, false, nullptr, 0, stream_);
+}
+
+int gsvc_rast_backward_ragged_det(const gsvc_rast_settings* st, int32_t n_views, const gsvc_rast_view* views_host,
+                                  int32_t n_out, const int32_t* counts_host, int32_t sh_M, int64_t capacity,
+                                  const float* means3D, const float* shs, const float* colors_precomp,
+                                  const float* scales, const float* rotations, const float* cov3D_precomp,
+                                  const int32_t* radii, const void* geom, const void* image, const void* binning,
+                                  void* scratch, int32_t scratch_is_zero, const float* dL_dout, float* dL_dmeans3D,
+                                  float* dL_dmeans2D, float* dL_dcolors, float* dL_dopacities, float* dL_dscales,
+                                  float* dL_drotations, float* dL_dcov3D, float* dL_dshs, void* partials,
+                                  size_t partials_bytes, void* stream_)
+{
+    return backward_ragged_impl(st, n_views, views_host, n_out, counts_host, sh_M, capacity, means3D, shs,
+                                colors_precomp, scales, rotations, cov3D_precomp, radii, geom, image, binning, scratch,
+                                scratch_is_zero, dL_dout, dL_dmeans3D, dL_dmeans2D, dL_dcolors, dL_dopacities,
+                                dL_dscales, dL_drotations, dL_dcov3D, dL_dshs, true, partials, partials_bytes, stream_);
 }
 
 int gsvc_rast_export_keys(const gsvc_rast_settings* st, int32_t n_views, int64_t capacity, const void* image,

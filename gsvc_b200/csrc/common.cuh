@@ -183,6 +183,29 @@ inline size_t bin_bytes(long long cap)
 //  Cholesky factor in feat3; preprocess_backward turns the moments into dL/dpix, dL/dcov2D (a congruence with L)
 inline size_t bwd_scratch_bytes(int P) { return align_up((size_t)P * 48, 256) + 256; }
 
+// Partials of the deterministic blend backward (docs/SPEC.md U14), per instance of the binning capacity:
+//  val [cap][4][9]  the 9 half-warp sums of the instance's hit on each 8x8 block of its tile (blocks row-major)
+//  hit [cap][4]     one byte per (instance, block): non-zero when that slot was written; zeroed before every backward
+struct DetPartials {
+    float* val;
+    unsigned char* hit;
+};
+template <typename F>
+__host__ __device__ inline DetPartials det_partials(F* buf, unsigned long long cap)
+{
+    char* p = reinterpret_cast<char*>(const_cast<float*>(buf));
+    DetPartials d;
+    d.val = carve<float>(p, (size_t)cap * 36);
+    d.hit = reinterpret_cast<unsigned char*>(carve<unsigned int>(p, (size_t)cap));
+    return d;
+}
+inline size_t det_partials_bytes(long long cap)
+{
+    char* p = nullptr;
+    carve<float>(p, (size_t)cap * 36); carve<unsigned int>(p, (size_t)cap);
+    return (size_t)p + 256;
+}
+
 // U2: order-preserving float -> uint32 (ascending key == ascending view depth, negatives included)
 __host__ __device__ inline unsigned int ordered_u32(float z)
 {
@@ -389,6 +412,10 @@ cudaError_t launch_render_forward(const DevSettings& s, GeomView g, ImageView im
                                   float* out_color, cudaStream_t st);
 cudaError_t launch_render_backward(const DevSettings& s, int rows, GeomView g, ImageView im, BinView b, long long cap,
                                    const float* dL_dout, float4* acc, bool acc_is_zero, cudaStream_t st);
+// the deterministic form (docs/SPEC.md U14): `partials` holds det_partials_bytes(cap); acc is fully overwritten
+cudaError_t launch_render_backward_det(const DevSettings& s, int P, int rows, GeomView g, ImageView im, BinView b,
+                                       long long cap, const float* dL_dout, float4* acc, void* partials,
+                                       cudaStream_t st);
 struct BwdOutputs {
     float* dL_dmeans3D; float* dL_dmeans2D; float* dL_dcolors; float* dL_dopacities;   // dL_dmeans2D is [n_views,P,3]
     float* dL_dscales; float* dL_drotations; float* dL_dcov3D; float* dL_dshs;

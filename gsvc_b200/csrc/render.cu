@@ -373,6 +373,12 @@ __device__ __forceinline__ float half_sum(float v)
     return v;
 }
 
+// DET = false: the 9 sums of every (block, Gaussian) hit are added into the Gaussian's row of `acc` ([P][12]) with
+// atomics, in whatever order the hits land.  DET = true (docs/SPEC.md U14): `acc` is the partials buffer of
+// det_partials(), and each hit's 9 sums are STORED into the slot of its (instance, block), whose hit flag is set;
+// det_reduce_kernel then adds every row's slots in a fixed order.  Slots of hits that are never replayed keep their
+// zeroed flag and are not read.
+template <bool DET>
 __global__ void __launch_bounds__(BWD_THREADS, 12)
 render_backward_kernel(DevSettings s, GeomView geo, ImageView im, BinView bin, unsigned long long cap,
                        const float* __restrict__ dL_dout, float* __restrict__ acc /* [P][12] */)
@@ -566,7 +572,17 @@ render_backward_kernel(DevSettings s, GeomView geo, ImageView im, BinView bin, u
             float d_b = lo(s_b) + hi(s_b);
             const float sum8 = half_reduce8(v, lane);
             d_b = half_sum(d_b);
-            if (red_lane && valid) atomicAdd(acc + (size_t)__float_as_uint(f2v.w) * 12 + red_off, l16 == 1 ? d_b : sum8);
+            if constexpr (DET) {
+                if (valid) {
+                    // instance rg.x + list position, block (warp, half) of the tile in row-major order
+                    const size_t slot = ((size_t)rg.x + (unsigned int)(posb - k)) * 4 + warp * 2 + half;
+                    const DetPartials dp = det_partials(acc, cap);
+                    if (red_lane) dp.val[slot * 9 + red_off] = l16 == 1 ? d_b : sum8;
+                    if (l16 == 0) dp.hit[slot] = 1;
+                }
+            } else {
+                if (red_lane && valid) atomicAdd(acc + (size_t)__float_as_uint(f2v.w) * 12 + red_off, l16 == 1 ? d_b : sum8);
+            }
         }
     }
 }
@@ -582,8 +598,90 @@ cudaError_t launch_render_backward(const DevSettings& s, int rows, GeomView g, I
     const int T = s.gx * s.gy * s.n_views;
     if (T <= 0 || rows <= 0) return cudaSuccess;
     count_launch();
-    return launch_pdl(render_backward_kernel, dim3(T), dim3(BWD_THREADS), st, s, g, im, b, (unsigned long long)cap,
-                      dL_dout, reinterpret_cast<float*>(acc));
+    return launch_pdl(render_backward_kernel<false>, dim3(T), dim3(BWD_THREADS), st, s, g, im, b,
+                      (unsigned long long)cap, dL_dout, reinterpret_cast<float*>(acc));
+}
+
+// ---- fixed-order reduction of the deterministic backward (docs/SPEC.md U14) ------------------------------------
+// One thread per row.  Its rectangle's tiles are visited in row-major order; in each tile the row's instance is found
+// by a binary search of the tile's sorted (depth key, id) pairs for the row's own pair (the sort's order, ties broken
+// by the id; a Gaussian occurs at most once per tile), and the flagged slots of its four blocks are added in block
+// order.  The sum is kept in double and rounded once into the fp32 accumulator row, which is fully written (zeros for
+// a culled row, and for every row of a void launch, as the atomic path leaves them).
+constexpr int REDUCE_THREADS = 128;
+
+__global__ void __launch_bounds__(REDUCE_THREADS)
+det_reduce_kernel(DevSettings s, int P, int rows, GeomView geo, ImageView im, BinView bin, unsigned long long cap,
+                  const float* __restrict__ partials, float4* __restrict__ acc)
+{
+    pdl_prologue();
+    const int r = blockIdx.x * REDUCE_THREADS + threadIdx.x;
+    if (r >= rows) return;
+    double sum[9];
+#pragma unroll
+    for (int i = 0; i < 9; i++) sum[i] = 0.0;
+    const ushort4 rc = geo.rect[r];
+    if (im.hdr->overflow == 0u && rc.z > rc.x && rc.w > rc.y) {
+        int v = 0;
+        if (s.ragged) {
+            while (v + 1 < s.n_views && r >= s.rows.off[v + 1]) v++;
+        } else {
+            v = r / P;
+        }
+        const DetPartials dp = det_partials(partials, cap);
+        const unsigned int key = ordered_u32(geo.feat2[r].w);
+        const unsigned int* const hit4 = reinterpret_cast<const unsigned int*>(dp.hit);
+        const unsigned int* const ids = bin.point_list;
+        const unsigned int* const keys = bin.depth_keys;
+        const int tbase = v * s.gx * s.gy;
+        for (int ty = rc.y; ty < rc.w; ty++) {
+            for (int tx = rc.x; tx < rc.z; tx++) {
+                const uint2 rg = im.ranges[tbase + ty * s.gx + tx];
+                if ((unsigned long long)rg.y > cap) continue;
+                // first position whose (key, id) is not below the row's
+                unsigned int lo = rg.x, hi = rg.y;
+                while (lo < hi) {
+                    const unsigned int mid = lo + ((hi - lo) >> 1);
+                    const unsigned int km = __ldg(keys + mid), im_ = __ldg(ids + mid);
+                    if (km < key || (km == key && im_ < (unsigned int)r)) lo = mid + 1;
+                    else hi = mid;
+                }
+                if (lo >= rg.y || __ldg(ids + lo) != (unsigned int)r) continue;
+                const unsigned int f = hit4[lo];
+                const float* const pv = dp.val + (size_t)lo * 36;
+#pragma unroll
+                for (int b = 0; b < 4; b++) {
+                    if ((f >> (8 * b)) & 0xffu) {
+#pragma unroll
+                        for (int i = 0; i < 9; i++) sum[i] += (double)pv[9 * b + i];
+                    }
+                }
+            }
+        }
+    }
+    acc[3 * (size_t)r] = make_float4((float)sum[0], (float)sum[1], (float)sum[2], (float)sum[3]);
+    acc[3 * (size_t)r + 1] = make_float4((float)sum[4], (float)sum[5], (float)sum[6], (float)sum[7]);
+    acc[3 * (size_t)r + 2] = make_float4((float)sum[8], 0.f, 0.f, 0.f);
+}
+
+cudaError_t launch_render_backward_det(const DevSettings& s, int P, int rows, GeomView g, ImageView im, BinView b,
+                                       long long cap, const float* dL_dout, float4* acc, void* partials,
+                                       cudaStream_t st)
+{
+    const DetPartials dp = det_partials(static_cast<float*>(partials), (unsigned long long)cap);
+    cudaError_t e = cudaMemsetAsync(dp.hit, 0, (size_t)cap * 4, st);
+    if (e != cudaSuccess) return e;
+    const int T = s.gx * s.gy * s.n_views;
+    if (rows <= 0) return cudaSuccess;
+    if (T > 0) {
+        count_launch();
+        e = launch_pdl(render_backward_kernel<true>, dim3(T), dim3(BWD_THREADS), st, s, g, im, b,
+                       (unsigned long long)cap, dL_dout, static_cast<float*>(partials));
+        if (e != cudaSuccess) return e;
+    }
+    count_launch();
+    return launch_pdl(det_reduce_kernel, dim3((rows + REDUCE_THREADS - 1) / REDUCE_THREADS), dim3(REDUCE_THREADS), st,
+                      s, P, rows, g, im, b, (unsigned long long)cap, static_cast<const float*>(partials), acc);
 }
 
 }  // namespace gsvc

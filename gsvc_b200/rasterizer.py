@@ -16,6 +16,12 @@ one view through the batched entry points (gsvc_rast_forward_views_launch, + gsv
 on overflow; gsvc_rast_backward_views), the same kernels and buffer sizes as the single-view entry points.  A batch
 over per-view Gaussian sets (rasterize_views(..., counts=...)) goes through the same Function and the
 gsvc_rast_*_ragged entry points.
+
+Under torch.use_deterministic_algorithms(True) the backward takes the deterministic form of the blend backward
+(gsvc_rast_backward_*_det, docs/SPEC.md U14): every gradient, means2D's included, is the same bit for bit on every
+run.  The flag is read when the backward is issued, so a CUDA graph (GraphedStep), a HostStepPipeline step and a
+sharding.packed_backward target keep the mode they were captured or issued under.  A batch whose forward adds three
+or more views into one output image is refused under the flag: the order of those adds is not fixed.
 """
 from __future__ import annotations
 
@@ -336,6 +342,12 @@ class _RasterizeViews(torch.autograd.Function):
         device = means3D.device
         single = batch is None
         ragged = counts is not None
+        if not single and torch.are_deterministic_algorithms_enabled():
+            shared = max(batch.out_image.count(o) for o in set(batch.out_image))
+            if shared >= 3:
+                raise RasterizerError(f"{shared} views add into one output image: under "
+                                      "torch.use_deterministic_algorithms(True) at most two views may share an image "
+                                      "(the order of three or more adds is not fixed)")
         with _on_device(device):
             # the reference builds new settings on every render(): the drop-in's descriptor is built per call
             nv = _NativeViews(None, device, rs) if single else batch.native(device)
@@ -465,39 +477,45 @@ class _RasterizeViews(torch.autograd.Function):
             widths = (3, 3 if ragged else 3 * V, 1, 3 if col is not None else 0, ctx.sh_M * 3 if sh is not None else 0,
                       3 if sc is not None else 0, 4 if rot is not None else 0, 6 if cov is not None else 0)
             n_scratch = 0 if n_acc else L.gsvc_rast_backward_scratch_bytes(rows) // 4
+            # the deterministic blend backward's per-instance partials (docs/SPEC.md U14), after the scratch
+            det = torch.are_deterministic_algorithms_enabled()
+            n_part = L.gsvc_rast_backward_partials_bytes(ctx.capacity) // 4 if det else 0
             # the accumulators inside the forward state were zeroed by the preprocess kernel; a backward
             # dirties them, so a second backward over the same graph (retain_graph) asks for a clear
             acc_clean = 1 if (n_acc and not getattr(ctx, "acc_dirty", False)) else 0
             ctx.acc_dirty = True
-            flat = torch.empty((sum(widths) * P + n_scratch + 64 + 4 * len(widths),), dtype=_F32, device=device)
+            flat = torch.empty((sum(widths) * P + n_scratch + n_part + 64 + 4 * len(widths),), dtype=_F32,
+                               device=device)
             outs, off = [], 0
             for w in widths:
                 outs.append(flat[off:off + w * P] if w else None)
                 off = (off + w * P + 3) & ~3  # every slice starts 16-byte aligned (float4 stores)
             off = (off + 63) & ~63  # 256-byte aligned scratch
             scratch_p = base + n_geom + n_img if n_acc else flat.data_ptr() + 4 * off
+            part = (flat.data_ptr() + 4 * (off + n_scratch), 4 * n_part) if det else ()
             g_means3D, g_means2D, g_opac, g_col, g_sh, g_sc, g_rot, g_cov = outs
             try:
                 if exchange is not None:
-                    _lib.check(L.gsvc_rast_backward_views_exchange(
+                    fn = "gsvc_rast_backward_views_exchange" + ("_det" if det else "")
+                    _lib.check(getattr(L, fn)(
                         nv.ref, V, nv.views, n_out, P, ctx.sh_M, ctx.capacity, _ptr(means3D), _ptr(sh), _ptr(col),
                         _ptr(sc), _ptr(rot), _ptr(cov), _ptr(radii), base, base + n_geom, bin_p, scratch_p, acc_clean,
-                        _ptr(g_out), _ptr(g_means2D), _ptr(packed), C.byref(exchange.exchange_struct()),
-                        _stream_ptr(device)), "gsvc_rast_backward_views_exchange")
+                        _ptr(g_out), _ptr(g_means2D), _ptr(packed), C.byref(exchange.exchange_struct()), *part,
+                        _stream_ptr(device)), fn)
                 elif ragged:
-                    _lib.check(L.gsvc_rast_backward_ragged(
+                    fn = "gsvc_rast_backward_ragged" + ("_det" if det else "")
+                    _lib.check(getattr(L, fn)(
                         nv.ref, V, nv.views, n_out, ctx.counts_c, ctx.sh_M, ctx.capacity, _ptr(means3D), _ptr(sh),
                         _ptr(col), _ptr(sc), _ptr(rot), _ptr(cov), _ptr(radii), base, base + n_geom, bin_p, scratch_p,
                         acc_clean, _ptr(g_out), _ptr(g_means3D), _ptr(g_means2D), _ptr(g_col), _ptr(g_opac),
-                        _ptr(g_sc), _ptr(g_rot), _ptr(g_cov), _ptr(g_sh), _stream_ptr(device)),
-                        "gsvc_rast_backward_ragged")
+                        _ptr(g_sc), _ptr(g_rot), _ptr(g_cov), _ptr(g_sh), *part, _stream_ptr(device)), fn)
                 else:
-                    _lib.check(L.gsvc_rast_backward_views(
+                    fn = "gsvc_rast_backward_views" + ("_det" if det else "")
+                    _lib.check(getattr(L, fn)(
                         nv.ref, V, nv.views, n_out, P, ctx.sh_M, ctx.capacity, _ptr(means3D), _ptr(sh), _ptr(col),
                         _ptr(sc), _ptr(rot), _ptr(cov), _ptr(radii), base, base + n_geom, bin_p, scratch_p, acc_clean,
                         _ptr(g_out), _ptr(g_means3D), _ptr(g_means2D), _ptr(g_col), _ptr(g_opac), _ptr(g_sc),
-                        _ptr(g_rot), _ptr(g_cov), _ptr(g_sh), _ptr(packed), _stream_ptr(device)),
-                        "gsvc_rast_backward_views")
+                        _ptr(g_rot), _ptr(g_cov), _ptr(g_sh), _ptr(packed), *part, _stream_ptr(device)), fn)
             except Exception:
                 if ctx.rs.debug:
                     torch.save((means3D, sh, col, sc, rot, cov, radii, grad_out_color)

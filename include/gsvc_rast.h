@@ -220,6 +220,29 @@ GSVC_RAST_API int gsvc_rast_backward_views(const gsvc_rast_settings *st, int32_t
                              float *dL_dcov3D, float *dL_dshs, float *dL_packed, void *stream);
 
 /*
+ * Deterministic blend backward (docs/SPEC.md U14): bit-identical gradients on every run.  The atomic backward adds the
+ * sums of every (8x8 block, Gaussian) hit into the Gaussian's accumulator in whatever order the hits land.  These
+ * forms store each hit's sums into a slot of `partials` and add every Gaussian's slots in a fixed order (the tiles of
+ * its rectangle row-major, then the four blocks of a tile), in double, rounded once.  `partials`:
+ * gsvc_rast_backward_partials_bytes(capacity) bytes of device memory, any content (the call clears the part it needs:
+ * 4 bytes per instance); 144 bytes per instance of capacity in all.  A NULL or too small buffer is
+ * GSVC_RAST_ERR_INVALID before any CUDA work.  `scratch` is fully overwritten, whatever scratch_is_zero says.
+ * Each _det entry point takes its twin's arguments plus (partials, partials_bytes) and is otherwise the same call.
+ * What stays order-dependent: the forward of a batch that maps three or more views onto one output image (its atomic
+ * adds onto the zeroed image), and the exchange's sum over the ranks.
+ */
+GSVC_RAST_API size_t gsvc_rast_backward_partials_bytes(int64_t capacity);
+GSVC_RAST_API int gsvc_rast_backward_views_det(const gsvc_rast_settings *st, int32_t n_views,
+                             const gsvc_rast_view *views_host, int32_t n_out, int32_t P, int32_t sh_M, int64_t capacity,
+                             const float *means3D, const float *shs, const float *colors_precomp, const float *scales,
+                             const float *rotations, const float *cov3D_precomp, const int32_t *radii,
+                             const void *geom, const void *image, const void *binning, void *scratch,
+                             int32_t scratch_is_zero, const float *dL_dout, float *dL_dmeans3D, float *dL_dmeans2D,
+                             float *dL_dcolors, float *dL_dopacities, float *dL_dscales, float *dL_drotations,
+                             float *dL_dcov3D, float *dL_dshs, float *dL_packed, void *partials, size_t partials_bytes,
+                             void *stream);
+
+/*
  * Batched views over per-view Gaussian sets ("ragged" batches, docs/SPEC.md "Binning").  The reference regenerates its
  * neural Gaussians on every render() call (ortho_gaussian_renderer/guassian.py:147-246: per-view visibility mask,
  * embeddings from the view's camera, training noise), so every view of a training iteration or a decoded frame has a
@@ -252,6 +275,15 @@ GSVC_RAST_API int gsvc_rast_backward_ragged(const gsvc_rast_settings *st, int32_
                              int32_t scratch_is_zero, const float *dL_dout, float *dL_dmeans3D, float *dL_dmeans2D,
                              float *dL_dcolors, float *dL_dopacities, float *dL_dscales, float *dL_drotations,
                              float *dL_dcov3D, float *dL_dshs, void *stream);
+GSVC_RAST_API int gsvc_rast_backward_ragged_det(const gsvc_rast_settings *st, int32_t n_views,
+                             const gsvc_rast_view *views_host, int32_t n_out, const int32_t *counts_host, int32_t sh_M,
+                             int64_t capacity, const float *means3D, const float *shs, const float *colors_precomp,
+                             const float *scales, const float *rotations, const float *cov3D_precomp,
+                             const int32_t *radii, const void *geom, const void *image, const void *binning,
+                             void *scratch, int32_t scratch_is_zero, const float *dL_dout, float *dL_dmeans3D,
+                             float *dL_dmeans2D, float *dL_dcolors, float *dL_dopacities, float *dL_dscales,
+                             float *dL_drotations, float *dL_dcov3D, float *dL_dshs, void *partials,
+                             size_t partials_bytes, void *stream);
 
 /*
  * Densification statistic of the step at the rasterizer boundary.  The reference calls
@@ -331,6 +363,14 @@ GSVC_RAST_API int gsvc_rast_backward_views_exchange(const gsvc_rast_settings *st
                              const void *image, const void *binning, void *scratch, int32_t scratch_is_zero,
                              const float *dL_dout, float *dL_dmeans2D, float *dL_packed,
                              const gsvc_rast_exchange *exchange, void *stream);
+/* the deterministic form (gsvc_rast_backward_views_det); the sum over the ranks is not part of its promise */
+GSVC_RAST_API int gsvc_rast_backward_views_exchange_det(const gsvc_rast_settings *st, int32_t n_views,
+                             const gsvc_rast_view *views_host, int32_t n_out, int32_t P, int32_t sh_M, int64_t capacity,
+                             const float *means3D, const float *shs, const float *colors_precomp, const float *scales,
+                             const float *rotations, const float *cov3D_precomp, const int32_t *radii, const void *geom,
+                             const void *image, const void *binning, void *scratch, int32_t scratch_is_zero,
+                             const float *dL_dout, float *dL_dmeans2D, float *dL_packed,
+                             const gsvc_rast_exchange *exchange, void *partials, size_t partials_bytes, void *stream);
 
 /*
  * Stage exports for bit-exact parity tests (not used on the hot path).
